@@ -2,9 +2,10 @@
 // sm_100a only; no CPU fallback -- every entry point needs a CUDA device.
 //
 // Kernel inventory (one item per thread, 128-thread CTAs, grid = ceil(n/128) >> 148 SMs):
-//   k_decode_g1 / k_decode_g2   K1  compressed bytes -> affine Montgomery limb-SoA + decode code
+//   k_decode_g1 / k_decode_g2   K1  compressed bytes -> affine Montgomery limb-SoA + decode code | k_decode_g2<false>: no subgroup test (verify_batch, split form)
 //   k_hash_to_g2                K2  message -> H(m) affine limb-SoA            | split form (default): k_hash_field -> k_hash_map (2n threads) -> k_hash_clear
-//   k_miller                    K4  (pk, H(m), sig) -> Fp12 Miller value limb-SoA | split form: 8 x (k_miller_lines (2n threads) -> k_miller_accum)
+//   k_miller                    K4  (pk, H(m), sig) -> Fp12 Miller value limb-SoA | split form: 8 x (k_miller_lines (2n threads) -> k_miller_accum);
+//                                   in verify_batch the last pair of launches also tests sig in G2 on the running point [|x|] sig -> ST_BAD_SIG
 //   k_final_exp                 K5  Fp12 -> GT, is_one -> status                   | split form: k_final_step<0>, 5 x (k_final_squarings -> k_final_step<k>)
 //   k_miller_accum_coop, k_final_hard_coop   six lanes per item: passes of at most VERIFY_COOP_BELOW items (latency), blsgpu_set_coop
 //   k_gt_reduce                 K5' strided product of GT values (per-batch accumulator)
@@ -40,7 +41,8 @@ static inline unsigned nblk(size_t n, unsigned tpb = TPB) { return (unsigned)((n
 
 // resident CTAs per SM of single kernels (register cap 65536 / (TPB * MINB)); BLS_MINB is the default for all stage kernels.  Measured at 2^20
 // (profiles/r02_tuning.md): the two decoders gain 4 % / 2 % at 4 CTAs (128 registers), the compressed-squaring run 1 % at 3; k_hash_to_g2 loses 6 % at 3,
-// its split forms k_hash_field / k_hash_map gain 1 % of the stage at 4 / 3.
+// its split forms k_hash_field / k_hash_map gain 1 % of the stage at 4 / 3.  k_decode_g2<false> (no subgroup test) takes 35.7 ms at 4 and 35.4 ms
+// at 3 (152 registers, no spills), the step the same within its run-to-run spread (profiles/r03_sig_subgroup.md): both forms stay at 4.
 #ifndef BLS_MINB_DG1
 #define BLS_MINB_DG1 4
 #endif
@@ -146,10 +148,11 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_DG1) k_decode_g1(const uint8_t* 
     if (soa) soa_store_g1(soa, n, i, p);
     code[i] = (uint8_t)rc;
 }
-__global__ void __launch_bounds__(TPB, BLS_MINB_DG2) k_decode_g2(const uint8_t* in96, size_t n, u32x4* soa, uint8_t* code) {
+// SUBGROUP = false: on-curve decode only, for blsgpu_verify_batch's split path, whose Miller loop tests membership (k_miller_lines)
+template <bool SUBGROUP> __global__ void __launch_bounds__(TPB, BLS_MINB_DG2) k_decode_g2(const uint8_t* in96, size_t n, u32x4* soa, uint8_t* code) {
     phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
-    g2_aff p; int rc = g2_decode(p, in96 + 96 * i);
+    g2_aff p; int rc = g2_decode<SUBGROUP>(p, in96 + 96 * i);
     if (soa) soa_store_g2(soa, n, i, p);
     code[i] = (uint8_t)rc;
 }
@@ -244,8 +247,11 @@ __global__ void __launch_bounds__(TPB, BLS_MINB) k_miller(const u32x4* pk_soa, c
 // doubling / addition steps of ONE pair per thread (2n threads: small state, small code) for a range of iterations and leaves the line
 // coefficients, already scaled by the G1 coordinates, in global memory; k_miller_accum squares f and multiplies the lines in (fp12_sqr and
 // mul_by_014 only).  Line buffer: step s, pair j, coefficient k at rows ((2 s + j) * 3 + k) * 6 .. of an n-column limb-SoA matrix.
+// sig_sub (nullable): the last launch (i_lo = 0) stores the signature's subgroup test there (1 = in G2) for every item with status ST_OK
+// and a finite signature -- pair 0 ends on [|x|] sig (miller_end_in_subgroup) -- and the last k_miller_accum(_coop) folds it into the
+// status.  Not status[] itself: the pair-1 thread of the same item reads that in this launch.
 __global__ void __launch_bounds__(TPB, BLS_MINB_LINES) k_miller_lines(const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags, const uint8_t* status,
-                                                                size_t n, u32x4* t_soa, u32x4* lines, int i_hi, int i_lo) {
+                                                                size_t n, u32x4* t_soa, u32x4* lines, int i_hi, int i_lo, uint8_t* sig_sub) {
     size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (t >= 2 * n) return;
     int j = t >= n; size_t i = t - (j ? n : 0);
     if (status[i] != ST_OK) return;
@@ -264,8 +270,12 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_LINES) k_miller_lines(const u32x
         }
     }
     if (i_lo != 0) { soa_store_fp2(t_soa, n, i, 3 * j, r.x); soa_store_fp2(t_soa, n, i, 3 * j + 1, r.y); soa_store_fp2(t_soa, n, i, 3 * j + 2, r.z); }
+    else if (j == 0 && sig_sub) sig_sub[i] = miller_end_in_subgroup(r, q) ? 1 : 0;
 }
-__global__ void __launch_bounds__(TPB, BLS_MINB_ACCUM) k_miller_accum(const uint8_t* flags, const uint8_t* status, size_t n, u32x4* f_soa, const u32x4* lines, int i_hi, int i_lo) {
+// sig_sub (nullable, see k_miller_lines): in the last launch an item whose signature failed the subgroup test gets ST_BAD_SIG instead of its f.
+// Only items with status ST_OK get here, so ST_BAD_PK keeps precedence as in k_hash_field / k_status_merge.
+__global__ void __launch_bounds__(TPB, BLS_MINB_ACCUM) k_miller_accum(const uint8_t* flags, uint8_t* status, size_t n, u32x4* f_soa, const u32x4* lines, int i_hi, int i_lo,
+                                                                const uint8_t* sig_sub) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     if (status[i] != ST_OK) return;
     uint8_t fl = flags[i]; bool use0 = !(fl & FL_SIG_INF), use1 = !(fl & FL_HM_INF);
@@ -280,6 +290,7 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_ACCUM) k_miller_accum(const uint
         }
     }
     if (i_lo == 0) fp12_conj(f, f);
+    if (i_lo == 0 && sig_sub && use0 && !sig_sub[i]) { status[i] = ST_BAD_SIG; return; }
     soa_store_fp12(f_soa, n, i, f);
 }
 // the 63 compressed squarings of one exp_by_x: in = an Fp12 array (cyclotomic elements), out = six snapshots of four Fp2 (24 x 6 uint4 rows per item)
@@ -368,7 +379,9 @@ __global__ void __launch_bounds__(128, 2) k_final_hard_coop(u32x4* f_soa, const 
 // The accumulator update of the split Miller loop with six lanes per item (small passes, blsgpu_set_coop): lane k holds the w^k coefficient of f,
 // a line l0 + l1 v + l2 v w sits in lanes 0, 2, 3 (w^0, w^2, w^3) of an otherwise zero operand, a pair that is switched off multiplies by one.
 // Three to five generic six-lane products per iteration instead of one squaring and two sparse products in one thread: more work, a third of the chain.
-__global__ void __launch_bounds__(128, 2) k_miller_accum_coop(const uint8_t* flags, const uint8_t* status, size_t n, u32x4* f_soa, const u32x4* lines, int i_hi, int i_lo) {
+// sig_sub: as in k_miller_accum.  Lane 0 writes the status after the last coop_mul, whose __syncwarp orders it after every lane's read.
+__global__ void __launch_bounds__(128, 2) k_miller_accum_coop(const uint8_t* flags, uint8_t* status, size_t n, u32x4* f_soa, const u32x4* lines, int i_hi, int i_lo,
+                                                            const uint8_t* sig_sub) {
     __shared__ coop_smem sm[4];
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane / 6;
     coop_lane c = coop_init(&sm[warp]);
@@ -391,6 +404,7 @@ __global__ void __launch_bounds__(128, 2) k_miller_accum_coop(const uint8_t* fla
             }
     }
     if (i_lo == 0) f = coop_conj(c, f);
+    if (active && i_lo == 0 && sig_sub && use[0] && !sig_sub[item]) { if (c.k == 0) status[item] = ST_BAD_SIG; return; }
     if (active) soa_store_fp2(f_soa, n, item, COOP_TOWER_POS[c.k], f);
 }
 // out[t] = prod_{i = t, t+T, ...} in[i] over items with status <= ST_FALSE (status == NULL: all items)
@@ -865,7 +879,7 @@ int blsgpu_deserialize_g2(blsgpu_ctx* ctx, const uint8_t* in96, size_t n, uint8_
     if (int rc = ws_reserve(ctx, al(96 * n) + al(n) + 4096)) return rc;
     const uint8_t* din; if (int rc = stage_in(ctx, din, in96, 96 * n)) return rc;
     uint8_t* dst = stage_out(ctx, status, n);
-    LAUNCH(k_decode_g2, nblk(n), TPB, din, n, (u32x4*)nullptr, dst);
+    LAUNCH(k_decode_g2<true>, nblk(n), TPB, din, n, (u32x4*)nullptr, dst);
     if (int rc = finish_out(ctx, status, dst, n)) return rc;
     return finish_call(ctx);
 }
@@ -899,28 +913,33 @@ static int hash_stage(blsgpu_ctx* ctx, const uint8_t* dmsg, const uint32_t* doff
     } else LAUNCH(k_hash_to_g2, nblk(n), TPB, dmsg, doff, n, code_pk, code_sig, hm_soa, flags, dstatus);
     return 0;
 }
-// Miller loop in its split form: iterations 62..0 eight at a time, lines of both pairs (a pair switched off in flags costs nothing), then the accumulator update
-static int miller_stage_split(blsgpu_ctx* ctx, const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags, const uint8_t* dstatus, size_t n,
-                              u32x4* f_soa, u32x4* t_soa /* 36 n rows */, u32x4* lines /* MILLER_LINE_STEPS * 36 n rows */, bool coop = false) {
+// Miller loop in its split form: iterations 62..0 eight at a time, lines of both pairs (a pair switched off in flags costs nothing), then the accumulator update.
+// sig_sub (n bytes, nullable): the signatures were decoded without the subgroup test, and the loop does it (k_miller_lines); failures become ST_BAD_SIG
+static int miller_stage_split(blsgpu_ctx* ctx, const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags, uint8_t* dstatus, size_t n,
+                              u32x4* f_soa, u32x4* t_soa /* 36 n rows */, u32x4* lines /* MILLER_LINE_STEPS * 36 n rows */, uint8_t* sig_sub, bool coop = false) {
     for (int hi = 62; hi >= 0; hi -= MILLER_LINE_ITERS) {
         int lo = hi - MILLER_LINE_ITERS + 1 < 0 ? 0 : hi - MILLER_LINE_ITERS + 1;
-        LAUNCH(k_miller_lines, nblk(2 * n), TPB, pk_soa, hm_soa, sig_soa, flags, dstatus, n, t_soa, lines, hi, lo);
-        if (coop) LAUNCH(k_miller_accum_coop, nblk(n, 20), 128, flags, dstatus, n, f_soa, (const u32x4*)lines, hi, lo);
-        else LAUNCH(k_miller_accum, nblk(n), TPB, flags, dstatus, n, f_soa, (const u32x4*)lines, hi, lo);
+        LAUNCH(k_miller_lines, nblk(2 * n), TPB, pk_soa, hm_soa, sig_soa, flags, (const uint8_t*)dstatus, n, t_soa, lines, hi, lo, sig_sub);
+        if (coop) LAUNCH(k_miller_accum_coop, nblk(n, 20), 128, flags, dstatus, n, f_soa, (const u32x4*)lines, hi, lo, (const uint8_t*)sig_sub);
+        else LAUNCH(k_miller_accum, nblk(n), TPB, flags, dstatus, n, f_soa, (const u32x4*)lines, hi, lo, (const uint8_t*)sig_sub);
     }
     return 0;
 }
-// core of verify once pk (limb-SoA + code) is known: decode sig, hash, Miller, final exp, epilogue
+// core of verify once pk (limb-SoA + code) is known: decode sig, hash, Miller, final exp, epilogue.
+// sig_sub_in_miller: with the split stage kernels, the signature's subgroup test runs on the Miller loop's running point (k_miller_lines) instead of
+// in the decoder, which saves the decoder's [|x|] sig ladder (the loop computes the same point); the outcome is the same ST_BAD_SIG.
 static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code_pk, const uint8_t* dmsg, const uint32_t* doff, const uint8_t* dsig, size_t n,
-                       uint8_t* dstatus, uint32_t* dbitmap, u32x4* gt_acc /* limb-SoA n=1, multiplied into; nullable */, bool forked = false) {
+                       uint8_t* dstatus, uint32_t* dbitmap, u32x4* gt_acc /* limb-SoA n=1, multiplied into; nullable */, bool forked = false, bool sig_sub_in_miller = false) {
     u32x4* sig_soa = ws_take<u32x4>(ctx, 12 * n); u32x4* hm_soa = ws_take<u32x4>(ctx, 12 * n); u32x4* f_soa = ws_take<u32x4>(ctx, 36 * n);
     uint8_t* code_sig = ws_take<uint8_t>(ctx, n); uint8_t* flags = ws_take<uint8_t>(ctx, n);
+    uint8_t* sig_sub = sig_sub_in_miller && ctx->split ? ws_take<uint8_t>(ctx, n) : nullptr;
+    auto decode_sig = sig_sub ? k_decode_g2<false> : k_decode_g2<true>;
     if (forked) {
         // Small pass (the caller recorded ctx->fork before it enqueued the key decoder on ctx->stream): the signature decoder and the hash run on
         // the two lane streams beside it -- three independent serial chains instead of one after the other -- and the status rule follows the join.
         cudaStream_t main_stream = ctx->stream; int rc = 0;
         ctx->stream = ctx->lane_stream[0]; cudaStreamWaitEvent(ctx->stream, ctx->fork, 0);
-        k_decode_g2<<<nblk(n), TPB, 0, ctx->stream>>>(dsig, n, sig_soa, code_sig); ctx->launches++; cudaEventRecord(ctx->lane_done[0], ctx->stream);
+        decode_sig<<<nblk(n), TPB, 0, ctx->stream>>>(dsig, n, sig_soa, code_sig); ctx->launches++; cudaEventRecord(ctx->lane_done[0], ctx->stream);
         ctx->stream = ctx->lane_stream[1]; cudaStreamWaitEvent(ctx->stream, ctx->fork, 0);
         rc = hash_stage(ctx, dmsg, doff, n, nullptr, nullptr, hm_soa, f_soa, flags, nullptr); cudaEventRecord(ctx->lane_done[1], ctx->stream);
         ctx->stream = main_stream;
@@ -930,7 +949,7 @@ static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code
         LAUNCH(k_status_merge, nblk(n, 256), 256, code_pk, (const uint8_t*)code_sig, n, flags, dstatus);
     } else {
     STAGE_MARK(1);
-    LAUNCH(k_decode_g2, nblk(n), TPB, dsig, n, sig_soa, code_sig);
+    LAUNCH(decode_sig, nblk(n), TPB, dsig, n, sig_soa, code_sig);
     STAGE_MARK(2);
     if (int rc = hash_stage(ctx, dmsg, doff, n, code_pk, code_sig, hm_soa, f_soa, flags, dstatus)) return rc;
     }
@@ -943,7 +962,7 @@ static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code
         // iterations 62..0 eight at a time: lines of both pairs, then the accumulator update
         u32x4* t_soa = ws_take<u32x4>(ctx, 36 * n); y1_soa = t_soa; y2_soa = ws_take<u32x4>(ctx, 36 * n);      // the running points are dead once the loop ends
         u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * n);
-        if (int rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, n, f_soa, t_soa, lines, coop)) return rc;
+        if (int rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, n, f_soa, t_soa, lines, sig_sub, coop)) return rc;
         snap_soa = lines;                                      // 144 rows of the 396-row line buffer, which is dead once the loop ends
     } else {
 #if BLS_F_IN_SMEM
@@ -982,7 +1001,7 @@ static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code
     return 0;
 }
 static size_t verify_ws_bytes(size_t n, size_t mb) {
-    return 2 * al(576 * n) + al((size_t)MILLER_LINE_STEPS * 2 * 288 * n) /* state of the split stage kernels: running points / y1, y2, line buffer / snapshots */ + al(48 * n) + al(96 * n) + al(mb + 1) + al(4 * (n + 1)) + al(n) * 6 + al(96 * n) + 2 * al(192 * n) + al(576 * n) + al(8 * ((n + 63) / 64)) +
+    return 2 * al(576 * n) + al((size_t)MILLER_LINE_STEPS * 2 * 288 * n) /* state of the split stage kernels: running points / y1, y2, line buffer / snapshots */ + al(48 * n) + al(96 * n) + al(mb + 1) + al(4 * (n + 1)) + al(n) * 7 + al(96 * n) + 2 * al(192 * n) + al(576 * n) + al(8 * ((n + 63) / 64)) +
            al(576 * ((n + 7) / 8)) + al(576 * ((n + 63) / 64)) + 3 * al(576) + 65536;
 }
 static int ensure_lanes(blsgpu_ctx* ctx);
@@ -1011,7 +1030,7 @@ static int verify_range(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg
     if (forked) { if ((rc = ensure_lanes(ctx))) return rc; forked = ctx->stream != ctx->lane_stream[0] && ctx->stream != ctx->lane_stream[1]; }
     if (forked) CU(cudaEventRecord(ctx->fork, ctx->stream));
     LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-    if ((rc = verify_core(ctx, pk_soa, code_pk, dmsg, doff, dsig, m, dstatus, dbitmap, gt_acc, forked))) return rc;
+    if ((rc = verify_core(ctx, pk_soa, code_pk, dmsg, doff, dsig, m, dstatus, dbitmap, gt_acc, forked, true))) return rc;
     if ((rc = finish_out(ctx, status + base, dstatus, m))) return rc;
     if (ok_bitmap && (rc = finish_out(ctx, ok_bitmap + base / 64, (uint64_t*)dbitmap, (m + 63) / 64))) return rc;
     return 0;
@@ -1125,7 +1144,7 @@ int blsgpu_verify_batch_rlc(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t*
         u32x4* rs = ws_take<u32x4>(ctx, 18 * m); u32x4* ja = ws_take<u32x4>(ctx, 18 * ((m + 7) / 8)); u32x4* jb = ws_take<u32x4>(ctx, 18 * ((m + 63) / 64)); u32x4* jone = ws_take<u32x4>(ctx, 18);
         u32x4* ta = ws_take<u32x4>(ctx, 36 * ((m + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((m + 63) / 64)); u32x4* one = ws_take<u32x4>(ctx, 36);
         LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-        LAUNCH(k_decode_g2, nblk(m), TPB, dsig, m, sig_soa, code_sig);
+        LAUNCH(k_decode_g2<true>, nblk(m), TPB, dsig, m, sig_soa, code_sig);
         if ((rc = hash_stage(ctx, dmsg, doff, m, code_pk, code_sig, hm_soa, f_soa, flags, dstatus))) break;
         LAUNCH(k_any_bad, nblk(((m + 31) / 32) * 32, 256), 256, (const uint8_t*)dstatus, m, bad);
         LAUNCH(k_rlc_scale, nblk(m), TPB, pk_soa, (const u32x4*)sig_soa, flags, (const uint8_t*)dstatus, m, base, (const uint8_t*)dseed, rs);
@@ -1141,7 +1160,7 @@ int blsgpu_verify_batch_rlc(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t*
         }
         if (ctx->split) {                                        // verify_ws_bytes counts the running-point array and the line buffer
             u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
-            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines))) break;
+            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr))) break;
         } else LAUNCH(k_miller, nblk(m), TPB, (const u32x4*)pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, m, f_soa);
         if ((rc = gt_product(ctx, f_soa, dstatus, m, ta, tb, one))) break;
         LAUNCH(k_gt_mul_into, 1, 32, f_acc, (const u32x4*)one);
@@ -1196,7 +1215,7 @@ int blsgpu_verify_batch_rlc_bisect(blsgpu_ctx* ctx, const uint8_t* pk48, const u
         u32x4* rs = ws_take<u32x4>(ctx, 18 * m); u32x4* ja = ws_take<u32x4>(ctx, 18 * P * T0); u32x4* jb = ws_take<u32x4>(ctx, 18 * P * T0);
         u32x4* ta = ws_take<u32x4>(ctx, 36 * P * T0); u32x4* tb = ws_take<u32x4>(ctx, 36 * P * T0); uint8_t* dok = ws_take<uint8_t>(ctx, P);
         LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-        LAUNCH(k_decode_g2, nblk(m), TPB, dsig, m, sig_soa, code_sig);
+        LAUNCH(k_decode_g2<true>, nblk(m), TPB, dsig, m, sig_soa, code_sig);
         if ((rc = hash_stage(ctx, dmsg, doff, m, code_pk, code_sig, hm_soa, f_soa, flags, dstatus))) return rc;
         LAUNCH(k_rlc_scale, nblk(m), TPB, pk_soa, (const u32x4*)sig_soa, flags, (const uint8_t*)dstatus, m, base, (const uint8_t*)dseed, rs);
         const u32x4* s_piece; const u32x4* f_piece;
@@ -1212,7 +1231,7 @@ int blsgpu_verify_batch_rlc_bisect(blsgpu_ctx* ctx, const uint8_t* pk48, const u
         }
         if (ctx->split) {
             u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
-            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines))) return rc;
+            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr))) return rc;
         } else LAUNCH(k_miller, nblk(m), TPB, (const u32x4*)pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, m, f_soa);
         {
             const u32x4* cur = f_soa; const uint8_t* st = dstatus; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ta, tb}; int which = 0;
@@ -1276,7 +1295,7 @@ int blsgpu_pairing_gt(blsgpu_ctx* ctx, const uint8_t* g1_48, const uint8_t* g2_9
     uint8_t* dst = status && ctx->ptr_mode == BLSGPU_DEVICE ? status : ws_take<uint8_t>(ctx, nprod);
     uint8_t* dgt = stage_out(ctx, gt, 576 * nprod);
     LAUNCH(k_decode_g1, nblk(tot), TPB, d1, tot, s1, c1);
-    LAUNCH(k_decode_g2, nblk(tot), TPB, d2, tot, s2, c2);
+    LAUNCH(k_decode_g2<true>, nblk(tot), TPB, d2, tot, s2, c2);
     LAUNCH(k_miller_pairs, nblk(nprod), TPB, (const u32x4*)s1, (const u32x4*)s2, (const uint8_t*)c1, (const uint8_t*)c2, npairs, nprod, f, dst);
     uint8_t* scratch = ws_take<uint8_t>(ctx, nprod);       // is_one outcome, not reported by this hook
     LAUNCH(k_final_exp, nblk(nprod), TPB, f, (const uint8_t*)dst, scratch, nprod);
@@ -1346,7 +1365,7 @@ int blsgpu_g2_aggregate(blsgpu_ctx* ctx, const uint8_t* pts96, const uint32_t* s
     u32x4* soa = ws_take<u32x4>(ctx, 12 * npts + 1); uint8_t* code = ws_take<uint8_t>(ctx, npts + 1);
     u32x4* osoa = ws_take<u32x4>(ctx, 12 * nseg); uint8_t* oinf = ws_take<uint8_t>(ctx, nseg);
     uint8_t* dout = stage_out(ctx, out96, 96 * nseg); uint8_t* dst = stage_out(ctx, status, nseg);
-    if (npts) LAUNCH(k_decode_g2, nblk(npts), TPB, din, npts, soa, code);
+    if (npts) LAUNCH(k_decode_g2<true>, nblk(npts), TPB, din, npts, soa, code);
     { int L = seg_lanes(npts / nseg); u32x4* ojac = ws_take<u32x4>(ctx, 18 * nseg);
       LAUNCH(k_segsum<fp2>, nblk(nseg, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, dseg, (size_t)0, (const uint64_t*)nullptr, nseg, ojac, dst, (uint8_t)ST_BAD_SIG, (const uint32_t*)nullptr, L);
       LAUNCH(k_jac_to_aff<fp2>, nblk(nseg), TPB, (const u32x4*)ojac, nseg, osoa, oinf); }
@@ -1411,7 +1430,7 @@ int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, const uint8_t* pks48, const u
         LAUNCH(k_hash_to_g2, nblk(npairs), TPB, dmsg, doff, npairs, (const uint8_t*)code_pk, (const uint8_t*)code_inf, hm_soa, pflags, pstatus);
         LAUNCH(k_miller, nblk(npairs), TPB, (const u32x4*)pk_soa, (const u32x4*)hm_soa, (const u32x4*)zero_g2, (const uint8_t*)pflags, (const uint8_t*)pstatus, npairs, f_pair);
     }
-    LAUNCH(k_decode_g2, nblk(nsig), TPB, dsig, nsig, sig_soa, code_sig);
+    LAUNCH(k_decode_g2<true>, nblk(nsig), TPB, dsig, nsig, sig_soa, code_sig);
     LAUNCH(k_aggv_sig_status, nblk(nsig), TPB, (const uint8_t*)code_sig, nsig, sstatus, sflags);
     CU(cudaMemsetAsync(zero_g1, 0, 96 * nsig, ctx->stream)); CU(cudaMemsetAsync(zero_hm, 0, 192 * nsig, ctx->stream));
     LAUNCH(k_miller, nblk(nsig), TPB, (const u32x4*)zero_g1, (const u32x4*)zero_hm, (const u32x4*)sig_soa, (const uint8_t*)sflags, (const uint8_t*)sstatus, nsig, f_sig);

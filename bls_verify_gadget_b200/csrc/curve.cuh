@@ -199,8 +199,9 @@ BLS_HD void g1_encode(uint8_t* b, const g1_aff& a, bool inf) {
     fp_canon_to_be48(b, fp_from_mont(a.x));
     b[0] |= 0x80; if (fp_canon_is_larger_half(fp_from_mont(a.y))) b[0] |= 0x20;
 }
-// 96 bytes (x.c1 || x.c0, big-endian) -> affine G2
-BLS_HD int g2_decode(g2_aff& out, const uint8_t* b) {
+// 96 bytes (x.c1 || x.c0, big-endian) -> affine G2.  SUBGROUP = false stops after the square root: DEC_OK then means "a point on
+// the curve", and the caller owes the membership test (the split Miller loop of blsgpu_verify_batch does it, miller_end_in_subgroup).
+template <bool SUBGROUP = true> BLS_HD int g2_decode(g2_aff& out, const uint8_t* b) {
     uint32_t flags = b[0];
     out.x = fp2_zero(); out.y = fp2_zero();
     if (!(flags & 0x80)) return DEC_BAD_FLAGS;
@@ -211,7 +212,7 @@ BLS_HD int g2_decode(g2_aff& out, const uint8_t* b) {
     fp2 y; if (!fp2_sqrt(y, y2)) return DEC_NOT_ON_CURVE;
     if (fp2_lex_largest(y) != ((flags & 0x20) != 0)) y = fp2_neg(y);
     out.x = x; out.y = y;
-    if (!g2_in_subgroup(out)) return DEC_NOT_IN_SUBGROUP;
+    if (SUBGROUP && !g2_in_subgroup(out)) return DEC_NOT_IN_SUBGROUP;
     return DEC_OK;
 }
 BLS_HD void g2_encode(uint8_t* b, const g2_aff& a, bool inf) {

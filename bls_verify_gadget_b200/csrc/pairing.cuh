@@ -43,6 +43,29 @@ BLS_NOINLINE void miller_add(g2_proj& r, const g2_aff& q, fp2& c0, fp2& c1, fp2&
     r.z = fp2_mul(r.z, e);
     c0 = fp2_sub(fp2_mul(theta, q.x), fp2_mul(lambda, q.y)); c1 = fp2_neg(theta); c2 = lambda;
 }
+// Subgroup test of a signature on the running point its pair leaves at the end of the Miller loop.  The pair (-g1, sig) runs
+// R <- 2R (+ sig) over bits 62..0 of |x| from R = sig: the double-and-add of [|x|] sig.  The test accepts iff Z != 0 and
+// (X/Z, Y/Z) = -psi(sig), which is g2_in_subgroup's condition [|x|] sig = -psi(sig).  It is exact for every finite point sig on
+// the curve, with nothing tracked beside R, because of the two formulas above (homogeneous projective: affine (X/Z, Y/Z)):
+//  * miller_dbl: Z3 = b h = Y^2 (2 Y Z) = 2 Y^3 Z.  With Z != 0 and Y != 0 it is the tangent doubling: every output is homogeneous of
+//    degree 4 in (X, Y, Z), and at Z = 1, with b' = 4(1+u) and y^2 = x^3 + b', X3/Z3 = x (y^2 - 9b') / (4y^2) = l^2 - 2x and
+//    Y3/Z3 = (y^4 + 18b'y^2 - 27b'^2) / (8y^3) = l (x - X3/Z3) - y for l = 3x^2 / (2y); and Z3 != 0.  Y = 0 (a point of order 2)
+//    or Z = 0 gives Z3 = 0.
+//  * miller_add: Z3 = Z e = Z l^3 with l = X - q.x Z.  With Z != 0 and l != 0 (R != +-Q) it is the chord addition (degree 4 again; at
+//    Z = 1, X3/Z3 = t^2/l^2 - x - q.x and Y3/Z3 = (t/l)(x - X3/Z3) - y for t = Y - q.y) and Z3 != 0.  l = 0 (R = +-Q) or Z = 0 gives Z3 = 0.
+// Z = 0 stays 0 whatever X and Y hold, since both formulas multiply Z into Z3.  By induction over the 63 doublings and 5 additions:
+// either no step was exceptional and R = [|x|] sig with Z != 0, or one was and Z = 0 at the end.
+//  * sig in G2 (prime order r): before a doubling R = [k] sig with 2 <= 2k <= |x|, so Y = 0 would mean [2k] sig = O; before an
+//    addition R = [k] sig with k even, 2 <= k < |x|, so R = +-sig would mean [k -+ 1] sig = O with 1 <= k -+ 1 <= |x|.  |x| < r rules
+//    all of them out: Z != 0, R = [|x|] sig, and R = -psi(sig) holds in G2.  Accepted, as g2_in_subgroup accepts.
+//  * sig not in G2: with no exceptional step the comparison is g2_in_subgroup's on the same point, so the answers agree (rejected);
+//    after an exceptional step Z = 0 and the test rejects, which is again g2_in_subgroup's answer, since it accepts G2 points only.
+// The Z != 0 test and the comparisons come after all arithmetic and are combined without a branch (DESIGN "ptxas and carry chains").
+BLS_NOINLINE bool miller_end_in_subgroup(const g2_proj& r, const g2_aff& sig) {
+    g2_jac sj, ps; jac_from_aff(sj, sig); g2_psi(ps, sj);                // Z = 1: psi(sig) affine
+    fp2 px = fp2_mul(ps.X, r.z), py = fp2_mul(ps.Y, r.z);
+    return !fp2_is_zero(r.z) & fp2_eq(r.x, px) & fp2_eq(fp2_neg(r.y), py);
+}
 BLS_HD void miller_ell(fp12& f, const fp2& c0, const fp2& c1, const fp2& c2, const g1_aff& p) {
     fp12_mul_by_014(f, c0, fp2_mul_fp(c1, p.x), fp2_mul_fp(c2, p.y));
 }

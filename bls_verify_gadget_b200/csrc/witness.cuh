@@ -597,7 +597,7 @@ static int witness_run(blsgpu_ctx* ctx, const wit_prog& p, const uint8_t* pk48, 
     uint2* zbool_all = want_zbool ? ws_take<uint2>(ctx, groups * p.nvars) : nullptr;
     long long* sint_all = ws_take<long long>(ctx, groups * (p.n_islots + 1) * 32);
     LAUNCH(k_decode_g1, nblk(nkeys_total), TPB, dpk, nkeys_total, pk_soa, code_pk);
-    LAUNCH(k_decode_g2, nblk(nwit), TPB, dsig, nwit, sig_soa, code_sig);
+    LAUNCH(k_decode_g2<true>, nblk(nwit), TPB, dsig, nwit, sig_soa, code_sig);
     if (bitmap) LAUNCH(k_witness_inputs_agg, nblk(np), TPB, (const u32x4*)pk_soa, (const uint8_t*)code_pk, p.nkeys, dbm, (const u32x4*)sig_soa, (const uint8_t*)code_sig, dmsg, p.msg_len, nwit, np, inputs, dstatus);
     else LAUNCH(k_witness_inputs, nblk(np), TPB, (const u32x4*)pk_soa, (const uint8_t*)code_pk, (const u32x4*)sig_soa, (const uint8_t*)code_sig, dmsg, p.msg_len, nwit, np, inputs, dstatus);
     if (p.xrules && !want_zbool) return fail(ctx, BLSGPU_ERR_ARG, "the level-synchronous replay works on the packed 0/1 view");
