@@ -38,7 +38,7 @@ def lib():
 EXPORTS = ["blsgpu_create", "blsgpu_destroy", "blsgpu_last_error", "blsgpu_set_stream", "blsgpu_set_pointer_mode", "blsgpu_synchronize",
            "blsgpu_launch_count", "blsgpu_set_profiling", "blsgpu_stage_times", "blsgpu_set_chunk", "blsgpu_set_lanes", "blsgpu_set_split", "blsgpu_set_coop", "blsgpu_verify_batch", "blsgpu_verify_batch_rlc", "blsgpu_verify_batch_rlc_bisect", "blsgpu_fast_aggregate_verify_batch", "blsgpu_aggregate_verify_batch", "blsgpu_g1_uncompress", "blsgpu_g1_compress", "blsgpu_g2_uncompress", "blsgpu_g2_compress", "blsgpu_pool_create", "blsgpu_pool_free", "blsgpu_pool_fast_aggregate_verify", "blsgpu_hash_to_g2_batch", "blsgpu_g1_aggregate",
            "blsgpu_g2_aggregate", "blsgpu_deserialize_g1", "blsgpu_deserialize_g2", "blsgpu_sk_to_pk_batch", "blsgpu_sign_batch", "blsgpu_pairing_gt",
-           "blsgpu_gt_fold", "blsgpu_fp_mul_raw", "blsgpu_imad_peak", "blsgpu_r1cs_load", "blsgpu_r1cs_check", "blsgpu_r1cs_free", "blsgpu_r1cs_row_classes", "blsgpu_r1cs_load_file", "blsgpu_r1cs_check_file", "blsgpu_witness_load", "blsgpu_witness_gen", "blsgpu_witness_check", "blsgpu_witness_free", "blsgpu_witness_msg_len", "blsgpu_set_witness_mode", "blsgpu_witness_load_aggregate", "blsgpu_witness_shape", "blsgpu_witness_gen_aggregate", "blsgpu_witness_check_aggregate",
+           "blsgpu_gt_fold", "blsgpu_fp_mul_raw", "blsgpu_imad_peak", "blsgpu_r1cs_load", "blsgpu_r1cs_check", "blsgpu_r1cs_free", "blsgpu_r1cs_row_classes", "blsgpu_r1cs_load_file", "blsgpu_r1cs_check_file", "blsgpu_witness_load", "blsgpu_witness_gen", "blsgpu_witness_check", "blsgpu_witness_free", "blsgpu_witness_msg_len", "blsgpu_witness_load_aggregate", "blsgpu_witness_shape", "blsgpu_witness_gen_aggregate", "blsgpu_witness_check_aggregate",
            "blsgpu_create_multi", "blsgpu_destroy_multi", "blsgpu_multi_last_error", "blsgpu_multi_ndev", "blsgpu_multi_nccl_version", "blsgpu_multi_ctx", "blsgpu_multi_verify_batch", "blsgpu_multi_peek"]
 
 _sz = ctypes.c_size_t; _vp = ctypes.c_void_p
@@ -232,13 +232,13 @@ class Context:
         c = (ctypes.c_uint64 * 4)(); self._ck(lib().blsgpu_r1cs_row_classes(self._h, int(handle), c))
         return dict(zip(("truth_table", "generic", "long", "segments"), [int(x) for x in c]))
     # ---- GPU witness generation (program from bls_verify_gadget_b200.gadget.verify_program)
-    def witness_load(self, program, levels=True):
-        """program: the dict of gadget.verify_program; levels=False keeps the strictly sequential replay (one warp per 32 assignments)"""
+    def witness_load(self, program):
+        """program: the dict of gadget.verify_program (with its level order: the replay runs level by level)"""
         r = np.ascontiguousarray(program["rules16"], dtype=np.uint8); lp = np.ascontiguousarray(program["lc_ptr"], dtype=np.uint64)
         lc = np.ascontiguousarray(program["lc_col"], dtype=np.uint32); cf = np.ascontiguousarray(program["lc_coef48"], dtype=np.uint8)
-        od = np.ascontiguousarray(program["order"], dtype=np.uint32) if levels else None; lv = np.ascontiguousarray(program["level_ptr"], dtype=np.uint64) if levels else None
+        od = np.ascontiguousarray(program["order"], dtype=np.uint32); lv = np.ascontiguousarray(program["level_ptr"], dtype=np.uint64)
         h = ctypes.c_int(-1); nkeys = int(program.get("nkeys", 0))
-        args = (self._h, _p(r), _p(lp), _p(lc), _p(cf), _sz(r.size // 16), _sz(program["nvars"]), _sz(lp.size - 1), _sz(lc.size), _p(od), _p(lv), _sz(lv.size - 1 if levels else 0))
+        args = (self._h, _p(r), _p(lp), _p(lc), _p(cf), _sz(r.size // 16), _sz(program["nvars"]), _sz(lp.size - 1), _sz(lc.size), _p(od), _p(lv), _sz(lv.size - 1))
         if nkeys: self._ck(lib().blsgpu_witness_load_aggregate(*args, _sz(nkeys), ctypes.byref(h)))      # an aggregate_verify program (gadget.aggregate_verify_program)
         else: self._ck(lib().blsgpu_witness_load(*args, ctypes.byref(h)))
         return h.value
@@ -276,7 +276,6 @@ class Context:
         bits = np.zeros((n, words), np.uint64); allsat = np.zeros(n, np.uint8); st = np.empty(n, np.uint8)
         self._ck(lib().blsgpu_witness_check_aggregate(self._h, int(wit_handle), int(r1cs_handle), _p(pk), _p(bm), _p(m), _p(sg), _sz(n), _p(bits), _p(allsat), _p(st))); return bits, allsat, st
     def witness_free(self, handle): lib().blsgpu_witness_free(self._h, int(handle))
-    def set_witness_mode(self, cluster=True): self._ck(lib().blsgpu_set_witness_mode(self._h, 1 if cluster else 0))
 
 
 class MultiContext:

@@ -75,21 +75,6 @@ static inline unsigned nblk(size_t n, unsigned tpb = TPB) { return (unsigned)((n
 #define MILLER_LINE_STEPS 11       // most doubling + addition steps in 8 iterations (62..55 holds the additions of bits 62, 60, 57)
 #endif
 
-// Phase skew: the IMAD.WIDE pipe issues one warp instruction per 4 cycles per SM sub-partition and a single warp inside
-// fp_mul saturates it; two warps that start together stay in lockstep (both in their IMAD phase, then both in their ALU
-// phase), leaving each pipe idle half of the time.  Delaying every second warp of a sub-partition by about one phase at
-// kernel entry moves the pair to the stable anti-phase schedule.  BLS_SKEW = delay in cycles (0 = off).
-#ifndef BLS_F_IN_SMEM
-#define BLS_F_IN_SMEM 0
-#endif
-#ifndef BLS_SKEW
-#define BLS_SKEW 0
-#endif
-__device__ __forceinline__ void phase_skew() {
-#if BLS_SKEW > 0
-    if ((threadIdx.x >> 5) & 4) { long long t0 = clock64(); while (clock64() - t0 < BLS_SKEW) { } }
-#endif
-}
 // ================================================================================================ kernels
 __global__ void __launch_bounds__(TPB, BLS_MINB) k_fp_mul_raw(const fp* a, const fp* b, fp* out, size_t n, int reps) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
@@ -142,7 +127,6 @@ __global__ void __launch_bounds__(256) k_imad_peak(uint32_t* sink, int iters, in
 }
 
 __global__ void __launch_bounds__(TPB, BLS_MINB_DG1) k_decode_g1(const uint8_t* in48, size_t n, u32x4* soa, uint8_t* code) {
-    phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     g1_aff p; int rc = g1_decode(p, in48 + 48 * i);
     if (soa) soa_store_g1(soa, n, i, p);
@@ -150,7 +134,6 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_DG1) k_decode_g1(const uint8_t* 
 }
 // SUBGROUP = false: on-curve decode only, for blsgpu_verify_batch's split path, whose Miller loop tests membership (k_miller_lines)
 template <bool SUBGROUP> __global__ void __launch_bounds__(TPB, BLS_MINB_DG2) k_decode_g2(const uint8_t* in96, size_t n, u32x4* soa, uint8_t* code) {
-    phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     g2_aff p; int rc = g2_decode<SUBGROUP>(p, in96 + 96 * i);
     if (soa) soa_store_g2(soa, n, i, p);
@@ -159,7 +142,6 @@ template <bool SUBGROUP> __global__ void __launch_bounds__(TPB, BLS_MINB_DG2) k_
 // status/flags from the two decode codes (bls.rs:434-447), then H(m) for the items still alive
 __global__ void __launch_bounds__(TPB, BLS_MINB_HASH) k_hash_to_g2(const uint8_t* msg, const uint32_t* off, size_t n, const uint8_t* code_pk, const uint8_t* code_sig,
                                                     u32x4* hm_soa, uint8_t* flags, uint8_t* status) {
-    phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     uint8_t st = ST_OK, fl = 0;
     if (code_pk) {
@@ -223,17 +205,11 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_HCLEAR) k_hash_clear(const u32x4
 }
 __global__ void __launch_bounds__(TPB, BLS_MINB) k_miller(const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags,
                                                 const uint8_t* status, size_t n, u32x4* f_soa) {
-    phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     if (status[i] != ST_OK) return;
     g1_aff pk; g2_aff hm, sig;
     soa_load_g1(pk, pk_soa, n, i); soa_load_g2(hm, hm_soa, n, i); soa_load_g2(sig, sig_soa, n, i);
-#if BLS_F_IN_SMEM
-    extern __shared__ uint4 f_smem[];                       // accumulator f in shared memory, 592-byte stride (conflict-free 128-bit accesses)
-    fp12& f = *reinterpret_cast<fp12*>(f_smem + threadIdx.x * 37);
-#else
     fp12 f;
-#endif
     stage_miller(f, pk, hm, sig, flags[i]);
     soa_store_fp12(f_soa, n, i, f);
 }
@@ -344,7 +320,6 @@ __global__ void __launch_bounds__(TPB, BLS_MINB) k_miller_pairs(const u32x4* g1_
     soa_store_fp12(f_soa, nprod, i, f);
 }
 __global__ void __launch_bounds__(TPB, BLS_MINB) k_final_exp(u32x4* f_soa, const uint8_t* status_in, uint8_t* status_out, size_t n) {
-    phase_skew();
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     if (status_in[i] != ST_OK) { status_out[i] = status_in[i]; return; }
     fp12 f, gt; soa_load_fp12(f, f_soa, n, i);
@@ -683,7 +658,6 @@ struct blsgpu_ctx {
     uint8_t* rlc_acc;                   // accumulators of blsgpu_verify_batch_rlc that live across passes (allocated on first use)
     struct { u32x4* soa; uint8_t* code; size_t n; } pool[16];   // resident decoded validator pools
     int coop;                           // hard part of the final exponentiation with six lanes per item (coop.cuh): 0 = never, 1 = always, 2 (default) = for passes of at most VERIFY_COOP_BELOW items
-    int wit_cluster;                    // 1 = witness replay with one thread-block cluster per group of 32 assignments; 0 (default) = grid-wide level barrier
     int lanes; cudaStream_t lane_stream[4]; cudaEvent_t lane_done[4], fork;   // concurrent sub-ranges of a verify pass
     int split;                          // 1 (default) = hash-to-G2, Miller loop and final exponentiation as sequences of short specialised launches, 0 = one launch each
     size_t chunk;                       // items per internal pass of verify_batch (bounds the workspace); multiple of 64
@@ -770,7 +744,7 @@ int blsgpu_create(blsgpu_ctx** out, int device) {
     if (prop.major != 10) return BLSGPU_ERR_CUDA;                         // sm_100a cubin only: no other device can run it
     if (cudaSetDevice(device) != cudaSuccess) return BLSGPU_ERR_CUDA;
     blsgpu_ctx* c = new (std::nothrow) blsgpu_ctx(); if (!c) return BLSGPU_ERR_ALLOC;
-    memset(c, 0, sizeof *c); c->device = device; c->ptr_mode = BLSGPU_HOST; c->chunk = VERIFY_CHUNK_DEFAULT; c->lanes = 2; c->wit_cluster = 0; c->split = 1; c->coop = 2;
+    memset(c, 0, sizeof *c); c->device = device; c->ptr_mode = BLSGPU_HOST; c->chunk = VERIFY_CHUNK_DEFAULT; c->lanes = 2; c->split = 1; c->coop = 2;
     if (cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return BLSGPU_ERR_CUDA; }
     c->stream = c->own_stream;
     *out = c; return 0;
@@ -795,7 +769,6 @@ int blsgpu_set_pointer_mode(blsgpu_ctx* ctx, int mode) { if (!ctx || (mode != BL
 int blsgpu_synchronize(blsgpu_ctx* ctx) { if (!ctx) return BLSGPU_ERR_ARG; dev_guard guard_; CU(cudaSetDevice(ctx->device)); CU(cudaStreamSynchronize(ctx->stream)); return 0; }
 uint64_t blsgpu_launch_count(blsgpu_ctx* ctx) { return ctx ? ctx->launches : 0; }
 int blsgpu_set_coop(blsgpu_ctx* ctx, int on) { if (!ctx || on < 0 || on > 2) return BLSGPU_ERR_ARG; ctx->coop = on; return 0; }
-int blsgpu_set_witness_mode(blsgpu_ctx* ctx, int cluster) { if (!ctx) return BLSGPU_ERR_ARG; ctx->wit_cluster = cluster ? 1 : 0; return 0; }
 int blsgpu_set_split(blsgpu_ctx* ctx, int on) { if (!ctx) return BLSGPU_ERR_ARG; ctx->split = on ? 1 : 0; return 0; }
 int blsgpu_set_lanes(blsgpu_ctx* ctx, int lanes) { if (!ctx || lanes < 1 || lanes > 4) return BLSGPU_ERR_ARG; ctx->lanes = lanes; return 0; }
 int blsgpu_set_chunk(blsgpu_ctx* ctx, size_t items) { if (!ctx || items < 64 || (items & 63)) return BLSGPU_ERR_ARG; ctx->chunk = items; return 0; }
@@ -965,12 +938,7 @@ static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code
         if (int rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, n, f_soa, t_soa, lines, sig_sub, coop)) return rc;
         snap_soa = lines;                                      // 144 rows of the 396-row line buffer, which is dead once the loop ends
     } else {
-#if BLS_F_IN_SMEM
-    { static bool attr_set = false; if (!attr_set) { cudaFuncSetAttribute(k_miller, cudaFuncAttributeMaxDynamicSharedMemorySize, TPB * 592); attr_set = true; }
-      k_miller<<<nblk(n), TPB, TPB * 592, ctx->stream>>>(pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, n, f_soa); ctx->launches++; CU(cudaGetLastError()); }
-#else
-    LAUNCH(k_miller, nblk(n), TPB, pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, n, f_soa);
-#endif
+        LAUNCH(k_miller, nblk(n), TPB, pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, n, f_soa);
     }
     STAGE_MARK(4);
     if (coop) {

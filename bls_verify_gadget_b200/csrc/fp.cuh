@@ -538,19 +538,12 @@ BLS_NOINLINE fp fp_inv_raw(const fp& x) {
     for (int i = 0; i < 6; i++) { r.l[2 * i] = (uint32_t)w[i]; r.l[2 * i + 1] = (uint32_t)(w[i] >> 32); }
     return r;
 }
-#ifndef BLS_INV_GCD
-#define BLS_INV_GCD 1
-#endif
 // Montgomery form in and out: (aR)^-1 R^3 R^-1 = a^-1 R
 BLS_HD fp fp_inv(const fp& a) {
-#if BLS_INV_GCD
     const uint32_t O[12] = BLS_C_R3; fp r3;
 #pragma unroll
     for (int i = 0; i < 12; i++) r3.l[i] = O[i];
     return fp_mul(fp_inv_raw(a), r3);
-#else
-    return fp_inv_fermat(a);
-#endif
 }
 // t = a^((p-3)/4).  Then a*t = a^((p+1)/4) is the candidate square root and (a*t)*t = a^((p-1)/2) the Legendre symbol.
 BLS_HD fp fp_pow_pm3d4(const fp& a) { return fp_pow(a, EXP_P_MINUS_3_DIV_4, 12); }

@@ -11,21 +11,8 @@ struct fp2 { fp c0, c1; };
 
 BLS_HD fp2 fp2_zero() { fp2 r; r.c0 = fp_zero(); r.c1 = fp_zero(); return r; }
 BLS_HD fp2 fp2_one() { fp2 r; r.c0 = fp_one(); r.c1 = fp_zero(); return r; }
-#ifndef BLS_FP2_ADDSUB_OUTOFLINE
-#define BLS_FP2_ADDSUB_OUTOFLINE 0
-#endif
-#if BLS_FP2_ADDSUB_OUTOFLINE == 2 && defined(__CUDACC__)
-BLS_NOINLINE fp2 fp2_add(fp2 a, fp2 b) { fp2 r; r.c0 = fp_add(a.c0, b.c0); r.c1 = fp_add(a.c1, b.c1); return r; }
-BLS_NOINLINE fp2 fp2_sub(fp2 a, fp2 b) { fp2 r; r.c0 = fp_sub(a.c0, b.c0); r.c1 = fp_sub(a.c1, b.c1); return r; }
-#elif BLS_FP2_ADDSUB_OUTOFLINE == 1
-BLS_NOINLINE void fp2_add_p(fp2& r, const fp2& a, const fp2& b);
-BLS_NOINLINE void fp2_sub_p(fp2& r, const fp2& a, const fp2& b);
-BLS_HD fp2 fp2_add(const fp2& a, const fp2& b) { fp2 r; fp2_add_p(r, a, b); return r; }
-BLS_HD fp2 fp2_sub(const fp2& a, const fp2& b) { fp2 r; fp2_sub_p(r, a, b); return r; }
-#else
 BLS_HD fp2 fp2_add(const fp2& a, const fp2& b) { fp2 r; r.c0 = fp_add(a.c0, b.c0); r.c1 = fp_add(a.c1, b.c1); return r; }
 BLS_HD fp2 fp2_sub(const fp2& a, const fp2& b) { fp2 r; r.c0 = fp_sub(a.c0, b.c0); r.c1 = fp_sub(a.c1, b.c1); return r; }
-#endif
 BLS_HD fp2 fp2_dbl(const fp2& a) { return fp2_add(a, a); }
 BLS_HD fp2 fp2_half(const fp2& a) { fp2 r; r.c0 = fp_half(a.c0); r.c1 = fp_half(a.c1); return r; }
 BLS_HD fp2 fp2_neg(const fp2& a) { fp2 r; r.c0 = fp_neg(a.c0); r.c1 = fp_neg(a.c1); return r; }
@@ -35,84 +22,18 @@ BLS_HD fp2 fp2_mul_u(const fp2& a) { fp2 r; r.c0 = fp_neg(a.c1); r.c1 = a.c0; re
 BLS_HD bool fp2_is_zero(const fp2& a) { return fp_is_zero(a.c0) & fp_is_zero(a.c1); }
 BLS_HD bool fp2_eq(const fp2& a, const fp2& b) { return fp_eq(a.c0, b.c0) & fp_eq(a.c1, b.c1); }
 BLS_HD fp2 fp2_csel(bool c, const fp2& a, const fp2& b) { fp2 r; r.c0 = fp_csel(c, a.c0, b.c0); r.c1 = fp_csel(c, a.c1, b.c1); return r; }
-// Out-of-line arithmetic works memory-to-memory (operands by reference in the thread's local memory, staged with
-// 128-bit loads/stores): nothing is live in registers across a call, so the 300-IMAD cores exist once in the
-// instruction cache and the callers stay small.  BLS_FP2_MODE selects what is inlined inside fp2_mul/fp2_sqr:
-//   0 = calls to the out-of-line fp_mul/fp_sqr, 1 = the three (two) Montgomery products inlined (18 / 12 KB bodies),
-//   2 = by-value register ABI (no memory staging); measured fastest on B200 (profiles/r01_tuning.md)
-#ifndef BLS_FP2_MODE
-#define BLS_FP2_MODE 2
-#endif
-#if BLS_FP2_MODE == 1
-#define BLS_FPM fp_mul_inl
-#else
-#define BLS_FPM fp_mul
-#endif
-BLS_NOINLINE void fp2_mul_p(fp2& r, const fp2& a, const fp2& b) {   // Karatsuba: 3 products
-    fp a0 = a.c0, a1 = a.c1, b0 = b.c0, b1 = b.c1;
-#if BLS_FP2_LAZY
-    { fpw T0, T1, T2; fp_mul_wide(T0, a0, b0); fp_mul_wide(T1, a1, b1);
-      fp sa, sb; fp_add_raw(sa, a0, a1); fp_add_raw(sb, b0, b1); fp_mul_wide(T2, sa, sb);
-      fpw_sub(T2, T2, T0); fpw_sub(T2, T2, T1); fpw_sub(T0, T0, T1); fpw_add(T0, T0, fpw_p_squared());
-      r.c0 = fp_redc_wide(T0); r.c1 = fp_redc_wide(T2); return; }
-#endif
-    fp t0 = BLS_FPM(a0, b0), t1 = BLS_FPM(a1, b1);
-    fp t2 = BLS_FPM(fp_add(a0, a1), fp_add(b0, b1));
-    r.c0 = fp_sub(t0, t1); r.c1 = fp_sub(fp_sub(t2, t0), t1);
-}
-BLS_NOINLINE void fp2_sqr_p(fp2& r, const fp2& a) {                 // 2 products
-    fp a0 = a.c0, a1 = a.c1;
-    fp t = BLS_FPM(a0, a1);
-    r.c0 = BLS_FPM(fp_add(a0, a1), fp_sub(a0, a1)); r.c1 = fp_add(t, t);
-}
-BLS_NOINLINE void fp2_mul_fp_p(fp2& r, const fp2& a, const fp& s) {
-    fp a0 = a.c0, a1 = a.c1, ss = s;
-    r.c0 = BLS_FPM(a0, ss); r.c1 = BLS_FPM(a1, ss);
-}
-#ifndef BLS_FP2_LAZY
-#define BLS_FP2_LAZY 0
-#endif
-#if BLS_FP2_MODE >= 2 && defined(__CUDACC__)
-// mode 2: operands and results by value in registers, three (two) calls to the out-of-line fp_mul
-// mode 3: the same with the Montgomery products inlined, so the additions can be scheduled into the IMAD stream
-#if BLS_FP2_MODE == 3
-#define BLS_FPM2 fp_mul_inl
-#else
-#define BLS_FPM2 fp_mul
-#endif
-#if BLS_FP2_LAZY
-// Lazy reduction: three unreduced 768-bit products, double-width Karatsuba recombination, two Montgomery reductions
-// (744 IMAD.WIDE instead of 900).  c1 = T2 - T0 - T1 >= 0; c0 = T0 - T1 + p^2 in (0, 2p^2) < p 2^384.
-BLS_NOINLINE fp2 fp2_mul(fp2 a, fp2 b) {
-    fpw T0, T1, T2;
-    fp_mul_wide(T0, a.c0, b.c0); fp_mul_wide(T1, a.c1, b.c1);
-    fp sa, sb; fp_add_raw(sa, a.c0, a.c1); fp_add_raw(sb, b.c0, b.c1);          // < 2p < 2^382: no reduction needed
-    fp_mul_wide(T2, sa, sb);
-    fpw_sub(T2, T2, T0); fpw_sub(T2, T2, T1);
-    fpw_sub(T0, T0, T1); fpw_add(T0, T0, fpw_p_squared());
-    fp2 r; r.c0 = fp_redc_wide(T0); r.c1 = fp_redc_wide(T2); return r;
-}
-#else
-BLS_NOINLINE fp2 fp2_mul(fp2 a, fp2 b) {
-    fp t0 = BLS_FPM2(a.c0, b.c0), t1 = BLS_FPM2(a.c1, b.c1);
-    fp t2 = BLS_FPM2(fp_add(a.c0, a.c1), fp_add(b.c0, b.c1));
+// Operands and results by value, three (two) calls to the out-of-line fp_mul: measured faster on B200 than memory-to-memory
+// operands, than inlined Montgomery products and than a lazily reduced Karatsuba form (profiles/r01_tuning.md).
+BLS_NOINLINE fp2 fp2_mul(fp2 a, fp2 b) {                           // Karatsuba: 3 products
+    fp t0 = fp_mul(a.c0, b.c0), t1 = fp_mul(a.c1, b.c1);
+    fp t2 = fp_mul(fp_add(a.c0, a.c1), fp_add(b.c0, b.c1));
     fp2 r; r.c0 = fp_sub(t0, t1); r.c1 = fp_sub(t2, fp_add(t0, t1)); return r;
 }
-#endif
-BLS_NOINLINE fp2 fp2_sqr(fp2 a) {
-    fp t = BLS_FPM2(a.c0, a.c1);
-    fp2 r; r.c0 = BLS_FPM2(fp_add(a.c0, a.c1), fp_sub(a.c0, a.c1)); r.c1 = fp_add(t, t); return r;
+BLS_NOINLINE fp2 fp2_sqr(fp2 a) {                                  // 2 products
+    fp t = fp_mul(a.c0, a.c1);
+    fp2 r; r.c0 = fp_mul(fp_add(a.c0, a.c1), fp_sub(a.c0, a.c1)); r.c1 = fp_add(t, t); return r;
 }
 BLS_HD fp2 fp2_mul_fp(const fp2& a, const fp& s) { fp2 r; r.c0 = fp_mul(a.c0, s); r.c1 = fp_mul(a.c1, s); return r; }
-#else
-BLS_HD fp2 fp2_mul(const fp2& a, const fp2& b) { fp2 r; fp2_mul_p(r, a, b); return r; }
-BLS_HD fp2 fp2_sqr(const fp2& a) { fp2 r; fp2_sqr_p(r, a); return r; }
-BLS_HD fp2 fp2_mul_fp(const fp2& a, const fp& s) { fp2 r; fp2_mul_fp_p(r, a, s); return r; }
-#endif
-#if BLS_FP2_ADDSUB_OUTOFLINE == 1
-BLS_NOINLINE void fp2_add_p(fp2& r, const fp2& a, const fp2& b) { fp x0 = a.c0, x1 = a.c1, y0 = b.c0, y1 = b.c1; r.c0 = fp_add(x0, y0); r.c1 = fp_add(x1, y1); }
-BLS_NOINLINE void fp2_sub_p(fp2& r, const fp2& a, const fp2& b) { fp x0 = a.c0, x1 = a.c1, y0 = b.c0, y1 = b.c1; r.c0 = fp_sub(x0, y0); r.c1 = fp_sub(x1, y1); }
-#endif
 
 BLS_HD fp fp2_norm(const fp2& a) { return fp_add(fp_sqr(a.c0), fp_sqr(a.c1)); }
 BLS_HD fp2 fp2_inv(const fp2& a) {                            // 0 -> 0

@@ -176,11 +176,7 @@ template <class LOAD> BLS_HD void fp12_decompress_product_from(fp12& r, LOAD loa
     }
     r = acc;
 }
-#ifndef BLS_KARABINA
-#define BLS_KARABINA 1
-#endif
 BLS_NOINLINE void fp12_exp_by_x(fp12& r, const fp12& a) {
-#if BLS_KARABINA
     fp12c c, snap[6]; fp12_compress(c, a);
     const uint64_t x = BLS_X_ABS; int k = 0;
     for (int i = 1; i <= 63; i++) {
@@ -189,9 +185,6 @@ BLS_NOINLINE void fp12_exp_by_x(fp12& r, const fp12& a) {
     }
     fp12 acc; fp12_decompress_product(acc, snap, 6);
     fp12_conj(r, acc);
-#else
-    fp12_exp_by_x_gs(r, a);
-#endif
 }
 // f^(3 (p^12 - 1)/r): the exact chain of ark-ec's Bls12::final_exponentiation
 BLS_NOINLINE void final_exponentiation(fp12& r, const fp12& f) {

@@ -15,11 +15,11 @@
 //    side sum, a larger coefficient as a masked addition of its canonical value (warp-uniform branches), and test a row that
 //    touched nothing else as a * b == c on integers;
 //  * a few hundred rows carry 300-760 general coefficients (linear combinations that grow through runs of cyclotomic
-//    squarings).  Round 1 cut rows longer than R1_LONG into R1_SEG-entry segments, one warp each, and combined them afterwards
+//    squarings).  Round 1 cut rows longer than R1_LONG into 32-entry segments, one warp each, and combined them afterwards
 //    (with the round-1 term code a 760-term row serialised ~10^7 instructions on one warp: 34 ms per group).  With the term paths of
-//    round 2 a term costs ~70 warp instructions, and the long rows run one warp per ROW again, longest first (k_r1cs_long_rows):
+//    round 2 a term costs ~70 warp instructions, and the long rows run one warp per ROW, longest first (k_r1cs_long_rows):
 //    no partial sums through global memory, one closing reduction per combination instead of one per segment -- 651 -> 506 us per
-//    group for the 21,537 long rows of the verify circuit.  The segment kernels stay behind R1_LONG_ROWS = 0.
+//    group for the 21,537 long rows of the verify circuit.
 // Coefficients +1 / -1 (the bulk of boolean/uint gadget rows) skip the multiply; coefficients of magnitude below 2^32 (2, 3, 4, 12,
 // 2^k ...: 80 % of the remaining ones in the verify circuit) take fp_mul_small (24 MACs); z stays canonical:
 // coeff(Montgomery) x z(canonical) -> canonical, no conversion of z needed.
@@ -30,11 +30,9 @@
 struct r1cs_sys {
     size_t nrows, ncols, nnz[3];
     uint64_t* rowptr[3]; uint32_t* col[3]; fp* coeff[3]; fp* coeffc[3]; uint8_t* cls[3];
-    uint8_t* is_long; size_t n_long, n_seg;
-    uint32_t* long_row;            // [n_long] row index
-    uint32_t* long_sorted;         // [n_long] the same rows, longest first (k_r1cs_long_rows takes them in this order: longest-processing-time-first over the warps)
-    uint32_t* seg_ptr;             // [n_long * 3 + 1] first segment of (long row, matrix)
-    uint64_t* seg_lo; uint64_t* seg_hi; uint8_t* seg_mat;     // [n_seg] non-zero range and matrix of a segment
+    size_t n_long;
+    size_t n_rounds;               // 32-term metadata rounds k_r1cs_long_rows walks: sum over long rows and matrices of ceil(nnz / 32)
+    uint32_t* long_sorted;         // [n_long] long rows, longest first (k_r1cs_long_rows takes them in this order: longest-processing-time-first over the warps)
     // rows specialised at load time (see "row classes" below)
     uint4* lut_a; uint2* lut_b;    // [nrows] truth-table rows: (col0 | need_b << 31, col1, col2, table) and (col3, col4); col0 = R1_NOT_LUT for other rows
     uint32_t* gen_rows; size_t n_gen, n_lut;     // short rows that are evaluated term by term (lane = assignment)
@@ -45,9 +43,6 @@ enum { R1_GENERAL = 0, R1_PLUS_ONE = 1, R1_MINUS_ONE = 2, R1_SMALL_POS = 3, R1_S
 #ifndef R1_LONG
 #define R1_LONG 8          // rows that are not truth-table rows and have more non-zeros than this take the lane-parallel metadata path (k_r1cs_long_rows);
 #endif                     // measured on the verify circuit: 16 -> 3.67 ms per 128 assignments, 8 / 4 / 2 -> 3.54 / 3.55 / 3.54
-#ifndef R1_SEG
-#define R1_SEG 32
-#endif
 // The row kernels are bound by the latency of the z gather (1.5 KB per non-zero and 32 witnesses, from HBM: a group's
 // transposed z is 1 GB), not by registers: more resident warps than the pairing kernels' 8 per SM
 #ifndef R1_MINB
@@ -110,7 +105,7 @@ __device__ __forceinline__ fp r1cs_load_z(const u32x4* zt, uint32_t col, int lan
 }
 // One non-zero: class c, column cj with its packed 0/1 view zb, |coefficient| low word cf (small classes).  Every branch is
 // warp-uniform (class per non-zero, zbool per column).  Terms on 0/1 columns with coefficient +-1 or |c| < 2^32 go to the integer
-// side sum (at most R1_SEG terms: |sum| < 2^39); `touched` records whether the field accumulator was used at all.
+// side sum (|term| < 2^32: no overflow below 2^31 terms); `touched` records whether the field accumulator was used at all.
 // Terms on field-valued columns with coefficient +-1 or |c| < 2^32 go to the LAZY 14-limb sum `la` (fp_lacc_*: 12 IMAD.WIDE per term, one
 // Barrett reduction per range instead of one per term; a negative coefficient enters as |c| (p - z)).
 __device__ __forceinline__ void r1cs_term(const r1cs_sys& s, int m, uint64_t k, uint32_t cj, uint32_t c, uint2 zb, uint32_t cf, const u32x4* zt, int lane,
@@ -139,7 +134,7 @@ __device__ __forceinline__ void r1cs_term(const r1cs_sys& s, int m, uint64_t k, 
     else if (c == R1_SMALL_POS) fp_lacc_mad(la, zv, cf);
     else { fp nz; fp_sub_raw(nz, fp_modulus(), zv); fp_lacc_mad(la, nz, c == R1_MINUS_ONE ? 1u : BLS_P0 - cf); }      // z = 0 enters as |c| p = 0 (mod p)
 }
-// sum over the non-zeros [lo, hi) of one matrix (a segment of a long row): field part returned, integer part in side_out
+// sum over the non-zeros [lo, hi) of one matrix: field part returned, integer part in side_out
 __device__ __forceinline__ fp r1cs_range_dot(const r1cs_sys& s, int m, uint64_t lo, uint64_t hi, const u32x4* zt, const uint2* zbool, int lane, int64_t& side_out, bool& touched) {
     const uint32_t* col = s.col[m]; const uint8_t* cls = s.cls[m];
     fp acc = fp_zero(); int64_t side = 0; touched = false;
@@ -157,9 +152,8 @@ __device__ __forceinline__ fp r1cs_range_dot(const r1cs_sys& s, int m, uint64_t 
 }
 // The same sum with the terms' metadata fetched LANE-PARALLEL: lane t loads column, class, packed view and small coefficient of term
 // lo + t (two dependent rounds of independent loads for up to 32 terms), then the terms are evaluated from register broadcasts.  The
-// term-by-term walk above chains column -> packed view (-> gather) per term: fine for the 7-term short rows, but a 32-entry segment of
-// a long row (k_r1cs_segments: long-scoreboard stalls were 36 % of its samples) and the latency-bound witness replay pay that
-// latency once per term.  All 32 lanes must call it together.
+// term-by-term walk above chains column -> packed view (-> gather) per term: fine for the 7-term short rows, but a long row (long-scoreboard
+// stalls were 36 % of the samples of the round-1 segment kernel) and the latency-bound witness replay pay that latency once per term.  All 32 lanes must call it together.
 // metadata of up to 32 consecutive non-zeros, one per lane
 struct r1cs_meta { uint32_t col, c, cf, n; uint2 zb; uint64_t base; };
 __device__ __forceinline__ void r1cs_meta_fetch(r1cs_meta& t, const r1cs_sys& s, int m, uint64_t lo, uint64_t hi, int lane) {       // round 1: column, class, small coefficient
@@ -307,47 +301,26 @@ __global__ void __launch_bounds__(256) k_r1cs_lut(r1cs_sys s, const uint2* zbool
 #ifndef R1_MINB_ROWS
 #define R1_MINB_ROWS R1_MINB
 #endif
-#ifndef R1_ROWS_WIDE
-#define R1_ROWS_WIDE 0          // overlapped metadata rounds in the listed-row kernel: measured equal (4.26 vs 4.23 ms per 128 assignments), off
-#endif
-#ifndef R1_MINB_SEG
-#define R1_MINB_SEG R1_MINB
-#endif
 __global__ void __launch_bounds__(TPB, R1_MINB_ROWS) k_r1cs_rows_list(r1cs_sys s, const u32x4* zt, const uint2* zbool, size_t w0, size_t g, size_t words, uint64_t* sat_bits) {
     size_t warp = blockIdx.x * (size_t)(TPB / 32) + (threadIdx.x >> 5), nwarps = gridDim.x * (size_t)(TPB / 32); int lane = threadIdx.x & 31;
     size_t n = s.n_gen + (size_t)*s.fb_count;
     for (size_t i = warp; i < n; i += nwarps) {
         size_t row = i < s.n_gen ? s.gen_rows[i] : s.fb_rows[i - s.n_gen];
         int64_t sa, sb, sc; bool ta, tb, tc;
-#if R1_ROWS_WIDE
-        // the three combinations' metadata in overlapped rounds (a listed row has at most 16 non-zeros): rows, then columns / classes, then packed views
-        uint64_t lo0 = s.rowptr[0][row], hi0 = s.rowptr[0][row + 1], lo1 = s.rowptr[1][row], hi1 = s.rowptr[1][row + 1], lo2 = s.rowptr[2][row], hi2 = s.rowptr[2][row + 1];
-        r1cs_meta m0, m1, m2;
-        r1cs_meta_fetch(m0, s, 0, lo0, hi0, lane); r1cs_meta_fetch(m1, s, 1, lo1, hi1, lane); r1cs_meta_fetch(m2, s, 2, lo2, hi2, lane);
-        r1cs_meta_views(m0, zbool, lane); r1cs_meta_views(m1, zbool, lane); r1cs_meta_views(m2, zbool, lane);
-        r1cs_accum ac; fp a, b, c;
-        r1cs_accum_zero(ac); r1cs_meta_eval<1>(m0, s, 0, zt, lane, ac); a = r1cs_accum_close(ac, sa, ta);
-        r1cs_accum_zero(ac); r1cs_meta_eval<1>(m1, s, 1, zt, lane, ac); b = r1cs_accum_close(ac, sb, tb);
-        r1cs_accum_zero(ac); r1cs_meta_eval<1>(m2, s, 2, zt, lane, ac); c = r1cs_accum_close(ac, sc, tc);
-#else
         fp a = r1cs_range_dot(s, 0, s.rowptr[0][row], s.rowptr[0][row + 1], zt, zbool, lane, sa, ta);
         fp b = r1cs_range_dot(s, 1, s.rowptr[1][row], s.rowptr[1][row + 1], zt, zbool, lane, sb, tb);
         fp c = r1cs_range_dot(s, 2, s.rowptr[2][row], s.rowptr[2][row + 1], zt, zbool, lane, sc, tc);
-#endif
         bool ok;
         if (!(ta | tb | tc)) ok = (__int128)sa * (__int128)sb == (__int128)sc;      // only 0/1 columns with small coefficients: |a b - c| < 2^80 < p, so equality mod p is equality
         else ok = r1cs_product_ok(r1cs_finalize(a, sa, ta), r1cs_finalize(b, sb, tb), r1cs_finalize(c, sc, tc));
         if ((size_t)lane < g && ok) atomicOr((unsigned long long*)&sat_bits[(w0 + lane) * words + (row >> 6)], 1ull << (row & 63));
     }
 }
-// one warp per long row, longest rows first: the three combinations through the lane-parallel metadata path, product test, bit.  Replaces the
-// segment + combine pair (R1_LONG_ROWS): no partial sums through global memory (301 MB per launch), one closing reduction per combination
+// one warp per long row, longest rows first: the three combinations through the lane-parallel metadata path, product test, bit.  Replaced
+// round 1's segment + combine pair: no partial sums through global memory (301 MB per launch), one closing reduction per combination
 // instead of one per 32-term segment (5.4 segments per long row on the verify circuit).
-#ifndef R1_LONG_ROWS
-#define R1_LONG_ROWS 1
-#endif
 #ifndef R1_MINB_LONG
-#define R1_MINB_LONG R1_MINB_SEG
+#define R1_MINB_LONG R1_MINB
 #endif
 __global__ void __launch_bounds__(TPB, R1_MINB_LONG) k_r1cs_long_rows(r1cs_sys s, const u32x4* zt, const uint2* zbool, size_t w0, size_t g, size_t words, uint64_t* sat_bits) {
     size_t li = blockIdx.x * (size_t)(TPB / 32) + (threadIdx.x >> 5); int lane = threadIdx.x & 31;
@@ -358,29 +331,6 @@ __global__ void __launch_bounds__(TPB, R1_MINB_LONG) k_r1cs_long_rows(r1cs_sys s
     fp b = r1cs_range_dot_wide(s, 1, s.rowptr[1][row], s.rowptr[1][row + 1], zt, zbool, lane, sb, tb); b = r1cs_finalize(b, sb, tb);
     fp c = r1cs_range_dot_wide(s, 2, s.rowptr[2][row], s.rowptr[2][row + 1], zt, zbool, lane, sc, tc); c = r1cs_finalize(c, sc, tc);
     bool ok = r1cs_product_ok(a, b, c);
-    if ((size_t)lane < g && ok) atomicOr((unsigned long long*)&sat_bits[(w0 + lane) * words + (row >> 6)], 1ull << (row & 63));
-}
-// one warp per segment of a long row: partial dot product of 32 witnesses -> part (limb-SoA over n_seg * 32 slots)
-__global__ void __launch_bounds__(TPB, R1_MINB_SEG) k_r1cs_segments(r1cs_sys s, const u32x4* zt, const uint2* zbool, u32x4* part) {
-    size_t sg = blockIdx.x * (size_t)(TPB / 32) + (threadIdx.x >> 5); int lane = threadIdx.x & 31;
-    if (sg >= s.n_seg) return;
-    int64_t side; bool touched;
-    fp v = r1cs_range_dot_wide(s, s.seg_mat[sg], s.seg_lo[sg], s.seg_hi[sg], zt, zbool, lane, side, touched);
-    v = r1cs_finalize(v, side, touched);
-    soa_store_fp(part, s.n_seg * 32, sg * 32 + lane, 0, v);
-}
-// one warp per long row: add the partial sums of each matrix, test the product, OR the bit into the row's word
-__global__ void __launch_bounds__(TPB, R1_MINB) k_r1cs_combine(r1cs_sys s, const u32x4* part, size_t w0, size_t g, size_t words, uint64_t* sat_bits) {
-    size_t li = blockIdx.x * (size_t)(TPB / 32) + (threadIdx.x >> 5); int lane = threadIdx.x & 31;
-    if (li >= s.n_long) return;
-    fp v[3];
-    for (int m = 0; m < 3; m++) {
-        fp acc = fp_zero();
-        for (uint32_t sg = s.seg_ptr[li * 3 + m]; sg < s.seg_ptr[li * 3 + m + 1]; sg++) acc = fp_add(acc, soa_load_fp(part, s.n_seg * 32, (size_t)sg * 32 + lane, 0));
-        v[m] = acc;
-    }
-    size_t row = s.long_row[li];
-    bool ok = r1cs_product_ok(v[0], v[1], v[2]);            // all 32 lanes take part in the vote inside; only the store is masked
     if ((size_t)lane < g && ok) atomicOr((unsigned long long*)&sat_bits[(w0 + lane) * words + (row >> 6)], 1ull << (row & 63));
 }
 // one warp per assignment: AND over its bit words (coalesced), lane 0 writes the flag
@@ -404,7 +354,7 @@ template <class T> static int r1cs_upload(blsgpu_ctx* ctx, T** dst, const std::v
 }
 static void r1cs_release(r1cs_sys* s) {
     for (int m = 0; m < 3; m++) { cudaFree(s->rowptr[m]); cudaFree(s->col[m]); cudaFree(s->coeff[m]); cudaFree(s->coeffc[m]); cudaFree(s->cls[m]); }
-    cudaFree(s->is_long); cudaFree(s->long_row); cudaFree(s->long_sorted); cudaFree(s->seg_ptr); cudaFree(s->seg_lo); cudaFree(s->seg_hi); cudaFree(s->seg_mat);
+    cudaFree(s->long_sorted);
     cudaFree(s->lut_a); cudaFree(s->lut_b); cudaFree(s->gen_rows); cudaFree(s->fb_rows); cudaFree(s->fb_count);
     delete s;
 }
@@ -436,8 +386,8 @@ static int r1cs_build(blsgpu_ctx* ctx, r1cs_sys* s, const uint64_t* const rowptr
             CU(cudaStreamSynchronize(ctx->stream));
         }
     }
-    // row classes: long rows with their segments, truth-table rows, generic short rows
-    std::vector<uint8_t> is_long(nrows, 0), seg_mat; std::vector<uint32_t> long_row, seg_ptr, gen_rows, lut_rows; std::vector<uint64_t> seg_lo, seg_hi;
+    // row classes: truth-table rows, long rows, generic short rows
+    std::vector<uint32_t> long_row, gen_rows, lut_rows; size_t n_rounds = 0;
     std::vector<uint4> lut_a(nrows); std::vector<uint2> lut_b(nrows);
     for (size_t r = 0; r < nrows; r++) {
         lut_a[r] = make_uint4(R1_NOT_LUT, R1_NO_COL, R1_NO_COL, 0u); lut_b[r] = make_uint2(R1_NO_COL, R1_NO_COL);
@@ -454,25 +404,14 @@ static int r1cs_build(blsgpu_ctx* ctx, r1cs_sys* s, const uint64_t* const rowptr
             lut_b[r] = make_uint2(d > 3 ? c[3] : R1_NO_COL, d > 4 ? c[4] : R1_NO_COL);
             lut_rows.push_back((uint32_t)r);
         } else if (len > R1_LONG) {
-            is_long[r] = 1; long_row.push_back((uint32_t)r);
-            for (int m = 0; m < 3; m++) {
-                seg_ptr.push_back((uint32_t)seg_lo.size());
-                for (uint64_t k = hrp[m][r]; k < hrp[m][r + 1]; k += R1_SEG) { seg_lo.push_back(k); seg_hi.push_back(k + R1_SEG < hrp[m][r + 1] ? k + R1_SEG : hrp[m][r + 1]); seg_mat.push_back((uint8_t)m); }
-            }
+            long_row.push_back((uint32_t)r);
+            for (int m = 0; m < 3; m++) n_rounds += (hrp[m][r + 1] - hrp[m][r] + 31) / 32;
         } else gen_rows.push_back((uint32_t)r);
     }
-    seg_ptr.push_back((uint32_t)seg_lo.size());
-    s->n_long = long_row.size(); s->n_seg = seg_lo.size(); s->n_gen = gen_rows.size(); s->n_lut = lut_rows.size();
-    if (int rc = r1cs_upload(ctx, &s->is_long, is_long)) return rc;
-    if (int rc = r1cs_upload(ctx, &s->long_row, long_row)) return rc;
-    {   std::vector<uint32_t> ls = long_row;
-        auto len_of = [&](uint32_t r) { size_t l = 0; for (int m = 0; m < 3; m++) l += hrp[m][r + 1] - hrp[m][r]; return l; };
-        std::stable_sort(ls.begin(), ls.end(), [&](uint32_t x, uint32_t y) { return len_of(x) > len_of(y); });
-        if (int rc = r1cs_upload(ctx, &s->long_sorted, ls)) return rc; }
-    if (int rc = r1cs_upload(ctx, &s->seg_ptr, seg_ptr)) return rc;
-    if (int rc = r1cs_upload(ctx, &s->seg_lo, seg_lo)) return rc;
-    if (int rc = r1cs_upload(ctx, &s->seg_hi, seg_hi)) return rc;
-    if (int rc = r1cs_upload(ctx, &s->seg_mat, seg_mat)) return rc;
+    s->n_long = long_row.size(); s->n_rounds = n_rounds; s->n_gen = gen_rows.size(); s->n_lut = lut_rows.size();
+    {   auto len_of = [&](uint32_t r) { size_t l = 0; for (int m = 0; m < 3; m++) l += hrp[m][r + 1] - hrp[m][r]; return l; };
+        std::stable_sort(long_row.begin(), long_row.end(), [&](uint32_t x, uint32_t y) { return len_of(x) > len_of(y); });
+        if (int rc = r1cs_upload(ctx, &s->long_sorted, long_row)) return rc; }
     if (int rc = r1cs_upload(ctx, &s->lut_a, lut_a)) return rc;
     if (int rc = r1cs_upload(ctx, &s->lut_b, lut_b)) return rc;
     if (int rc = r1cs_upload(ctx, &s->gen_rows, gen_rows)) return rc;
@@ -559,30 +498,23 @@ int blsgpu_r1cs_check_file(blsgpu_ctx* ctx, int handle, const char* path, size_t
     return rc;
 }
 }
-// rows per class of a loaded system: counts[0] truth-table rows, [1] generic short rows, [2] long rows, [3] segments of the long rows
+// rows per class of a loaded system: counts[0] truth-table rows, [1] generic short rows, [2] long rows, [3] 32-term metadata rounds
+// k_r1cs_long_rows walks (sum over long rows and matrices of ceil(nnz / 32))
 int blsgpu_r1cs_row_classes(blsgpu_ctx* ctx, int handle, uint64_t counts[4]) {
     if (!ctx || handle < 0 || handle >= 16 || !ctx->r1cs[handle] || !counts) return BLSGPU_ERR_ARG;
-    const r1cs_sys* s = ctx->r1cs[handle]; counts[0] = s->n_lut; counts[1] = s->n_gen; counts[2] = s->n_long; counts[3] = s->n_seg; return 0;
+    const r1cs_sys* s = ctx->r1cs[handle]; counts[0] = s->n_lut; counts[1] = s->n_gen; counts[2] = s->n_long; counts[3] = s->n_rounds; return 0;
 }
 }
 // one group of <= 32 assignments given in the transposed layout (zt, zbool): truth-table rows first (plain stores: this initialises
-// the group's slice of the output), then the rows that fell back, the generic short rows, and the long rows' segments + combination
+// the group's slice of the output), then the rows that fell back, the generic short rows, and the long rows
 #ifndef R1_FB_BLOCKS
 #define R1_FB_BLOCKS 888          // 148 SMs x 6 resident CTAs: one grid-stride pass over both lists
 #endif
-static int r1cs_check_group(blsgpu_ctx* ctx, const r1cs_sys& s, const u32x4* zt, const uint2* zbool, u32x4* part, size_t w0, size_t g, size_t words, uint64_t* dbits) {
+static int r1cs_check_group(blsgpu_ctx* ctx, const r1cs_sys& s, const u32x4* zt, const uint2* zbool, size_t w0, size_t g, size_t words, uint64_t* dbits) {
     CU(cudaMemsetAsync(s.fb_count, 0, 4, ctx->stream));
     LAUNCH(k_r1cs_lut, nblk(words * 64, 256), 256, s, zbool, w0, g, words, (uint32_t*)dbits);
     if (s.n_lut || s.n_gen) LAUNCH(k_r1cs_rows_list, R1_FB_BLOCKS, TPB, s, zt, zbool, w0, g, words, dbits);
-#if R1_LONG_ROWS
     if (s.n_long) LAUNCH(k_r1cs_long_rows, nblk(s.n_long, TPB / 32), TPB, s, zt, zbool, w0, g, words, dbits);
-    (void)part;
-#else
-    if (s.n_long) {
-        LAUNCH(k_r1cs_segments, nblk(s.n_seg, TPB / 32), TPB, s, zt, zbool, part);
-        LAUNCH(k_r1cs_combine, nblk(s.n_long, TPB / 32), TPB, s, (const u32x4*)part, w0, g, words, dbits);
-    }
-#endif
     return 0;
 }
 extern "C" {
@@ -593,12 +525,11 @@ int blsgpu_r1cs_check(blsgpu_ctx* ctx, int handle, const uint8_t* z48, size_t nw
     size_t words = (s.nrows + 63) / 64;
     bool host = ctx->ptr_mode == BLSGPU_HOST;
     // host mode stages one group of 32 witnesses at a time (32 * ncols * 48 bytes) so the workspace stays bounded
-    size_t zgroup = (size_t)R1_GROUP * s.ncols * 48, part_bytes = R1_LONG_ROWS ? 64 : (s.n_seg ? s.n_seg : 1) * 32 * 48;      // partial sums exist in the segment form only
-    if (int rc = ws_reserve(ctx, (host ? al(zgroup) : 0) + al(zgroup) + al(8 * s.ncols) + al(part_bytes) + (host ? al(8 * words * nwit) + al(nwit) : 0) + 8192)) return rc;
+    size_t zgroup = (size_t)R1_GROUP * s.ncols * 48;
+    if (int rc = ws_reserve(ctx, (host ? al(zgroup) : 0) + al(zgroup) + al(8 * s.ncols) + (host ? al(8 * words * nwit) + al(nwit) : 0) + 8192)) return rc;
     u32x4* zstage = host ? ws_take<u32x4>(ctx, zgroup / 16) : nullptr;
     u32x4* zt = ws_take<u32x4>(ctx, zgroup / 16);
     uint2* zbool = ws_take<uint2>(ctx, s.ncols);
-    u32x4* part = ws_take<u32x4>(ctx, part_bytes / 16);
     uint64_t* dbits = host ? ws_take<uint64_t>(ctx, words * nwit) : sat_bits;
     uint8_t* dall = all_sat ? (host ? ws_take<uint8_t>(ctx, nwit) : all_sat) : nullptr;
     for (size_t w0 = 0; w0 < nwit; w0 += R1_GROUP) {
@@ -607,7 +538,7 @@ int blsgpu_r1cs_check(blsgpu_ctx* ctx, int handle, const uint8_t* z48, size_t nw
         if (host) { CU(cudaMemcpyAsync(zstage, z48 + w0 * s.ncols * 48, g * s.ncols * 48, cudaMemcpyHostToDevice, ctx->stream)); zsrc = zstage; wbase = 0; }
         else { zsrc = (const u32x4*)z48; wbase = w0; }
         LAUNCH(k_r1cs_transpose, nblk(s.ncols, R1_TT), 256, zsrc, s.ncols, wbase, g, zt, zbool);
-        if (int rc = r1cs_check_group(ctx, s, zt, zbool, part, w0, g, words, dbits)) return rc;
+        if (int rc = r1cs_check_group(ctx, s, zt, zbool, w0, g, words, dbits)) return rc;
     }
     if (dall) LAUNCH(k_r1cs_all, nblk(nwit, 8), 256, (const uint64_t*)dbits, nwit, words, s.nrows, dall);
     if (host) {

@@ -14,46 +14,27 @@ struct fp12 { fp6 c0, c1; };
 BLS_CONST fp2 FROB1[6] = BLS_C_FROB1;     // xi^(i(p-1)/6)
 BLS_CONST fp FROB2[6] = BLS_C_FROB2;      // xi^(i(p^2-1)/6), in Fp
 
-// Fp6 values live in local memory, so the linear operations on them are out-of-line memory-to-memory routines
-// (BLS_FP6_OUTOFLINE, default on): inlined they are 3.5 KB each and made the Fp12 routines 20 KB+ apiece.
-#ifndef BLS_FP6_OUTOFLINE
-#define BLS_FP6_OUTOFLINE 1
-#endif
-#if BLS_FP6_OUTOFLINE
-#define BLS_FP6_LIN BLS_NOINLINE
-#else
-#define BLS_FP6_LIN BLS_HD
-#endif
-BLS_FP6_LIN void fp6_add(fp6& r, const fp6& a, const fp6& b) {
+// Fp6 values live in local memory, so the linear operations on them are out-of-line memory-to-memory routines: inlined they are
+// 3.5 KB each and made the Fp12 routines 20 KB+ apiece.
+BLS_NOINLINE void fp6_add(fp6& r, const fp6& a, const fp6& b) {
     const fp* x = &a.c0.c0; const fp* y = &b.c0.c0; fp* z = &r.c0.c0;
 #pragma unroll 1
     for (int i = 0; i < 6; i++) z[i] = fp_add(x[i], y[i]);
 }
-BLS_FP6_LIN void fp6_sub(fp6& r, const fp6& a, const fp6& b) {
+BLS_NOINLINE void fp6_sub(fp6& r, const fp6& a, const fp6& b) {
     const fp* x = &a.c0.c0; const fp* y = &b.c0.c0; fp* z = &r.c0.c0;
 #pragma unroll 1
     for (int i = 0; i < 6; i++) z[i] = fp_sub(x[i], y[i]);
 }
-BLS_FP6_LIN void fp6_neg(fp6& r, const fp6& a) {
+BLS_NOINLINE void fp6_neg(fp6& r, const fp6& a) {
     const fp* x = &a.c0.c0; fp* z = &r.c0.c0;
 #pragma unroll 1
     for (int i = 0; i < 6; i++) z[i] = fp_neg(x[i]);
 }
-BLS_FP6_LIN void fp6_mul_v(fp6& r, const fp6& a) { fp2 t = fp2_mul_xi(a.c2); fp2 u = a.c1, w = a.c0; r.c2 = u; r.c1 = w; r.c0 = t; }
+BLS_NOINLINE void fp6_mul_v(fp6& r, const fp6& a) { fp2 t = fp2_mul_xi(a.c2); fp2 u = a.c1, w = a.c0; r.c2 = u; r.c1 = w; r.c0 = t; }
 
-// BLS_LAZY (default): in the Miller loop the Fp6/Fp12 products are sums of Fp2 products accumulated UNREDUCED (wide.cuh) --
-// one Montgomery reduction per output coefficient, no conditional subtractions between the products, fewer Fp6 temporaries.
-// The final exponentiation keeps the separately reduced Karatsuba forms: measured faster there (profiles/r01_tuning.md).
-#ifndef BLS_LAZY
-#define BLS_LAZY 1
-#endif
-// 6 Fp2 products (Karatsuba over the cubic extension)
-// BLS_FP6_LOOP: the three diagonal and the three cross products as two 3-iteration loops (one copy of each body: a third of the
-// code; the instruction cache behind L0 holds 32 KB and the inlined form is 27 KB)
-#ifndef BLS_FP6_LOOP
-#define BLS_FP6_LOOP 1
-#endif
-#if BLS_FP6_LOOP
+// 6 Fp2 products (Karatsuba over the cubic extension): the three diagonal and the three cross products as two 3-iteration loops
+// (one copy of each body: a third of the code; the instruction cache behind L0 holds 32 KB and the inlined form is 27 KB)
 BLS_NOINLINE void fp6_mul(fp6& r, const fp6& a, const fp6& b) {
     const fp2* A = &a.c0; const fp2* B = &b.c0; fp2 v[3], t[3];
 #pragma unroll 1
@@ -67,18 +48,10 @@ BLS_NOINLINE void fp6_mul(fp6& r, const fp6& a, const fp6& b) {
     r.c1 = fp2_add(t[1], fp2_mul_xi(v[2]));
     r.c2 = fp2_add(t[2], v[1]);
 }
-#else
-BLS_NOINLINE void fp6_mul(fp6& r, const fp6& a, const fp6& b) {
-    fp2 v0 = fp2_mul(a.c0, b.c0), v1 = fp2_mul(a.c1, b.c1), v2 = fp2_mul(a.c2, b.c2);
-    fp2 t0 = fp2_sub(fp2_sub(fp2_mul(fp2_add(a.c1, a.c2), fp2_add(b.c1, b.c2)), v1), v2);
-    fp2 t1 = fp2_sub(fp2_sub(fp2_mul(fp2_add(a.c0, a.c1), fp2_add(b.c0, b.c1)), v0), v1);
-    fp2 t2 = fp2_sub(fp2_sub(fp2_mul(fp2_add(a.c0, a.c2), fp2_add(b.c0, b.c2)), v0), v2);
-    r.c0 = fp2_add(v0, fp2_mul_xi(t0));
-    r.c1 = fp2_add(t1, fp2_mul_xi(v2));
-    r.c2 = fp2_add(t2, v1);
-}
-#endif
-// schoolbook over the cubic extension, each output coefficient one 3-term dot product (27 wide products + 6 reductions =
+// In the Miller loop the Fp6/Fp12 products are sums of Fp2 products accumulated UNREDUCED (wide.cuh) -- one Montgomery reduction
+// per output coefficient, no conditional subtractions between the products, fewer Fp6 temporaries.  The final exponentiation keeps
+// the separately reduced Karatsuba forms: measured faster there (profiles/r01_tuning.md).
+// Schoolbook over the cubic extension, each output coefficient one 3-term dot product (27 wide products + 6 reductions =
 // 4,824 IMAD.WIDE against 5,400 for six separately reduced Karatsuba products)
 BLS_NOINLINE void fp6_mul_lz(fp6& r, const fp6& a, const fp6& b) {
     fp2 xb1 = fp2_mul_xi(b.c1), xb2 = fp2_mul_xi(b.c2);
@@ -86,19 +59,6 @@ BLS_NOINLINE void fp6_mul_lz(fp6& r, const fp6& a, const fp6& b) {
     fp2_dot3(t0, a.c0, b.c0, a.c1, xb2, a.c2, xb1);
     fp2_dot3(t1, a.c0, b.c1, a.c1, b.c0, a.c2, xb2);
     fp2_dot3(t2, a.c0, b.c2, a.c1, b.c1, a.c2, b.c0);
-    r.c0 = t0; r.c1 = t1; r.c2 = t2;
-}
-// a * (b0 + b1 v): 5 Fp2 products
-BLS_NOINLINE void fp6_mul_by_01(fp6& r, const fp6& a, const fp2& b0, const fp2& b1) {
-    fp2 v0 = fp2_mul(a.c0, b0), v1 = fp2_mul(a.c1, b1);
-    fp2 t0 = fp2_sub(fp2_mul(fp2_add(a.c1, a.c2), b1), v1);                       // a2 b1
-    fp2 t1 = fp2_sub(fp2_sub(fp2_mul(fp2_add(a.c0, a.c1), fp2_add(b0, b1)), v0), v1);   // a0 b1 + a1 b0
-    fp2 t2 = fp2_add(fp2_sub(fp2_mul(fp2_add(a.c0, a.c2), b0), v0), v1);           // a2 b0 + a1 b1
-    r.c0 = fp2_add(v0, fp2_mul_xi(t0)); r.c1 = t1; r.c2 = t2;
-}
-// a * (b1 v): 3 Fp2 products
-BLS_NOINLINE void fp6_mul_by_1(fp6& r, const fp6& a, const fp2& b1) {
-    fp2 t0 = fp2_mul_xi(fp2_mul(a.c2, b1)), t1 = fp2_mul(a.c0, b1), t2 = fp2_mul(a.c1, b1);
     r.c0 = t0; r.c1 = t1; r.c2 = t2;
 }
 BLS_NOINLINE void fp6_inv(fp6& r, const fp6& a) {
@@ -121,39 +81,25 @@ BLS_HD bool fp12_is_one(const fp12& a) {
 BLS_HD void fp12_conj(fp12& r, const fp12& a) { r.c0 = a.c0; fp6_neg(r.c1, a.c1); }
 
 // 3 Fp6 products
-#ifndef BLS_LAZY_FE
-#define BLS_LAZY_FE 0        // 1: the final exponentiation's Fp12 products also use the lazy Fp6 product (measured: profiles/r01_tuning.md)
-#endif
-#if BLS_LAZY_FE
-#define BLS_FP6_MUL_FE fp6_mul_lz
-#else
-#define BLS_FP6_MUL_FE fp6_mul
-#endif
 BLS_NOINLINE void fp12_mul(fp12& r, const fp12& a, const fp12& b) {
     fp6 t0, t1, t2, s0, s1;
-    BLS_FP6_MUL_FE(t0, a.c0, b.c0); BLS_FP6_MUL_FE(t1, a.c1, b.c1);
+    fp6_mul(t0, a.c0, b.c0); fp6_mul(t1, a.c1, b.c1);
     fp6_add(s0, a.c0, a.c1); fp6_add(s1, b.c0, b.c1);
-    BLS_FP6_MUL_FE(t2, s0, s1);
+    fp6_mul(t2, s0, s1);
     fp6_sub(t2, t2, t0); fp6_sub(r.c1, t2, t1);
     fp6_mul_v(t1, t1); fp6_add(r.c0, t0, t1);
 }
 // complex squaring: 2 Fp6 products
 BLS_NOINLINE void fp12_sqr(fp12& r, const fp12& a) {
     fp6 ab, s0, s1, t;
-#if BLS_LAZY
-#define BLS_FP6_MUL_SQR fp6_mul_lz
-#else
-#define BLS_FP6_MUL_SQR fp6_mul
-#endif
-    BLS_FP6_MUL_SQR(ab, a.c0, a.c1);
+    fp6_mul_lz(ab, a.c0, a.c1);
     fp6_add(s0, a.c0, a.c1);
     fp6_mul_v(t, a.c1); fp6_add(s1, a.c0, t);
-    BLS_FP6_MUL_SQR(s0, s0, s1);                   // (a0+a1)(a0+v a1) = a0^2 + v a1^2 + (1+v) a0a1
+    fp6_mul_lz(s0, s0, s1);                   // (a0+a1)(a0+v a1) = a0^2 + v a1^2 + (1+v) a0a1
     fp6_sub(s0, s0, ab); fp6_mul_v(t, ab); fp6_sub(r.c0, s0, t);
     fp6_add(r.c1, ab, ab);
 }
-// f * (c0 + c1 v + c4 v w): the sparse line element of the M-type twist (arkworks mul_by_014)
-#if BLS_LAZY
+// f * (c0 + c1 v + c4 v w): the sparse line element of the M-type twist (arkworks mul_by_014).
 // In the basis 1, w, .., w^5 (w^2 = v, w^6 = xi) f = sum g_k w^k with g = (c0.c0, c1.c0, c0.c1, c1.c1, c0.c2, c1.c2) and the
 // line is l0 + l2 w^2 + l3 w^3: out_k = g_k l0 + g_{k-2} l2 + g_{k-3} l3, indices mod 6, wrapped terms times xi (folded
 // into the line coefficient).  Six 3-term dot products: 9,648 IMAD.WIDE against 11,700, and no Fp6 temporaries.
@@ -168,17 +114,6 @@ BLS_NOINLINE void fp12_mul_by_014(fp12& f, const fp2& c0, const fp2& c1, const f
     fp2_dot3(o5, f.c1.c2, l0, f.c1.c1, l2, f.c0.c1, l3);
     f.c0.c0 = o0; f.c1.c0 = o1; f.c0.c1 = o2; f.c1.c1 = o3; f.c0.c2 = o4; f.c1.c2 = o5;
 }
-#else
-BLS_NOINLINE void fp12_mul_by_014(fp12& f, const fp2& c0, const fp2& c1, const fp2& c4) {
-    fp6 t0, t1, s;
-    fp6_mul_by_01(t0, f.c0, c0, c1);
-    fp6_mul_by_1(t1, f.c1, c4);
-    fp6_add(s, f.c0, f.c1);
-    fp6_mul_by_01(s, s, c0, fp2_add(c1, c4));
-    fp6_sub(s, s, t0); fp6_sub(f.c1, s, t1);
-    fp6_mul_v(t1, t1); fp6_add(f.c0, t0, t1);
-}
-#endif
 BLS_NOINLINE void fp12_inv(fp12& r, const fp12& a) {
     fp6 t0, t1;
     fp6_mul(t0, a.c0, a.c0); fp6_mul(t1, a.c1, a.c1); fp6_mul_v(t1, t1); fp6_sub(t0, t0, t1);
@@ -205,15 +140,10 @@ BLS_NOINLINE void fp12_frob2(fp12& r, const fp12& a) {
 }
 // Granger-Scott squaring for elements of the cyclotomic subgroup (after the easy part): 3 Fp4 squarings.
 // Inlined three / six times the routine is 52 KB and nearly half of its stall samples are `no_instruction` (32 KB instruction
-// cache behind L0).  BLS_CYCLO_COMPACT = 2 (default): ONE copy of the Fp4 squaring and of the two combinations inside a
-// 3-iteration loop over the coefficient pairs (20 KB, operands indexed in the thread's local memory where they live anyway):
-// final exponentiation 442 -> 423 ms at 2^20.  = 1: out-of-line helpers with operands and results by value: +5.6 % (argument
-// marshalling); helpers with operands by reference: +25 % (local-memory round trips).  = 0: fully inlined.  profiles/r01_tuning.md
-#ifndef BLS_CYCLO_COMPACT
-#define BLS_CYCLO_COMPACT 2
-#endif
-#if BLS_CYCLO_COMPACT == 2
-// loop form: one copy of the Fp4 squaring and of the two combinations, the three coefficient pairs selected by index
+// cache behind L0).  So ONE copy of the Fp4 squaring and of the two combinations sits inside a 3-iteration loop over the
+// coefficient pairs (20 KB, operands indexed in the thread's local memory where they live anyway): final exponentiation
+// 442 -> 423 ms at 2^20.  Out-of-line helpers with operands and results by value measured +5.6 % (argument marshalling), with
+// operands by reference +25 % (local-memory round trips).  profiles/r01_tuning.md
 BLS_NOINLINE void fp12_cyclo_sqr(fp12& r, const fp12& a) {
     const fp2* A = &a.c0.c0; fp12 out; fp2* R = &out.c0.c0;           // tower order: c0.c0 c0.c1 c0.c2 c1.c0 c1.c1 c1.c2
 #pragma unroll 1
@@ -229,43 +159,5 @@ BLS_NOINLINE void fp12_cyclo_sqr(fp12& r, const fp12& a) {
     }
     r = out;
 }
-#elif BLS_CYCLO_COMPACT && defined(__CUDACC__)
-struct fp4_pair { fp2 t0, t1; };
-BLS_NOINLINE fp4_pair fp4_sqr_v(fp2 a, fp2 b) {                       // (a + b y)^2, y^2 = xi
-    fp2 ab = fp2_mul(a, b);
-    fp2 s = fp2_mul(fp2_add(a, b), fp2_add(a, fp2_mul_xi(b)));
-    fp4_pair r; r.t0 = fp2_sub(fp2_sub(s, ab), fp2_mul_xi(ab)); r.t1 = fp2_dbl(ab); return r;
-}
-BLS_NOINLINE fp2 cyclo_comb_v(fp2 t, fp2 a) { fp2 z = fp2_add(t, a); z = fp2_dbl(z); return fp2_add(z, t); }      // 3 t + 2 a
-BLS_NOINLINE void fp12_cyclo_sqr(fp12& r, const fp12& a) {
-    fp4_pair p0 = fp4_sqr_v(a.c0.c0, a.c1.c1), p1 = fp4_sqr_v(a.c1.c0, a.c0.c2), p2 = fp4_sqr_v(a.c0.c1, a.c1.c2);
-    fp2 n00 = cyclo_comb_v(p0.t0, fp2_neg(a.c0.c0)), n11 = cyclo_comb_v(p0.t1, a.c1.c1);
-    fp2 n10 = cyclo_comb_v(fp2_mul_xi(p2.t1), a.c1.c0), n02 = cyclo_comb_v(p2.t0, fp2_neg(a.c0.c2));
-    fp2 n01 = cyclo_comb_v(p1.t0, fp2_neg(a.c0.c1)), n12 = cyclo_comb_v(p1.t1, a.c1.c2);
-    r.c0.c0 = n00; r.c1.c1 = n11; r.c1.c0 = n10; r.c0.c2 = n02; r.c0.c1 = n01; r.c1.c2 = n12;
-}
-#else
-BLS_HD void fp4_sqr(fp2& t0, fp2& t1, const fp2& a, const fp2& b) {    // (a + b y)^2, y^2 = xi
-    fp2 ab = fp2_mul(a, b);
-    fp2 s = fp2_mul(fp2_add(a, b), fp2_add(a, fp2_mul_xi(b)));
-    t0 = fp2_sub(fp2_sub(s, ab), fp2_mul_xi(ab));
-    t1 = fp2_dbl(ab);
-}
-BLS_NOINLINE void fp12_cyclo_sqr(fp12& r, const fp12& a) {
-    fp2 t0, t1, t2, t3, t4, t5;
-    fp4_sqr(t0, t1, a.c0.c0, a.c1.c1);
-    fp4_sqr(t2, t3, a.c1.c0, a.c0.c2);
-    fp4_sqr(t4, t5, a.c0.c1, a.c1.c2);
-    fp2 z;
-    z = fp2_sub(t0, a.c0.c0); z = fp2_dbl(z); r.c0.c0 = fp2_add(z, t0);
-    z = fp2_add(t1, a.c1.c1); z = fp2_dbl(z); r.c1.c1 = fp2_add(z, t1);
-    fp2 x5 = fp2_mul_xi(t5);
-    z = fp2_add(x5, a.c1.c0); z = fp2_dbl(z); r.c1.c0 = fp2_add(z, x5);
-    z = fp2_sub(t4, a.c0.c2); z = fp2_dbl(z); r.c0.c2 = fp2_add(z, t4);
-    z = fp2_sub(t2, a.c0.c1); z = fp2_dbl(z); r.c0.c1 = fp2_add(z, t2);
-    z = fp2_add(t3, a.c1.c2); z = fp2_dbl(z); r.c1.c2 = fp2_add(z, t3);
-}
-
-#endif
 
 }  // namespace bls

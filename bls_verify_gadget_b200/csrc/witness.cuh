@@ -7,8 +7,8 @@
 // ConstraintSystem in "prove" mode, src/constraints.rs:335-370); the values are checked bit for bit against the host
 // builder's assignment, which is pinned by the reference's own expectations (tests/test_gadget_circuit.py).
 //
-// Mapping: lane <-> assignment, warp <-> group of 32, rules strictly in order (a rule reads variables written by earlier
-// rules of the same lane: program order makes them visible).  Every branch is warp-uniform (rule kind, coefficient class).
+// Mapping: lane <-> assignment, groups of 32.  The rules run by dependency level (a rule reads only variables of earlier
+// levels), with a barrier between levels.  Every branch is warp-uniform (rule kind, coefficient class).
 // Included after r1cs.cuh in blsgpu.cu.
 #pragma once
 #include <cooperative_groups.h>
@@ -30,7 +30,7 @@ enum { WL_LUT = 0, WL_SUM = 1, WL_BIT = 2, WL_INPUT = 3, WL_ONE = 4 };
 struct wit_lrule { uint8_t kind, flags; uint16_t aux; uint32_t var; uint32_t a[6]; };
 struct wit_prog {
     size_t nvars, nout, nlc, nterms, nlevels;          // nvars: columns of the program (circuit variables, then scratch values); nout: circuit variables
-    wit_rule* rules; uint64_t* lc_ptr; uint32_t* col; fp* coeff; fp* coeffc; uint8_t* cls;
+    uint64_t* lc_ptr; uint32_t* col; fp* coeff; fp* coeffc; uint8_t* cls;
     wit_xrule* xrules; uint64_t* level_ptr;          // dependency levels: rules of one level are independent
     // "light" part (blsgpu_witness_load): rules whose operands and result are 0/1 values or small integers -- the SHA-256 / bit-decomposition
     // gadgets: 715 k of the verify program's 1.04 M rules on 10.4 k of its dependency levels -- run in k_witness_light, one CTA per group of
@@ -115,44 +115,9 @@ __device__ __forceinline__ fp wit_mul_canon(const fp& a, const fp& b) {
     }
     return fp_mul(fp_to_mont(a), b);
 }
-// inputs: fp [6 + 8 msg_len][nwit_padded] canonical (slot-major, so a warp reads 32 consecutive elements)
-__global__ void __launch_bounds__(32) k_witness_gen(wit_prog p, const fp* inputs, size_t nwit_padded, u32x4* zt_all) {
-    size_t group = blockIdx.x; int lane = threadIdx.x;
-    u32x4* zt = zt_all + group * p.nvars * 96;                        // 3 chunks x 32 lanes per variable
-    size_t w = group * 32 + lane;
-    fp one = fp_zero(); one.l[0] = 1;
-    wit_store(zt, 0, lane, one);
-    for (size_t v = 1; v < p.nvars; v++) {
-        wit_rule r = p.rules[v];
-        fp out;
-        switch (r.kind) {
-            case WR_MULADD: {
-                fp d = wit_lc(p, r.d, zt, nullptr, lane);
-                if (r.a) { fp a = wit_lc(p, r.a, zt, nullptr, lane), b = wit_lc(p, r.b, zt, nullptr, lane); out = fp_add(wit_mul_canon(a, b), d); }
-                else out = d;
-                break;
-            }
-            case WR_INV: out = wit_inv_canon(wit_lc(p, r.a, zt, nullptr, lane)); break;
-            case WR_NEQ: { fp a = wit_lc(p, r.a, zt, nullptr, lane); out = fp_zero(); out.l[0] = fp_is_zero(a) ? 0u : 1u; break; }
-            case WR_NEQMULT: { fp a = wit_lc(p, r.a, zt, nullptr, lane); out = fp_is_zero(a) ? one : wit_inv_canon(a); break; }
-            case WR_BIT: { fp a = wit_lc(p, r.a, zt, nullptr, lane); out = fp_zero(); out.l[0] = (a.l[r.aux >> 5] >> (r.aux & 31)) & 1u; break; }
-            case WR_FP2INV: {
-                fp2 x; x.c0 = fp_to_mont(wit_lc(p, r.a, zt, nullptr, lane)); x.c1 = fp_to_mont(wit_lc(p, r.b, zt, nullptr, lane));
-                fp2 iv = fp2_inv(x); out = fp_from_mont(r.aux ? iv.c1 : iv.c0); break;
-            }
-            case WR_FP12INV: {
-                fp12 x, iv; fp* xf = &x.c0.c0.c0;
-                for (int k = 0; k < 12; k++) xf[k] = fp_to_mont(wit_lc(p, r.a + k, zt, nullptr, lane));
-                fp12_inv(iv, x); out = fp_from_mont((&iv.c0.c0.c0)[r.aux]); break;
-            }
-            default: out = inputs[(size_t)r.aux * nwit_padded + w]; break;                 // WR_INPUT
-        }
-        wit_store(zt, v, lane, out);
-    }
-}
 // Level-synchronous form: one warp per (rule of the current level, group of 32 assignments); a grid-wide barrier between
 // levels (cooperative launch).  The verify circuit has 8,816 levels of ~80 rules: with 16 groups a level is ~1,300 independent
-// warp tasks, against ONE warp per group walking 707,809 rules in sequence in k_witness_gen (7.3 s, latency bound).
+// warp tasks, against ONE warp per group walking 707,809 rules in sequence (7.3 s, latency bound).
 #ifndef WIT_TPB
 #define WIT_TPB 128
 #endif
@@ -214,69 +179,6 @@ __global__ void __launch_bounds__(WIT_TPB, WIT_BPS) k_witness_levels(wit_prog p,
         pre = level + 1 < p.nlevels && warp < (hi_next - hi) * groups;
         if (pre) rn = p.xrules[hi + warp / groups];
         grid.sync();
-        lo = hi; hi = hi_next;
-    }
-}
-// Cluster form of the level-synchronous replay: one thread-block CLUSTER (WIT_CL CTAs on WIT_CL SMs, 8 x 256 threads = 64 warps) owns
-// one group of 32 assignments, one warp per rule of the current level, and the barrier between levels is the hardware cluster barrier
-// (~0.2 us) instead of a grid-wide barrier over every resident CTA (several us, 14.7 k times per launch).  Groups run independently
-// side by side (18 clusters fill the 148 SMs; further groups queue behind them), so a launch costs (levels x level latency) per WAVE
-// of 18 groups.  The next level's rule record -- static data -- is fetched BEFORE the barrier, so that after it only the loads
-// that depend on the previous level's values remain on the critical path.
-#ifndef WIT_CL
-#define WIT_CL 8
-#endif
-#define WIT_CL_TPB 256
-__device__ __forceinline__ void wit_eval_rule(const wit_prog& p, const wit_xrule& r, const fp* inputs, size_t nwit_padded, size_t group, u32x4* zt, uint2* zbw, int lane) {
-    const uint2* zb = zbw;
-    fp one = fp_zero(); one.l[0] = 1;
-    fp out;
-    switch (r.kind) {
-        case WR_MULADD: {
-            if (zb) { fp a, b, d; wit_lc3(p, r, zt, zb, lane, a, b, d); out = r.a_hi > r.a_lo ? fp_add(wit_mul_canon(a, b), d) : d; break; }
-            fp d = wit_lc_range(p, r.d_lo, r.d_hi, zt, zb, lane);
-            if (r.a_hi > r.a_lo) { fp a = wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane), b = wit_lc_range(p, r.b_lo, r.b_hi, zt, zb, lane); out = fp_add(wit_mul_canon(a, b), d); }
-            else out = d;
-            break;
-        }
-        case WR_INV: out = wit_inv_canon(wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane)); break;
-        case WR_NEQ: { fp a = wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane); out = fp_zero(); out.l[0] = fp_is_zero(a) ? 0u : 1u; break; }
-        case WR_NEQMULT: { fp a = wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane); out = fp_is_zero(a) ? one : wit_inv_canon(a); break; }
-        case WR_BIT: { fp a = wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane); out = fp_zero(); out.l[0] = (a.l[r.aux >> 5] >> (r.aux & 31)) & 1u; break; }
-        case WR_FP2INV: {
-            fp2 x; x.c0 = fp_to_mont(wit_lc_range(p, r.a_lo, r.a_hi, zt, zb, lane)); x.c1 = fp_to_mont(wit_lc_range(p, r.b_lo, r.b_hi, zt, zb, lane));
-            fp2 iv = fp2_inv(x); out = fp_from_mont(r.aux ? iv.c1 : iv.c0); break;
-        }
-        case WR_FP12INV: {
-            fp12 x, iv; fp* xf = &x.c0.c0.c0;
-            for (int k = 0; k < 12; k++) xf[k] = fp_to_mont(wit_lc(p, r.a_lo + k, zt, zb, lane));
-            fp12_inv(iv, x); out = fp_from_mont((&iv.c0.c0.c0)[r.aux]); break;
-        }
-        default: out = r.aux == 0xffff ? one : inputs[(size_t)r.aux * nwit_padded + group * 32 + lane]; break;       // WR_INPUT; 0xffff: the constant ONE (variable 0)
-    }
-    if (!zbw) { wit_store(zt, r.var, lane, out); return; }
-    bool small = out.l[0] < 2 && !(out.l[1] | out.l[2] | out.l[3] | out.l[4] | out.l[5] | out.l[6] | out.l[7] | out.l[8] | out.l[9] | out.l[10] | out.l[11]);
-    bool all = __all_sync(0xffffffffu, small); uint32_t pack = __ballot_sync(0xffffffffu, out.l[0] & 1u);
-    if (!all) wit_store(zt, r.var, lane, out);                // a 0/1 column lives in its packed word only (every reader tests the flag first)
-    if (lane == 0) zbw[r.var] = make_uint2(all ? pack : 0u, all ? 1u : 0u);
-}
-__global__ void __launch_bounds__(WIT_CL_TPB, 1) k_witness_cluster(wit_prog p, const fp* inputs, size_t nwit_padded, u32x4* zt_all, size_t groups, uint2* zbool_all) {
-    cooperative_groups::cluster_group cluster = cooperative_groups::this_cluster();
-    const unsigned CW = WIT_CL * (WIT_CL_TPB / 32);                                             // warps of the cluster
-    size_t group = blockIdx.x / WIT_CL; unsigned cw = cluster.block_rank() * (WIT_CL_TPB / 32) + (threadIdx.x >> 5); int lane = threadIdx.x & 31;
-    u32x4* zt = zt_all + group * p.nvars * 96; uint2* zbw = zbool_all ? zbool_all + group * p.nvars : nullptr;
-    uint64_t lo = p.level_ptr[0], hi = p.level_ptr[1];
-    wit_xrule rn; bool pre = lo + cw < hi;
-    if (pre) rn = p.xrules[lo + cw];
-    for (size_t level = 0; level < p.nlevels; level++) {
-        uint64_t hi_next = level + 2 <= p.nlevels ? p.level_ptr[level + 2] : hi;
-        for (uint64_t t = lo + cw; t < hi; t += CW) {
-            wit_xrule r = (t == lo + cw && pre) ? rn : p.xrules[t];
-            wit_eval_rule(p, r, inputs, nwit_padded, group, zt, zbw, lane);
-        }
-        pre = level + 1 < p.nlevels && hi + cw < hi_next;
-        if (pre) rn = p.xrules[hi + cw];                      // static data: travels while the cluster gathers at the barrier
-        cluster.sync();
         lo = hi; hi = hi_next;
     }
 }
@@ -393,7 +295,7 @@ __global__ void __launch_bounds__(256) k_witness_untranspose(const u32x4* zt_all
 }
 
 static void wit_release(wit_prog* p) {
-    cudaFree(p->rules); cudaFree(p->lc_ptr); cudaFree(p->col); cudaFree(p->coeff); cudaFree(p->coeffc); cudaFree(p->cls);
+    cudaFree(p->lc_ptr); cudaFree(p->col); cudaFree(p->coeff); cudaFree(p->coeffc); cudaFree(p->cls);
     cudaFree(p->xrules); cudaFree(p->level_ptr); cudaFree(p->lrules); cudaFree(p->llevel_ptr); cudaFree(p->lt_col); cudaFree(p->lt_coef);
     delete p;
 }
@@ -509,6 +411,7 @@ static void wit_split_program(wit_split& S, const wit_rule* hr, const uint64_t* 
 static int witness_load_impl(blsgpu_ctx* ctx, const uint8_t* rules16, const uint64_t* lc_ptr, const uint32_t* lc_col, const uint8_t* lc_coef48, size_t nvars, size_t nout, size_t nlc, size_t nterms,
                              const uint32_t* order, const uint64_t* level_ptr, size_t nlevels, size_t nkeys, int* handle) {
     if (!rules16 || !lc_ptr || !lc_col || !lc_coef48 || !handle || !nvars || !nout || nout > nvars) return fail(ctx, BLSGPU_ERR_ARG, "bad argument");
+    if (!order || !level_ptr || !nlevels) return fail(ctx, BLSGPU_ERR_ARG, "the witness program needs its level order (order, level_ptr, nlevels)");
     if (ctx->ptr_mode != BLSGPU_HOST) return fail(ctx, BLSGPU_ERR_ARG, "blsgpu_witness_load takes host pointers (the level-ordered rule tables are built on the host)");
     int h = -1; for (int i = 0; i < 4; i++) if (!ctx->wit[i]) { h = i; break; }
     if (h < 0) return fail(ctx, BLSGPU_ERR_ARG, "too many witness programs loaded");
@@ -524,9 +427,9 @@ static int witness_load_impl(blsgpu_ctx* ctx, const uint8_t* rules16, const uint
         p->ninputs = top; p->nkeys = nkeys; p->msg_len = (top - fixed) / 8;
     }
     size_t nt = nterms ? nterms : 1;
-    CU(cudaMalloc(&p->rules, 16 * nvars)); CU(cudaMalloc(&p->lc_ptr, 8 * (nlc + 1))); CU(cudaMalloc(&p->col, 4 * nt));
+    CU(cudaMalloc(&p->lc_ptr, 8 * (nlc + 1))); CU(cudaMalloc(&p->col, 4 * nt));
     CU(cudaMalloc(&p->coeff, 48 * nt)); CU(cudaMalloc(&p->coeffc, 48 * nt)); CU(cudaMalloc(&p->cls, nt));
-    CU(cudaMemcpyAsync(p->rules, rules16, 16 * nvars, cudaMemcpyHostToDevice, ctx->stream)); CU(cudaMemcpyAsync(p->lc_ptr, lc_ptr, 8 * (nlc + 1), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(p->lc_ptr, lc_ptr, 8 * (nlc + 1), cudaMemcpyHostToDevice, ctx->stream));
     if (nterms) {
         CU(cudaMemcpyAsync(p->col, lc_col, 4 * nterms, cudaMemcpyHostToDevice, ctx->stream));
         dev_tmp raw; CU(cudaMalloc(&raw.p, 48 * nterms));
@@ -534,20 +437,18 @@ static int witness_load_impl(blsgpu_ctx* ctx, const uint8_t* rules16, const uint
         LAUNCH(k_r1cs_prepare, nblk(nterms), TPB, (const uint8_t*)raw.p, nterms, p->coeff, p->coeffc, p->cls);
         CU(cudaStreamSynchronize(ctx->stream));
     }
-    if (order && level_ptr && nlevels) {                   // level-synchronous replay: light part + heavy part
-        wit_split S; wit_split_program(S, hr, lc_ptr, lc_col, lc_coef48, nvars, nout, order, nkeys, p->ninputs);
-        p->nlevels = S.hlevel_ptr.size() - 1; p->n_light = S.lrules.size(); p->n_llevels = S.llevel_ptr.size() / 2; p->n_islots = S.n_islots; p->n_lterms = S.lt_col.size();
-        size_t nx = S.xrules.size() ? S.xrules.size() : 1, nlr = S.lrules.size() ? S.lrules.size() : 1, nlt = S.lt_col.size() ? S.lt_col.size() : 1;
-        CU(cudaMalloc(&p->xrules, sizeof(wit_xrule) * nx)); CU(cudaMalloc(&p->level_ptr, 8 * S.hlevel_ptr.size()));
-        CU(cudaMalloc(&p->lrules, sizeof(wit_lrule) * nlr)); CU(cudaMalloc(&p->llevel_ptr, 4 * (S.llevel_ptr.size() ? S.llevel_ptr.size() : 1)));
-        CU(cudaMalloc(&p->lt_col, 4 * nlt)); CU(cudaMalloc(&p->lt_coef, 8 * nlt));
-        if (S.xrules.size()) CU(cudaMemcpyAsync(p->xrules, S.xrules.data(), sizeof(wit_xrule) * S.xrules.size(), cudaMemcpyHostToDevice, ctx->stream));
-        CU(cudaMemcpyAsync(p->level_ptr, S.hlevel_ptr.data(), 8 * S.hlevel_ptr.size(), cudaMemcpyHostToDevice, ctx->stream));
-        if (S.lrules.size()) CU(cudaMemcpyAsync(p->lrules, S.lrules.data(), sizeof(wit_lrule) * S.lrules.size(), cudaMemcpyHostToDevice, ctx->stream));
-        if (S.llevel_ptr.size()) CU(cudaMemcpyAsync(p->llevel_ptr, S.llevel_ptr.data(), 4 * S.llevel_ptr.size(), cudaMemcpyHostToDevice, ctx->stream));
-        if (S.lt_col.size()) { CU(cudaMemcpyAsync(p->lt_col, S.lt_col.data(), 4 * S.lt_col.size(), cudaMemcpyHostToDevice, ctx->stream)); CU(cudaMemcpyAsync(p->lt_coef, S.lt_coef.data(), 8 * S.lt_coef.size(), cudaMemcpyHostToDevice, ctx->stream)); }
-        CU(cudaStreamSynchronize(ctx->stream));
-    }
+    // level-synchronous replay: light part + heavy part
+    wit_split S; wit_split_program(S, hr, lc_ptr, lc_col, lc_coef48, nvars, nout, order, nkeys, p->ninputs);
+    p->nlevels = S.hlevel_ptr.size() - 1; p->n_light = S.lrules.size(); p->n_llevels = S.llevel_ptr.size() / 2; p->n_islots = S.n_islots; p->n_lterms = S.lt_col.size();
+    size_t nx = S.xrules.size() ? S.xrules.size() : 1, nlr = S.lrules.size() ? S.lrules.size() : 1, nlt = S.lt_col.size() ? S.lt_col.size() : 1;
+    CU(cudaMalloc(&p->xrules, sizeof(wit_xrule) * nx)); CU(cudaMalloc(&p->level_ptr, 8 * S.hlevel_ptr.size()));
+    CU(cudaMalloc(&p->lrules, sizeof(wit_lrule) * nlr)); CU(cudaMalloc(&p->llevel_ptr, 4 * (S.llevel_ptr.size() ? S.llevel_ptr.size() : 1)));
+    CU(cudaMalloc(&p->lt_col, 4 * nlt)); CU(cudaMalloc(&p->lt_coef, 8 * nlt));
+    if (S.xrules.size()) CU(cudaMemcpyAsync(p->xrules, S.xrules.data(), sizeof(wit_xrule) * S.xrules.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(p->level_ptr, S.hlevel_ptr.data(), 8 * S.hlevel_ptr.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (S.lrules.size()) CU(cudaMemcpyAsync(p->lrules, S.lrules.data(), sizeof(wit_lrule) * S.lrules.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (S.llevel_ptr.size()) CU(cudaMemcpyAsync(p->llevel_ptr, S.llevel_ptr.data(), 4 * S.llevel_ptr.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (S.lt_col.size()) { CU(cudaMemcpyAsync(p->lt_col, S.lt_col.data(), 4 * S.lt_col.size(), cudaMemcpyHostToDevice, ctx->stream)); CU(cudaMemcpyAsync(p->lt_coef, S.lt_coef.data(), 8 * S.lt_coef.size(), cudaMemcpyHostToDevice, ctx->stream)); }
     CU(cudaStreamSynchronize(ctx->stream));
     undo.p = nullptr; ctx->wit[h] = p; *handle = h; return 0;
 }
@@ -576,14 +477,14 @@ int blsgpu_witness_free(blsgpu_ctx* ctx, int handle) {
 }
 // decode, input slots and the level-synchronous replay for nwit triples: leaves the assignments in the transposed group layout
 // (group stride nvars * 96 u32x4) in the workspace; `extra` bytes of workspace are reserved for the caller's own buffers, which it
-// takes AFTER this returns.  want_zbool: also the packed 0/1 view per (group, variable).
+// takes AFTER this returns; also the packed 0/1 view per (group, variable).
 // bitmap == NULL: verify program (pk48 = nwit keys); else aggregate program (pk48 = nwit x p.nkeys keys, bitmap = nwit x p.nkeys bytes)
 static int witness_run(blsgpu_ctx* ctx, const wit_prog& p, const uint8_t* pk48, const uint8_t* bitmap, const uint8_t* msg, const uint8_t* sig96, size_t nwit, uint8_t* status, size_t extra,
-                       bool want_zbool, u32x4** zt_out, uint2** zbool_out, uint8_t** dstatus_out) {
+                       u32x4** zt_out, uint2** zbool_out, uint8_t** dstatus_out) {
     if ((bitmap != nullptr) != (p.nkeys != 0)) return fail(ctx, BLSGPU_ERR_ARG, p.nkeys ? "this is an aggregate_verify program: use the _aggregate entry points" : "this is a verify program: use blsgpu_witness_gen / _check");
     size_t groups = (nwit + 31) / 32, np = groups * 32, ninputs = p.ninputs, nk = p.nkeys ? p.nkeys : 1, nkeys_total = nwit * nk;
     if (int rc = ws_reserve(ctx, al(48 * nkeys_total) + al(nkeys_total) + al(96 * nwit) + al(p.msg_len * nwit + 1) + al(96 * nkeys_total) + al(192 * nwit) + 2 * al(np) + al(nkeys_total + np) + al(48 * ninputs * np) + al(groups * p.nvars * 1536) +
-                                 (want_zbool ? al(groups * p.nvars * 8) : 0) + al(groups * (p.n_islots + 1) * 256) + extra + 65536)) return rc;
+                                 al(groups * p.nvars * 8) + al(groups * (p.n_islots + 1) * 256) + extra + 65536)) return rc;
     const uint8_t *dpk, *dsig, *dmsg, *dbm = nullptr;
     if (int rc = stage_in(ctx, dpk, pk48, 48 * nkeys_total)) return rc;
     if (bitmap) { if (int rc = stage_in(ctx, dbm, bitmap, nkeys_total)) return rc; }
@@ -594,32 +495,20 @@ static int witness_run(blsgpu_ctx* ctx, const wit_prog& p, const uint8_t* pk48, 
     uint8_t* dstatus = status ? stage_out(ctx, status, nwit) : nullptr;
     fp* inputs = ws_take<fp>(ctx, ninputs * np);
     u32x4* zt_all = ws_take<u32x4>(ctx, groups * p.nvars * 96);
-    uint2* zbool_all = want_zbool ? ws_take<uint2>(ctx, groups * p.nvars) : nullptr;
+    uint2* zbool_all = ws_take<uint2>(ctx, groups * p.nvars);
     long long* sint_all = ws_take<long long>(ctx, groups * (p.n_islots + 1) * 32);
     LAUNCH(k_decode_g1, nblk(nkeys_total), TPB, dpk, nkeys_total, pk_soa, code_pk);
     LAUNCH(k_decode_g2<true>, nblk(nwit), TPB, dsig, nwit, sig_soa, code_sig);
     if (bitmap) LAUNCH(k_witness_inputs_agg, nblk(np), TPB, (const u32x4*)pk_soa, (const uint8_t*)code_pk, p.nkeys, dbm, (const u32x4*)sig_soa, (const uint8_t*)code_sig, dmsg, p.msg_len, nwit, np, inputs, dstatus);
     else LAUNCH(k_witness_inputs, nblk(np), TPB, (const u32x4*)pk_soa, (const uint8_t*)code_pk, (const u32x4*)sig_soa, (const uint8_t*)code_sig, dmsg, p.msg_len, nwit, np, inputs, dstatus);
-    if (p.xrules && !want_zbool) return fail(ctx, BLSGPU_ERR_ARG, "the level-synchronous replay works on the packed 0/1 view");
-    if (p.xrules && p.n_light) LAUNCH(k_witness_light, (unsigned)groups, WIT_LIGHT_TPB, p, (const fp*)inputs, np, zt_all, zbool_all, sint_all);      // 0/1 and small-integer rules first
-    if (p.xrules && ctx->wit_cluster) {                    // level-synchronous per group, hardware cluster barrier between levels
-        cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof cfg);
-        cfg.gridDim = dim3((unsigned)(groups * WIT_CL)); cfg.blockDim = dim3(WIT_CL_TPB); cfg.stream = ctx->stream;
-        cudaLaunchAttribute at[1]; at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = WIT_CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        wit_prog pc = p; const fp* in_c = inputs;
-        CU(cudaLaunchKernelEx(&cfg, k_witness_cluster, pc, in_c, np, zt_all, groups, zbool_all)); ctx->launches++;
-    } else if (p.xrules) {                                 // level-synchronous over the whole grid, cooperative launch: every block must be resident
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_witness_levels, WIT_TPB, 0)); if (per_sm > WIT_BPS) per_sm = WIT_BPS; CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, BLSGPU_ERR_CUDA, "k_witness_levels does not fit on an SM");
-        wit_prog pc = p; const fp* in_c = inputs; void* args[] = {(void*)&pc, (void*)&in_c, (void*)&np, (void*)&zt_all, (void*)&groups, (void*)&zbool_all};
-        CU(cudaLaunchCooperativeKernel((void*)k_witness_levels, dim3((unsigned)(per_sm * sms)), dim3(WIT_TPB), args, 0, ctx->stream)); ctx->launches++;
-    } else {
-        if (p.nvars != p.nout || want_zbool) return fail(ctx, BLSGPU_ERR_ARG, "the sequential replay needs a program without scratch columns (load it with its level order)");
-        LAUNCH(k_witness_gen, (unsigned)groups, 32, p, (const fp*)inputs, np, zt_all);
-    }
-    *zt_out = zt_all; if (zbool_out) *zbool_out = zbool_all; *dstatus_out = dstatus;
+    if (p.n_light) LAUNCH(k_witness_light, (unsigned)groups, WIT_LIGHT_TPB, p, (const fp*)inputs, np, zt_all, zbool_all, sint_all);      // 0/1 and small-integer rules first
+    // then the field rules, level-synchronous over the whole grid: cooperative launch, every block must be resident
+    int per_sm = 0, sms = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_witness_levels, WIT_TPB, 0)); if (per_sm > WIT_BPS) per_sm = WIT_BPS; CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
+    if (per_sm < 1) return fail(ctx, BLSGPU_ERR_CUDA, "k_witness_levels does not fit on an SM");
+    wit_prog pc = p; const fp* in_c = inputs; void* args[] = {(void*)&pc, (void*)&in_c, (void*)&np, (void*)&zt_all, (void*)&groups, (void*)&zbool_all};
+    CU(cudaLaunchCooperativeKernel((void*)k_witness_levels, dim3((unsigned)(per_sm * sms)), dim3(WIT_TPB), args, 0, ctx->stream)); ctx->launches++;
+    *zt_out = zt_all; *zbool_out = zbool_all; *dstatus_out = dstatus;
     return 0;
 }
 extern "C" {
@@ -633,8 +522,8 @@ static int witness_gen_core(blsgpu_ctx* ctx, int handle, const uint8_t* pk48, co
     size_t groups = (nwit + 31) / 32;
     bool host = ctx->ptr_mode == BLSGPU_HOST;
     size_t zbytes = nwit * p.nout * 48;
-    u32x4* zt_all; uint2* zbool_all = nullptr; uint8_t* dstatus;
-    if (int rc = witness_run(ctx, p, pk48, bitmap, msg, sig96, nwit, status, host ? al(zbytes) : 0, p.xrules != nullptr, &zt_all, &zbool_all, &dstatus)) return rc;
+    u32x4* zt_all; uint2* zbool_all; uint8_t* dstatus;
+    if (int rc = witness_run(ctx, p, pk48, bitmap, msg, sig96, nwit, status, host ? al(zbytes) : 0, &zt_all, &zbool_all, &dstatus)) return rc;
     uint8_t* dz = host ? ws_take<uint8_t>(ctx, zbytes) : z48;
     { dim3 grid(nblk(p.nout, 8), (unsigned)groups); k_witness_untranspose<<<grid, 256, 0, ctx->stream>>>((const u32x4*)zt_all, (const uint2*)zbool_all, p.nvars, p.nout, nwit, (u32x4*)dz); ctx->launches++; CU(cudaGetLastError()); }
     if (host) CU(cudaMemcpyAsync(z48, dz, zbytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -651,18 +540,16 @@ static int witness_check_core(blsgpu_ctx* ctx, int wit_handle, int r1cs_handle, 
     if (!nwit) return 0;
     wit_prog p = *ctx->wit[wit_handle]; r1cs_sys s = *ctx->r1cs[r1cs_handle];
     if (p.nout != s.ncols) return fail(ctx, BLSGPU_ERR_ARG, "witness program and R1CS system have different column counts");
-    if (!p.xrules) return fail(ctx, BLSGPU_ERR_ARG, "blsgpu_witness_check needs a program loaded with its level order");
-    size_t groups = (nwit + 31) / 32, words = (s.nrows + 63) / 64, part_bytes = R1_LONG_ROWS ? 64 : (s.n_seg ? s.n_seg : 1) * 32 * 48;
+    size_t groups = (nwit + 31) / 32, words = (s.nrows + 63) / 64;
     bool host = ctx->ptr_mode == BLSGPU_HOST;
     u32x4* zt_all; uint2* zbool_all; uint8_t* dstatus;
-    if (int rc = witness_run(ctx, p, pk48, bitmap, msg, sig96, nwit, status, al(part_bytes) + (host ? al(8 * words * nwit) + al(nwit) : 0), true, &zt_all, &zbool_all, &dstatus)) return rc;
-    u32x4* part = ws_take<u32x4>(ctx, part_bytes / 16);
+    if (int rc = witness_run(ctx, p, pk48, bitmap, msg, sig96, nwit, status, host ? al(8 * words * nwit) + al(nwit) : 0, &zt_all, &zbool_all, &dstatus)) return rc;
     uint64_t* dbits = host ? ws_take<uint64_t>(ctx, words * nwit) : sat_bits;
     uint8_t* dall = all_sat ? (host ? ws_take<uint8_t>(ctx, nwit) : all_sat) : nullptr;
     CU(cudaMemsetAsync(dbits, 0, 8 * words * nwit, ctx->stream));
     for (size_t gi = 0; gi < groups; gi++) {
         size_t w0 = gi * 32, g = nwit - w0 < 32 ? nwit - w0 : 32;
-        if (int rc = r1cs_check_group(ctx, s, zt_all + gi * p.nvars * 96, zbool_all + gi * p.nvars, part, w0, g, words, dbits)) return rc;
+        if (int rc = r1cs_check_group(ctx, s, zt_all + gi * p.nvars * 96, zbool_all + gi * p.nvars, w0, g, words, dbits)) return rc;
     }
     if (dall) LAUNCH(k_r1cs_all, nblk(nwit, 8), 256, (const uint64_t*)dbits, nwit, words, s.nrows, dall);
     if (host) {

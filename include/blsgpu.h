@@ -201,7 +201,8 @@ int blsgpu_r1cs_free(blsgpu_ctx* ctx, int handle);
 int blsgpu_r1cs_load_file(blsgpu_ctx* ctx, const char* path, int* handle, uint64_t shape4[4]);
 int blsgpu_r1cs_check_file(blsgpu_ctx* ctx, int handle, const char* path, size_t first, size_t count, uint64_t* sat_bits, uint8_t* all_sat);
 /* how blsgpu_r1cs_load classified the rows: counts[0] truth-table rows (<= 16 non-zeros on <= 5 distinct columns: evaluated bit-sliced over
- * 32 assignments when those columns are 0/1, generically otherwise), [1] generic short rows, [2] long rows, [3] their 32-entry segments */
+ * 32 assignments when those columns are 0/1, generically otherwise), [1] generic short rows, [2] long rows, [3] the 32-term
+ * metadata rounds the long-row kernel walks (sum over long rows and matrices of ceil(nnz / 32)) */
 int blsgpu_r1cs_row_classes(blsgpu_ctx* ctx, int handle, uint64_t counts[4]);
 
 /* ---- GPU witness generation for the verify circuit (SURVEY 8(f)-1; no counterpart in the reference, whose assignments come from
@@ -214,8 +215,9 @@ int blsgpu_r1cs_row_classes(blsgpu_ctx* ctx, int handle, uint64_t counts[4]);
  * blsgpu_r1cs_check; status[i] (nullable) = 0, or 2 / 3 when the key / signature does not decode to a non-identity point. */
 int blsgpu_witness_load(blsgpu_ctx* ctx, const uint8_t* rules16, const uint64_t* lc_ptr, const uint32_t* lc_col, const uint8_t* lc_coef48,
                         size_t ncols /* rules: circuit variables, then scratch columns */, size_t nvars /* circuit variables */, size_t nlc, size_t nterms,
-                        const uint32_t* order /* nullable: variables sorted by dependency level */, const uint64_t* level_ptr /* nlevels + 1 */, size_t nlevels,
-                        int* handle);   /* host pointers; with `order` the rules of one level run in parallel (blsgadget_program_levels) */
+                        const uint32_t* order /* variables sorted by dependency level */, const uint64_t* level_ptr /* nlevels + 1 */, size_t nlevels,
+                        int* handle);   /* host pointers; the rules of one level run in parallel.  order, level_ptr and nlevels come from
+                                         * blsgadget_program_levels and are required: BLSGPU_ERR_ARG without them */
 int blsgpu_witness_gen(blsgpu_ctx* ctx, int handle, const uint8_t* pk48, const uint8_t* msg, const uint8_t* sig96, size_t nwit,
                        uint8_t* z48, uint8_t* status);
 /* Generation and satisfaction check in one call: (pk, msg, sig) bytes in, per-constraint bits (words64 per assignment) and the
@@ -240,10 +242,6 @@ int blsgpu_witness_gen_aggregate(blsgpu_ctx* ctx, int handle, const uint8_t* pks
 int blsgpu_witness_check_aggregate(blsgpu_ctx* ctx, int wit_handle, int r1cs_handle, const uint8_t* pks48, const uint8_t* bitmap, const uint8_t* msg, const uint8_t* sig96, size_t nwit,
                                    uint64_t* sat_bits, uint8_t* all_sat, uint8_t* status);
 int blsgpu_witness_free(blsgpu_ctx* ctx, int handle);
-/* replay schedule: 0 (default) = one cooperative kernel over all groups with a grid-wide barrier per dependency level; 1 = one thread-block
- * cluster (8 SMs) per group of 32 assignments with the hardware cluster barrier between levels (measured slower on B200 at 512 and 2,048
- * assignments: at most 14 clusters of 8 are resident, profiles/r02_tuning.md).  Identical assignments either way. */
-int blsgpu_set_witness_mode(blsgpu_ctx* ctx, int cluster);
 
 /* ---- every GPU of the box behind one handle (SURVEY 8(b), 8(e)) ---------------------------------------------------------------------
  * blsgpu_create_multi: devices = ndev ordinals (NULL / ndev <= 0: every visible device); one single-GPU context and stream per device and

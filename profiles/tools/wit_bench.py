@@ -9,22 +9,18 @@ h = ctx.witness_load(prog); print('split', ctx.witness_shape(h))
 d_pk, d_msg, d_sig = (torch.from_numpy(x).to(dev) for x in (pk, msg, sig))
 z = torch.empty(n * nvars * 48, dtype=torch.uint8, device=dev); st = torch.empty(n, dtype=torch.uint8, device=dev)
 ctx.set_pointer_mode(True)
-for mode in (0, 1):
-  ctx.set_witness_mode(bool(mode))
-  for rep in range(2):
-    e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
-    e0.record(stream); ctx.witness_gen_ptr(h, d_pk.data_ptr(), d_msg.data_ptr(), d_sig.data_ptr(), n, z.data_ptr(), st.data_ptr()); e1.record(stream); torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1); print(f"witness_gen n={n} {'cluster' if mode else 'grid'}: {ms:.1f} ms = {n / (ms * 1e-3):.0f} assignments/s")
+for rep in range(2):
+  e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
+  e0.record(stream); ctx.witness_gen_ptr(h, d_pk.data_ptr(), d_msg.data_ptr(), d_sig.data_ptr(), n, z.data_ptr(), st.data_ptr()); e1.record(stream); torch.cuda.synchronize()
+  ms = e0.elapsed_time(e1); print(f"witness_gen n={n}: {ms:.1f} ms = {n / (ms * 1e-3):.0f} assignments/s")
 if len(sys.argv) > 2:      # fused generation + check (the packed 0/1 view is live in this path)
     c = G.verify_circuit(pk[:48].tobytes(), msg[:32].tobytes(), sig[:96].tobytes()); mats = c.matrices(); ctx.set_pointer_mode(False)
     rh = ctx.r1cs_load([m[0] for m in mats], [m[1] for m in mats], [m[2] for m in mats], c.nrows, c.ncols); ctx.set_pointer_mode(True)
     bits = torch.zeros(n * ((c.nrows + 63) // 64), dtype=torch.int64, device=dev); al = torch.zeros(n, dtype=torch.uint8, device=dev)
-    for mode in (0, 1):
-      ctx.set_witness_mode(bool(mode))
-      for rep in range(2):
-        e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
-        e0.record(stream); ctx.witness_check_ptr(h, rh, d_pk.data_ptr(), d_msg.data_ptr(), d_sig.data_ptr(), n, bits.data_ptr(), al.data_ptr(), st.data_ptr()); e1.record(stream); torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1); print(f"witness_check n={n} {'cluster' if mode else 'grid'}: {ms:.1f} ms = {n / (ms * 1e-3):.0f} assignments/s; all satisfied: {bool(al.all().item())}")
+    for rep in range(2):
+      e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
+      e0.record(stream); ctx.witness_check_ptr(h, rh, d_pk.data_ptr(), d_msg.data_ptr(), d_sig.data_ptr(), n, bits.data_ptr(), al.data_ptr(), st.data_ptr()); e1.record(stream); torch.cuda.synchronize()
+      ms = e0.elapsed_time(e1); print(f"witness_check n={n}: {ms:.1f} ms = {n / (ms * 1e-3):.0f} assignments/s; all satisfied: {bool(al.all().item())}")
 assert int(st.sum().item()) == 0
 # check a couple against the host
 zh, res = G.verify_witnesses([(pk[48*i:48*i+48].tobytes(), msg[32*i:32*i+32].tobytes(), sig[96*i:96*i+96].tobytes()) for i in (0, n - 1)], ncols=nvars)

@@ -8,18 +8,26 @@ P = 0x1a0111ea397fe69a4b1ba7b6434bacd764774b84f38512bf6730d2a0f6b0f6241eabfffeb1
 SO = os.path.join(ROOT, "tests", "_hostemu", "libdevcheck.so")
 def build():
     """nvcc build of devcheck.cu, redone when the CONTENT of any source differs from the stamp beside the library (mtimes do not
-    survive the copy to the GPU box); __graft_entry__.build() calls this so that the library travels prebuilt"""
-    import hashlib, subprocess
+    survive the copy to the GPU box); __graft_entry__.build() calls this so that the library travels prebuilt.  When the prebuilt copy
+    is stale and its directory cannot be written (a read-only tree), the library is built in a temporary directory instead"""
+    import hashlib, subprocess, tempfile
     csrc = os.path.join(ROOT, "bls_verify_gadget_b200", "csrc")
     src = [os.path.join(ROOT, "tests", "devcheck", f) for f in ("devcheck.cu", "ops.h")] + [os.path.join(csrc, f) for f in ("consts.cuh", "fp.cuh", "fp2.cuh", "wide.cuh", "tower.cuh", "curve.cuh", "pairing.cuh")]
     h = hashlib.sha256()
     for f in src: h.update(open(f, "rb").read())
-    stamp = SO + ".stamp"; digest = h.hexdigest()
-    if not os.path.exists(SO) or not os.path.exists(stamp) or open(stamp).read().strip() != digest:
-        os.makedirs(os.path.dirname(SO), exist_ok=True)
-        subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-shared", "-Xcompiler", "-fPIC", "-I", csrc, "-o", SO, src[0]])
-        open(stamp, "w").write(digest + "\n")
-    return SO
+    digest = h.hexdigest()
+    so = SO
+    try: os.makedirs(os.path.dirname(SO), exist_ok=True)
+    except OSError: pass
+    if not os.access(os.path.dirname(SO), os.W_OK) and not _fresh(SO, digest):
+        so = os.path.join(tempfile.gettempdir(), "blsgpu-devcheck-" + digest[:16], "libdevcheck.so"); os.makedirs(os.path.dirname(so), exist_ok=True)
+    if not _fresh(so, digest):
+        subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-shared", "-Xcompiler", "-fPIC", "-I", csrc, "-o", so, src[0]])
+        open(so + ".stamp", "w").write(digest + "\n")
+    return so
+def _fresh(so, digest):
+    stamp = so + ".stamp"
+    return os.path.exists(so) and os.path.exists(stamp) and open(stamp).read().strip() == digest
 def dev_lib():
     return ctypes.CDLL(os.environ.get("DEVCHECK_SO") or build())
 def rand_fp(rng, n):

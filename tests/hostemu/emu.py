@@ -6,9 +6,15 @@ SO = os.path.join(ROOT, "tests", "_hostemu", "libhostemu.so")
 SRC = [os.path.join(HERE, "hostemu.cpp"), os.path.join(ROOT, "tests", "devcheck", "ops.h")] + [os.path.join(ROOT, "bls_verify_gadget_b200", "csrc", f) for f in
       ("fp.cuh", "fp2.cuh", "tower.cuh", "curve.cuh", "h2c.cuh", "pairing.cuh", "stages.cuh", "consts.cuh", "wide.cuh")]
 def build():
+    """rebuilt when a source is newer than the library; in a read-only tree a stale library is rebuilt in a temporary directory"""
     if not os.path.exists(SO) or any(os.path.getmtime(s) > os.path.getmtime(SO) for s in SRC):
-        os.makedirs(os.path.dirname(SO), exist_ok=True)
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I", os.path.join(ROOT, "bls_verify_gadget_b200", "csrc"), "-o", SO, SRC[0]])
+        so = SO
+        try: os.makedirs(os.path.dirname(SO), exist_ok=True)
+        except OSError: pass
+        if not os.access(os.path.dirname(SO), os.W_OK):
+            import tempfile; so = os.path.join(tempfile.mkdtemp(prefix="blsgpu-hostemu-"), "libhostemu.so")
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I", os.path.join(ROOT, "bls_verify_gadget_b200", "csrc"), "-o", so, SRC[0]])
+        return so
     return SO
 _lib = None
 def lib():

@@ -463,11 +463,6 @@ def test_gpu_witness_generation_matches_host_builder(ctx, C):
     assert list(allsat) == [1 if e in (0, 1) else 0 for e in exp]                             # flagged items carry no assignment
     fbits, fall, fst = ctx.witness_check(h, hh, pk, msg, sig, c.nrows)                        # fused: generation + check without the row-major copy
     assert np.array_equal(fbits, bits) and np.array_equal(fall, allsat) and np.array_equal(fst, st)
-    ctx.set_witness_mode(True)                                                                # the cluster schedule (one thread-block cluster per group): same bytes
-    try:
-        z2, st2 = ctx.witness_gen(h, pk, msg, sig, nvars); assert np.array_equal(z2, z) and np.array_equal(st2, st)
-        cbits, call, cst = ctx.witness_check(h, hh, pk, msg, sig, c.nrows); assert np.array_equal(cbits, bits) and np.array_equal(call, allsat)
-    finally: ctx.set_witness_mode(False)
     ctx.r1cs_free(hh); ctx.witness_free(h)
 
 @pytest.mark.parametrize("mlen", [0, 31, 33, 250])
