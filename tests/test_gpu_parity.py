@@ -143,10 +143,10 @@ def test_aggregate_fixtures(ctx, eth):                                    # test
 def test_g1_segmented_aggregate_differential(ctx, C):
     from bls_verify_gadget_b200 import synth
     n = 700; pk, _ = ctx.sk_to_pk(synth.secret_keys(n)); pk = pk.reshape(n, 48).copy()
-    pk[10] = pk[11]                                                       # equal points: the doubling branch of the addition
-    pk[20, 0] ^= 0x20; pk[21] = pk[20]; pk[21, 0] ^= 0x20                 # P and -P adjacent
+    seg = [0, 1, 1, 3, 12, 22, 40, 41, 553, 700]                          # ragged, an empty segment, one of 512 (one lane per segment)
+    pk[4] = pk[3]                                                         # segment [3, 12) opens with K, K: the running sum equals the added point, the doubling branch of the addition
+    pk[13] = pk[12]; pk[13, 0] ^= 0x20                                    # segment [12, 22) opens with P, -P: the running sum cancels to the identity
     pk[30] = 0; pk[30, 0] = 0xc0                                          # identity member
-    seg = [0, 1, 1, 3, 12, 22, 40, 41, 553, 700]                          # ragged, an empty segment, one of 512
     out, st = ctx.g1_aggregate(pk.reshape(-1), seg); oout, ost = C.g1_aggregate(pk.reshape(-1), seg, threads=8)
     assert list(st) == list(ost) == [0, 4, 0, 0, 0, 0, 0, 0, 0]
     ok = st == 0
