@@ -22,7 +22,7 @@ extern "C" int dev_run_op(int op, const uint8_t* in, uint8_t* out, size_t n) {
     cudaMemcpy(din, in, bi, cudaMemcpyHostToDevice);
     switch (op) {
 #define L(K) case K: launch<K>(din, dout, n, d); break;
-        L(1) L(2) L(3) L(4) L(5) L(6) L(7) L(8) L(9) L(10) L(11) L(12) L(13) L(14) L(15) L(16) L(17) L(18) L(19) L(20) L(21) L(22) L(23) L(24) L(25) L(26) L(27) L(28) L(29) L(30) L(31) L(32) L(33) L(34) L(35) L(36) L(37) L(38) L(39) L(40) L(41)
+        L(1) L(2) L(3) L(4) L(5) L(6) L(7) L(8) L(9) L(10) L(11) L(12) L(13) L(14) L(15) L(16) L(17) L(18) L(19) L(20) L(21) L(22) L(23) L(24) L(25) L(26) L(27) L(28) L(29) L(30) L(31) L(32) L(33) L(34) L(35) L(36) L(37) L(38) L(39) L(40) L(41) L(42) L(43) L(44) L(45) L(46)
 #undef L
         default: cudaFree(din); cudaFree(dout); return -1;
     }

@@ -52,6 +52,11 @@ static inline op_desc op_shape(int op) {
         case 31: return {2, 1};   // fp_mul_lz (split wide accumulator + reduction) == fp_mul
         case 32: return {4, 2};   // fp2_dot, n = 1 == fp2_mul
         case 33: return {12, 2};  // fp2_dot, n = 3 == x0 y0 + x1 y1 + x2 y2
+        case 42: return {2, 6};   // sswu_map(u) -> xn, xd, y
+        case 43: return {6, 6};   // iso3_map(xn, xd, y) -> Jacobian X, Y, Z
+        case 44: return {6, 6};   // g2_clear_cofactor(Jacobian P)
+        case 45: return {2, 3};   // fp2_sgn0(a), fp2_lex_largest(a), fp_canon_is_larger_half(a.c0), each 0/1 in the low word
+        case 46: return {1, 2};   // Fp square root as g1_decode takes it: a * a^((p-3)/4), and y^2 == a in out[1].l[0]
         default: return {0, 0};
     }
 }
@@ -144,6 +149,12 @@ BLS_HD void run_op(int op, const fp* in, fp* out) {
                    for (int k = 0; k < 8; k++) { fp_lacc_mad(a, in[0], in[4].l[0]); fp_lacc_mad(a, in[1], in[5].l[0]); fp_lacc_mad(a, in[2], in[6].l[0]); fp_lacc_mad(a, nz, in[7].l[0]); }
                    out[0] = fp_lacc_reduce(a); break; }
         case 34: out[0] = fp_inv(in[0]); out[1] = fp_inv_fermat(in[0]); break;
+        case 42: ld2(a, in); sswu_map(b, c, d, a); st2(out, b); st2(out + 2, c); st2(out + 4, d); break;
+        case 43: ld2(a, in); ld2(b, in + 2); ld2(c, in + 4); iso3_map(P, a, b, c); st2(out, P.X); st2(out + 2, P.Y); st2(out + 4, P.Z); break;
+        case 44: ld2(P.X, in); ld2(P.Y, in + 2); ld2(P.Z, in + 4); g2_clear_cofactor(Q, P); st2(out, Q.X); st2(out + 2, Q.Y); st2(out + 4, Q.Z); break;
+        case 45: ld2(a, in); out[0] = fp_zero(); out[1] = fp_zero(); out[2] = fp_zero();
+                 out[0].l[0] = fp2_sgn0(a); out[1].l[0] = fp2_lex_largest(a) ? 1u : 0u; out[2].l[0] = fp_canon_is_larger_half(fp_from_mont(a.c0)) ? 1u : 0u; break;
+        case 46: { fp y = fp_mul(in[0], fp_pow_pm3d4(in[0])); out[0] = y; out[1] = fp_zero(); out[1].l[0] = fp_eq(fp_sqr(y), in[0]) ? 1u : 0u; break; }
         default: break;
     }
     (void)d;

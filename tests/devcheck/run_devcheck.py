@@ -9,10 +9,11 @@ SO = os.path.join(ROOT, "tests", "_hostemu", "libdevcheck.so")
 def build():
     """nvcc build of devcheck.cu, redone when the CONTENT of any source differs from the stamp beside the library (mtimes do not
     survive the copy to the GPU box); __graft_entry__.build() calls this so that the library travels prebuilt.  When the prebuilt copy
-    is stale and its directory cannot be written (a read-only tree), the library is built in a temporary directory instead"""
+    is stale and its directory cannot be written (a read-only tree), the library is built in a temporary directory instead.
+    The digest covers every header of csrc/, not only the ones devcheck.cu names: ops.h reaches h2c.cuh through stages.cuh"""
     import hashlib, subprocess, tempfile
     csrc = os.path.join(ROOT, "bls_verify_gadget_b200", "csrc")
-    src = [os.path.join(ROOT, "tests", "devcheck", f) for f in ("devcheck.cu", "ops.h")] + [os.path.join(csrc, f) for f in ("consts.cuh", "fp.cuh", "fp2.cuh", "wide.cuh", "tower.cuh", "curve.cuh", "pairing.cuh")]
+    src = [os.path.join(ROOT, "tests", "devcheck", f) for f in ("devcheck.cu", "ops.h")] + [os.path.join(csrc, f) for f in sorted(os.listdir(csrc)) if f.endswith(".cuh")]
     h = hashlib.sha256()
     for f in src: h.update(open(f, "rb").read())
     digest = h.hexdigest()
@@ -42,8 +43,8 @@ def edge_fp(rng, n):
         v = specials[pick[i]] if pick[i] < len(specials) else int.from_bytes(rng.bytes(48), "little") % P
         out[i] = np.frombuffer(v.to_bytes(48, "little"), np.uint8)
     return out
-EDGE_OPS = (1, 2, 3, 4, 8, 9, 10, 11, 12, 21, 22, 26, 27, 29, 30, 31, 32, 33, 34, 35, 36)      # pure field arithmetic: any canonical input is valid
-def check(ops=range(1, 42), n=256, seed=1, edge=False):
+EDGE_OPS = (1, 2, 3, 4, 8, 9, 10, 11, 12, 21, 22, 26, 27, 29, 30, 31, 32, 33, 34, 35, 36, 45, 46)      # pure field arithmetic: any canonical input is valid
+def check(ops=range(1, 47), n=256, seed=1, edge=False):
     D = dev_lib(); rng = np.random.default_rng(seed); bad = []
     for op in ops:
         n_in, n_out = emu.op_shape(op)
