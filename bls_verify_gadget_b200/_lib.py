@@ -36,7 +36,7 @@ def lib():
     return _lib
 
 EXPORTS = ["blsgpu_create", "blsgpu_destroy", "blsgpu_last_error", "blsgpu_set_stream", "blsgpu_set_pointer_mode", "blsgpu_synchronize",
-           "blsgpu_launch_count", "blsgpu_set_profiling", "blsgpu_stage_times", "blsgpu_set_chunk", "blsgpu_set_lanes", "blsgpu_set_split", "blsgpu_set_coop", "blsgpu_verify_batch", "blsgpu_verify_batch_rlc", "blsgpu_verify_batch_rlc_bisect", "blsgpu_fast_aggregate_verify_batch", "blsgpu_aggregate_verify_batch", "blsgpu_g1_uncompress", "blsgpu_g1_compress", "blsgpu_g2_uncompress", "blsgpu_g2_compress", "blsgpu_pool_create", "blsgpu_pool_free", "blsgpu_pool_fast_aggregate_verify", "blsgpu_hash_to_g2_batch", "blsgpu_g1_aggregate",
+           "blsgpu_launch_count", "blsgpu_set_profiling", "blsgpu_stage_times", "blsgpu_set_chunk", "blsgpu_set_lanes", "blsgpu_set_split", "blsgpu_set_coop", "blsgpu_verify_batch", "blsgpu_verify_batch_rlc", "blsgpu_verify_batch_rlc_bisect", "blsgpu_fast_aggregate_verify_batch", "blsgpu_aggregate_verify_batch", "blsgpu_g1_uncompress", "blsgpu_g1_compress", "blsgpu_g2_uncompress", "blsgpu_g2_compress", "blsgpu_pool_create", "blsgpu_pool_free", "blsgpu_pool_fast_aggregate_verify", "blsgpu_verify_signature_sets", "blsgpu_pool_verify_signature_sets", "blsgpu_hash_to_g2_batch", "blsgpu_g1_aggregate",
            "blsgpu_g2_aggregate", "blsgpu_deserialize_g1", "blsgpu_deserialize_g2", "blsgpu_sk_to_pk_batch", "blsgpu_sign_batch", "blsgpu_pairing_gt",
            "blsgpu_gt_fold", "blsgpu_fp_mul_raw", "blsgpu_imad_peak", "blsgpu_r1cs_load", "blsgpu_r1cs_check", "blsgpu_r1cs_free", "blsgpu_r1cs_row_classes", "blsgpu_r1cs_load_file", "blsgpu_r1cs_check_file", "blsgpu_witness_load", "blsgpu_witness_gen", "blsgpu_witness_check", "blsgpu_witness_free", "blsgpu_witness_msg_len", "blsgpu_witness_load_aggregate", "blsgpu_witness_shape", "blsgpu_witness_gen_aggregate", "blsgpu_witness_check_aggregate",
            "blsgpu_create_multi", "blsgpu_destroy_multi", "blsgpu_multi_last_error", "blsgpu_multi_ndev", "blsgpu_multi_nccl_version", "blsgpu_multi_ctx", "blsgpu_multi_verify_batch", "blsgpu_multi_peek"]
@@ -164,6 +164,45 @@ class Context:
         _need("sig96", sg, 96 * nc); _need("msg32", m, 32 * nc); _need("idx", ix, 4 * nc * k); _need("bitmap", bm, 8 * ((nc * k + 63) // 64))
         self.pool_fast_aggregate_verify_ptr(handle, ix, bm, k, m, sg, nc, st, agg)
         return (st, agg) if want_agg else st
+    # ---- signature sets: set s = keys [key_off[s], key_off[s+1]) of the flat list, one message, one signature
+    def verify_signature_sets_ptr(self, pks, key_off, bitmap, msg, msg_off, sig, nsets, seed16, status, ok_bitmap=None):
+        """-> number of sets re-run per set (raw pointers: numpy arrays in host mode, ints in device mode)"""
+        rerun = ctypes.c_uint64(0)
+        self._ck(lib().blsgpu_verify_signature_sets(self._h, _p(pks), _p(key_off), _p(bitmap), _p(msg), _p(msg_off), _p(sig), _sz(nsets), _p(seed16), _p(status), _p(ok_bitmap), ctypes.byref(rerun)))
+        return int(rerun.value)
+    def pool_verify_signature_sets_ptr(self, handle, idx, key_off, bitmap, msg, msg_off, sig, nsets, seed16, status, ok_bitmap=None):
+        rerun = ctypes.c_uint64(0)
+        self._ck(lib().blsgpu_pool_verify_signature_sets(self._h, int(handle), _p(idx), _p(key_off), _p(bitmap), _p(msg), _p(msg_off), _p(sig), _sz(nsets), _p(seed16), _p(status), _p(ok_bitmap), ctypes.byref(rerun)))
+        return int(rerun.value)
+    @staticmethod
+    def _sets_args(key_off, msgs, sig96, seed16, bitmap, fixed32):
+        ko = np.ascontiguousarray(key_off, dtype=np.uint32).reshape(-1); sg = _u8(sig96); n = sg.size // 96
+        _need("sig96", sg, 96 * n)
+        if ko.size != n + 1 or ko[0] != 0 or np.any(np.diff(ko.astype(np.int64)) < 0): raise ValueError("key_off must hold nsets + 1 non-decreasing offsets starting at 0")
+        if fixed32: flat, off = _u8(msgs), None; _need("msgs", flat, 32 * n)
+        else:
+            if len(msgs) != n: raise ValueError(f"{len(msgs)} messages for {n} signatures")
+            flat, off = pack_msgs(msgs)
+        nk = int(ko[-1]); bm = np.ascontiguousarray(bitmap, dtype=np.uint64) if bitmap is not None else None; _need("bitmap", bm, 8 * ((nk + 63) // 64))
+        seed = None
+        if seed16 is not None: seed = _u8(seed16); _need("seed16", seed, 16)
+        return ko, flat, off, sg, n, nk, bm, seed
+    def verify_signature_sets(self, pks48, key_off, msgs, sig96, seed16=None, bitmap=None, fixed32=False):
+        """set s = keys pks48[key_off[s]:key_off[s+1]] (48 bytes each), message msgs[s] (or 32 bytes each with fixed32), signature s.
+        seed16 None: one pairing check per set; else per-piece random linear combinations with the exact outcome.
+        -> (status uint8[nsets], ok_bitmap uint64[ceil(nsets/64)], sets re-run per set)"""
+        ko, flat, off, sg, n, nk, bm, seed = self._sets_args(key_off, msgs, sig96, seed16, bitmap, fixed32)
+        pk = _u8(pks48); _need("pks48", pk, 48 * nk)
+        st = np.empty(max(n, 1), np.uint8); ok = np.zeros(max((n + 63) // 64, 1), np.uint64)
+        rerun = self.verify_signature_sets_ptr(pk, ko, bm, flat, off, sg, n, seed, st, ok)
+        return st[:n], ok[:(n + 63) // 64], rerun
+    def pool_verify_signature_sets(self, handle, idx, key_off, msgs, sig96, seed16=None, bitmap=None, fixed32=False):
+        """verify_signature_sets with the keys as indices into a resident pool (pool_create)"""
+        ko, flat, off, sg, n, nk, bm, seed = self._sets_args(key_off, msgs, sig96, seed16, bitmap, fixed32)
+        ix = np.ascontiguousarray(idx, dtype=np.uint32).reshape(-1); _need("idx", ix, 4 * nk)
+        st = np.empty(max(n, 1), np.uint8); ok = np.zeros(max((n + 63) // 64, 1), np.uint64)
+        rerun = self.pool_verify_signature_sets_ptr(handle, ix, ko, bm, flat, off, sg, n, seed, st, ok)
+        return st[:n], ok[:(n + 63) // 64], rerun
     def hash_to_g2(self, msgs):
         flat, off = pack_msgs(msgs); out = np.empty(96 * len(msgs), np.uint8); self.hash_to_g2_ptr(flat, off, len(msgs), out); return out
     def g1_aggregate(self, pts48, seg_off):

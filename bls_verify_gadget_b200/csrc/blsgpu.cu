@@ -11,6 +11,7 @@
 //   k_gt_reduce                 K5' strided product of GT values (per-batch accumulator)
 //   k_status_bitmap                 status -> packed ok bitmap
 //   k_segsum_g1 / k_segsum_g2   K3  warp-per-segment aggregation, tree reduction in shared memory
+//   k_sets_rlc_prep                 signature sets, RLC form: status rule of the aggregate, [r] aggregate key, [r] signature (sets.cuh)
 //   k_scalar_mul_g1 / _g2       K6  [sk]G1, [sk]H(m)
 //   k_encode_g1 / k_encode_g2   K7  affine limb-SoA -> compressed bytes
 //   k_fp_mul_raw, k_imad_peak   K0  parity hook and integer-multiply roofline microbenchmark
@@ -472,7 +473,8 @@ template <> struct segsum_traits<fp2> { enum { K = 4 }; static __device__ __forc
 #define SEG_WARPS 4
 template <class F> __global__ void __launch_bounds__(32 * SEG_WARPS) k_segsum(const u32x4* pts_soa, const uint8_t* code, size_t npts, const uint32_t* seg_off, size_t seg_stride,
                                                                             const uint64_t* bitmap, size_t nseg, u32x4* out_jac, uint8_t* status, uint8_t bad_code,
-                                                                            const uint32_t* idx /* nullable: member i of the flat list is point idx[i] of the resident pool */, int L) {
+                                                                            const uint32_t* idx /* nullable: member i of the flat list is point idx[i] of the resident pool */, int L,
+                                                                            size_t pt_base /* without idx: member i is point i - pt_base (a pass of the flat list) */) {
     __shared__ jac<F> sm[SEG_WARPS][32];
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, sub = lane / L, sl = lane % L, per_warp = 32 / L;
     size_t s = (blockIdx.x * (size_t)SEG_WARPS + warp) * per_warp + sub;
@@ -484,7 +486,7 @@ template <class F> __global__ void __launch_bounds__(32 * SEG_WARPS) k_segsum(co
     for (size_t i = lo + sl; i < hi; i += L) {
         if (bitmap && !((bitmap[i >> 6] >> (i & 63)) & 1)) continue;
         cnt++;
-        size_t pi = idx ? (size_t)idx[i] : i;
+        size_t pi = idx ? (size_t)idx[i] : i - pt_base;
         if (pi >= npts) { bad = 1; continue; }
         uint8_t c = code[pi];
         if (c > DEC_INF) { bad = 1; continue; }
@@ -533,17 +535,23 @@ template <class F> __device__ __forceinline__ void jac_mul_u64(jac<F>& r, const 
     jac_set_identity(r);
     for (int i = 63; i >= 0; i--) { jac_dbl(r, r); if ((k >> i) & 1) jac_add_mixed(r, r, p); }
 }
+// the random-linear-combination weights of item i (k_rlc_scale, k_sets_rlc_prep), r = rlc_scalar(seed16, idx): pk_soa[i] <- [r] pk as affine, then
+// rsig = [r] sig_soa[i] (Jacobian; the identity when sig_inf).  pk has prime order > 2^64 and is not the identity: [r] pk never is.
+// The G1 result is stored and the signature loaded only between the two ladders, so neither is live across the other ladder.
+__device__ __forceinline__ void rlc_scale_item(u32x4* pk_soa, const u32x4* sig_soa, size_t n, size_t i, const g1_aff& pk, bool sig_inf,
+                                               const uint8_t* seed16, uint64_t idx, g2_jac& rsig) {
+    uint64_t r = rlc_scalar(seed16, idx);
+    { g1_jac rp; jac_mul_u64(rp, pk, r); g1_aff a; jac_to_aff(a, rp); soa_store_g1(pk_soa, n, i, a); }
+    if (sig_inf) jac_set_identity(rsig); else { g2_aff sg; soa_load_g2(sg, sig_soa, n, i); jac_mul_u64(rsig, sg, r); }
+}
 // pk <- [r] pk (affine, in place); rsig <- [r] sig (Jacobian); pair 0 of the Miller loop is switched off for the item
 __global__ void __launch_bounds__(TPB, BLS_MINB) k_rlc_scale(u32x4* pk_soa, const u32x4* sig_soa, uint8_t* flags, const uint8_t* status, size_t n, size_t idx0,
                                                               const uint8_t* seed16, u32x4* rsig_jac) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     g2_jac rs; jac_set_identity(rs);
     if (status[i] == ST_OK) {
-        uint64_t r = rlc_scalar(seed16, idx0 + i);
         g1_aff pk; soa_load_g1(pk, pk_soa, n, i);
-        g1_jac rp; jac_mul_u64(rp, pk, r);
-        g1_aff a; jac_to_aff(a, rp); soa_store_g1(pk_soa, n, i, a);          // pk has prime order r > 2^64: [r]pk is never the identity
-        if (!(flags[i] & FL_SIG_INF)) { g2_aff sg; soa_load_g2(sg, sig_soa, n, i); jac_mul_u64(rs, sg, r); }
+        rlc_scale_item(pk_soa, sig_soa, n, i, pk, (flags[i] & FL_SIG_INF) != 0, seed16, idx0 + i, rs);
         flags[i] |= FL_SIG_INF;
     }
     segsum_traits<fp2>::storej(rsig_jac, n, i, rs);
@@ -1150,6 +1158,40 @@ int blsgpu_verify_batch_rlc(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t*
 // whose equation fails is re-run through the per-item path (blsgpu_verify_batch) inside this call.  status[i] and ok_bitmap equal
 // blsgpu_verify_batch's except with probability <= 2^-64 per failing piece over the seed; fallback_items (nullable, host) = items re-run.
 #define RLC_PIECE 4096
+// The per-piece equations of a pass of m items whose weights are applied (pk_soa = [r] pk, rs = [r] sig, pair 0 switched off in flags):
+// per-piece sums of the scaled signatures and products of the Miller values (radix-8 trees, all pieces in one launch per level), then
+// ok[p] for every piece.  ja, jb: 18 P T0 rows, ta, tb: 36 P T0 rows (T0 = RLC_PIECE / 8); the split Miller loop takes its state from the workspace.
+static int rlc_pieces(blsgpu_ctx* ctx, const u32x4* rs, const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags, uint8_t* dstatus, size_t m,
+                      u32x4* f_soa, u32x4* ja, u32x4* jb, u32x4* ta, u32x4* tb, uint8_t* dok) {
+    const size_t L = RLC_PIECE, P = (m + L - 1) / L;
+    const u32x4* s_piece; const u32x4* f_piece;
+    {   // per-piece sums of the scaled signatures: radix-8 trees, all pieces in one launch per level
+        const u32x4* cur = rs; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ja, jb}; int which = 0;
+        while (true) {
+            size_t T = (len + 7) / 8; u32x4* out = bufs[which];
+            k_g2_jac_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
+            cur = out; cnt_n = P * T; len = T; which ^= 1;
+            if (T == 1) break;
+        }
+        s_piece = cur;
+    }
+    if (ctx->split) {
+        u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
+        if (int rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr)) return rc;
+    } else LAUNCH(k_miller, nblk(m), TPB, pk_soa, hm_soa, sig_soa, flags, (const uint8_t*)dstatus, m, f_soa);
+    {
+        const u32x4* cur = f_soa; const uint8_t* st = dstatus; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ta, tb}; int which = 0;
+        while (true) {
+            size_t T = (len + 7) / 8; u32x4* out = bufs[which];
+            k_gt_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, st, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
+            cur = out; st = nullptr; cnt_n = P * T; len = T; which ^= 1;
+            if (T == 1) break;
+        }
+        f_piece = cur;
+    }
+    LAUNCH(k_rlc_finish_seg, (unsigned)P, 32, f_piece, s_piece, P, dok);
+    return 0;
+}
 int blsgpu_verify_batch_rlc_bisect(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t n,
                                    const uint8_t seed16[16], uint8_t* status, uint64_t* ok_bitmap, uint64_t* fallback_items) {
     ENTER(); if (!pk48 || !msg || !sig96 || !seed16 || !status) return fail(ctx, BLSGPU_ERR_ARG, "null pointer");
@@ -1186,32 +1228,7 @@ int blsgpu_verify_batch_rlc_bisect(blsgpu_ctx* ctx, const uint8_t* pk48, const u
         LAUNCH(k_decode_g2<true>, nblk(m), TPB, dsig, m, sig_soa, code_sig);
         if ((rc = hash_stage(ctx, dmsg, doff, m, code_pk, code_sig, hm_soa, f_soa, flags, dstatus))) return rc;
         LAUNCH(k_rlc_scale, nblk(m), TPB, pk_soa, (const u32x4*)sig_soa, flags, (const uint8_t*)dstatus, m, base, (const uint8_t*)dseed, rs);
-        const u32x4* s_piece; const u32x4* f_piece;
-        {   // per-piece sums of the scaled signatures: radix-8 trees, all pieces in one launch per level
-            const u32x4* cur = rs; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ja, jb}; int which = 0;
-            while (true) {
-                size_t T = (len + 7) / 8; u32x4* out = bufs[which];
-                k_g2_jac_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
-                cur = out; cnt_n = P * T; len = T; which ^= 1;
-                if (T == 1) break;
-            }
-            s_piece = cur;
-        }
-        if (ctx->split) {
-            u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
-            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr))) return rc;
-        } else LAUNCH(k_miller, nblk(m), TPB, (const u32x4*)pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, m, f_soa);
-        {
-            const u32x4* cur = f_soa; const uint8_t* st = dstatus; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ta, tb}; int which = 0;
-            while (true) {
-                size_t T = (len + 7) / 8; u32x4* out = bufs[which];
-                k_gt_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, st, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
-                cur = out; st = nullptr; cnt_n = P * T; len = T; which ^= 1;
-                if (T == 1) break;
-            }
-            f_piece = cur;
-        }
-        LAUNCH(k_rlc_finish_seg, (unsigned)P, 32, f_piece, s_piece, P, dok);
+        if ((rc = rlc_pieces(ctx, rs, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, ja, jb, ta, tb, dok))) return rc;
         if ((rc = finish_out(ctx, status + base, dstatus, m))) return rc;
         CU(cudaMemcpyAsync(piece_ok.data() + base / L, dok, P, cudaMemcpyDeviceToHost, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
@@ -1316,7 +1333,7 @@ int blsgpu_g1_aggregate(blsgpu_ctx* ctx, const uint8_t* pts48, const uint32_t* s
     uint8_t* dout = stage_out(ctx, out48, 48 * nseg); uint8_t* dst = stage_out(ctx, status, nseg);
     if (npts) LAUNCH(k_decode_g1, nblk(npts), TPB, din, npts, soa, code);
     { int L = seg_lanes(npts / nseg); u32x4* ojac = ws_take<u32x4>(ctx, 9 * nseg);
-      LAUNCH(k_segsum<fp>, nblk(nseg, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, dseg, (size_t)0, (const uint64_t*)nullptr, nseg, ojac, dst, (uint8_t)ST_BAD_PK, (const uint32_t*)nullptr, L);
+      LAUNCH(k_segsum<fp>, nblk(nseg, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, dseg, (size_t)0, (const uint64_t*)nullptr, nseg, ojac, dst, (uint8_t)ST_BAD_PK, (const uint32_t*)nullptr, L, (size_t)0);
       LAUNCH(k_jac_to_aff<fp>, nblk(nseg), TPB, (const u32x4*)ojac, nseg, osoa, oinf); }
     LAUNCH(k_encode_g1, nblk(nseg), TPB, (const u32x4*)osoa, (const uint8_t*)oinf, nseg, dout);
     if (int rc = finish_out(ctx, out48, dout, 48 * nseg)) return rc; if (int rc = finish_out(ctx, status, dst, nseg)) return rc;
@@ -1335,7 +1352,7 @@ int blsgpu_g2_aggregate(blsgpu_ctx* ctx, const uint8_t* pts96, const uint32_t* s
     uint8_t* dout = stage_out(ctx, out96, 96 * nseg); uint8_t* dst = stage_out(ctx, status, nseg);
     if (npts) LAUNCH(k_decode_g2<true>, nblk(npts), TPB, din, npts, soa, code);
     { int L = seg_lanes(npts / nseg); u32x4* ojac = ws_take<u32x4>(ctx, 18 * nseg);
-      LAUNCH(k_segsum<fp2>, nblk(nseg, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, dseg, (size_t)0, (const uint64_t*)nullptr, nseg, ojac, dst, (uint8_t)ST_BAD_SIG, (const uint32_t*)nullptr, L);
+      LAUNCH(k_segsum<fp2>, nblk(nseg, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, dseg, (size_t)0, (const uint64_t*)nullptr, nseg, ojac, dst, (uint8_t)ST_BAD_SIG, (const uint32_t*)nullptr, L, (size_t)0);
       LAUNCH(k_jac_to_aff<fp2>, nblk(nseg), TPB, (const u32x4*)ojac, nseg, osoa, oinf); }
     LAUNCH(k_encode_g2, nblk(nseg), TPB, (const u32x4*)osoa, (const uint8_t*)oinf, (uint8_t)1, nseg, dout);
     if (int rc = finish_out(ctx, out96, dout, 96 * nseg)) return rc; if (int rc = finish_out(ctx, status, dst, nseg)) return rc;
@@ -1357,7 +1374,7 @@ int blsgpu_fast_aggregate_verify_batch(blsgpu_ctx* ctx, const uint8_t* pks48, co
     uint8_t* dstatus = stage_out(ctx, status, ncomm); uint8_t* dagg = stage_out(ctx, agg_pk48_out, 48 * ncomm);
     if (npts) LAUNCH(k_decode_g1, nblk(npts), TPB, dpks, npts, soa, code);
     { int L = seg_lanes(k); u32x4* ojac = ws_take<u32x4>(ctx, 9 * ncomm);
-      LAUNCH(k_segsum<fp>, nblk(ncomm, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, (const uint32_t*)nullptr, k, dbm, ncomm, ojac, agg_st, (uint8_t)ST_BAD_PK, (const uint32_t*)nullptr, L);
+      LAUNCH(k_segsum<fp>, nblk(ncomm, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)soa, (const uint8_t*)code, npts, (const uint32_t*)nullptr, k, dbm, ncomm, ojac, agg_st, (uint8_t)ST_BAD_PK, (const uint32_t*)nullptr, L, (size_t)0);
       LAUNCH(k_jac_to_aff<fp>, nblk(ncomm), TPB, (const u32x4*)ojac, ncomm, agg_soa, agg_inf); }
     if (dagg) LAUNCH(k_encode_g1, nblk(ncomm), TPB, (const u32x4*)agg_soa, (const uint8_t*)agg_inf, ncomm, dagg);
     LAUNCH(k_fav_status, nblk(ncomm), TPB, (const uint8_t*)agg_st, (const uint8_t*)agg_inf, (const uint8_t*)nullptr, ncomm, code_pk);
@@ -1457,7 +1474,7 @@ int blsgpu_pool_fast_aggregate_verify(blsgpu_ctx* ctx, int handle, const uint32_
     uint8_t* dstatus = stage_out(ctx, status, ncomm); uint8_t* dagg = stage_out(ctx, agg_pk48_out, 48 * ncomm);
     { int L = seg_lanes(k); u32x4* ojac = ws_take<u32x4>(ctx, 9 * ncomm);
       LAUNCH(k_segsum<fp>, nblk(ncomm, SEG_WARPS * (32 / L)), 32 * SEG_WARPS, (const u32x4*)ctx->pool[handle].soa, (const uint8_t*)ctx->pool[handle].code, ctx->pool[handle].n, (const uint32_t*)nullptr, k, dbm, ncomm,
-             ojac, agg_st, (uint8_t)ST_BAD_PK, didx, L);
+             ojac, agg_st, (uint8_t)ST_BAD_PK, didx, L, (size_t)0);
       LAUNCH(k_jac_to_aff<fp>, nblk(ncomm), TPB, (const u32x4*)ojac, ncomm, agg_soa, agg_inf); }
     if (dagg) LAUNCH(k_encode_g1, nblk(ncomm), TPB, (const u32x4*)agg_soa, (const uint8_t*)agg_inf, ncomm, dagg);
     LAUNCH(k_fav_status, nblk(ncomm), TPB, (const uint8_t*)agg_st, (const uint8_t*)agg_inf, (const uint8_t*)nullptr, ncomm, code_pk);
@@ -1468,6 +1485,7 @@ int blsgpu_pool_fast_aggregate_verify(blsgpu_ctx* ctx, int handle, const uint32_
 
 }  // extern "C"
 
+#include "sets.cuh"
 #include "r1cs.cuh"
 #include "witness.cuh"
 #include "multi.cuh"

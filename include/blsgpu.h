@@ -145,6 +145,28 @@ int blsgpu_pool_free(blsgpu_ctx* ctx, int handle);
 int blsgpu_pool_fast_aggregate_verify(blsgpu_ctx* ctx, int handle, const uint32_t* idx /* ncomm*k */, const uint64_t* bitmap, size_t k,
                                       const uint8_t* msg32, const uint8_t* sig96, size_t ncomm, uint8_t* status, uint8_t* agg_pk48_out);
 
+/* ---- signature sets (the shape of Lighthouse's verify_signature_sets / blst's verify_multiple_aggregate_signatures): set s = the keys
+ *      [key_off[s], key_off[s+1]) of pks48 (bitmap, nullable: bit i of the FLAT key list selects key i), the message
+ *      msg[msg_off[s] .. msg_off[s+1]) (msg_off NULL = fixed 32-byte messages) and the signature sig96[s].  Committees of any size, messages of any length.
+ * status[s] = exactly what blsgpu_fast_aggregate_verify_batch reports for that set:
+ *   0 / 1 = pairing check true / false;
+ *   2 = a selected key fails to decode / is outside the subgroup, no key is selected, or the aggregate is the identity;
+ *   3 = the signature fails to decode / is outside the subgroup.
+ * seed16 NULL: every set gets its own pairing check.
+ * seed16 set:  one random-linear-combination equation per piece of 4,096 sets, r_s = 64 non-zero bits of SHA-256(seed16 || le64(s)) (the derivation of
+ *              blsgpu_verify_batch_rlc); pieces whose equation fails are re-run per set inside the call, so status equals the seed16 == NULL outcome
+ *              except with probability <= 2^-64 per failing piece.  The seed must be unpredictable to whoever produced the sets.
+ * ok_bitmap (nullable): ceil(nsets/64) words, bit s set <=> status[s] == 0.  fallback_sets (nullable, HOST memory): sets re-run per set.
+ * In device pointer mode key_off is read back to the host once (the internal passes are planned there); a decreasing key_off is BLSGPU_ERR_ARG. */
+int blsgpu_verify_signature_sets(blsgpu_ctx* ctx, const uint8_t* pks48, const uint32_t* key_off, const uint64_t* bitmap,
+                                 const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t nsets,
+                                 const uint8_t* seed16, uint8_t* status, uint64_t* ok_bitmap, uint64_t* fallback_sets);
+/* the same with the keys given as indices into a resident pool (blsgpu_pool_create); an out-of-range index or an undecodable pool key
+ * makes its set 2 (as blsgpu_pool_fast_aggregate_verify) */
+int blsgpu_pool_verify_signature_sets(blsgpu_ctx* ctx, int handle, const uint32_t* idx, const uint32_t* key_off, const uint64_t* bitmap,
+                                      const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t nsets,
+                                      const uint8_t* seed16, uint8_t* status, uint64_t* ok_bitmap, uint64_t* fallback_sets);
+
 /* ---- hash_to_g2  (src/bls.rs:477-493; algorithm spec src/hasher.rs:58-173, 352-502, 294-348, 664-673) ------- */
 int blsgpu_hash_to_g2_batch(blsgpu_ctx* ctx, const uint8_t* msg, const uint32_t* msg_off, size_t n, uint8_t* out96);
 

@@ -153,6 +153,18 @@ struct BLS {                                                                    
         size_t n = sig96.size() / 96; std::vector<uint8_t> st(n);
         c.check(blsgpu_verify_batch(c.raw(), pk48.data(), msg32.data(), nullptr, sig96.data(), n, st.data(), nullptr, nullptr)); return st;
     }
+    // signature sets (no reference counterpart; blsgpu_verify_signature_sets): set s = keys [key_off[s], key_off[s+1]) of pks48, message
+    // msg[msg_off[s] .. msg_off[s+1]), signature s -> status per set.  seed16 (nullable): random-linear-combination form with the exact outcome.
+    static std::vector<uint8_t> verify_signature_sets(const std::vector<uint8_t>& pks48, const std::vector<uint32_t>& key_off, const std::vector<uint8_t>& msg,
+                                                      const std::vector<uint32_t>& msg_off, const std::vector<uint8_t>& sig96, const uint8_t* seed16 = nullptr,
+                                                      const uint64_t* bitmap = nullptr, uint64_t* fallback_sets = nullptr, Context& c = default_context()) {
+        size_t n = sig96.size() / 96; std::vector<uint8_t> st(n);
+        if (key_off.size() != n + 1 || msg_off.size() != n + 1 || key_off[n] > pks48.size() / 48 || msg_off[n] > msg.size()) throw std::invalid_argument("key_off / msg_off do not match the buffers");
+        uint8_t dummy = 0;
+        c.check(blsgpu_verify_signature_sets(c.raw(), pks48.empty() ? &dummy : pks48.data(), key_off.data(), bitmap, msg.empty() ? &dummy : msg.data(), msg_off.data(),
+                                             sig96.data(), n, seed16, st.data(), nullptr, fallback_sets));
+        return st;
+    }
 };
 
 }  // namespace blsgpu

@@ -38,6 +38,13 @@ extern "C" {
     // Eth2 aggregate_verify (distinct messages; tests/readme.md:4-7 names the category): one signature over k (pk_j, msg_j) pairs
     pub fn blsgpu_aggregate_verify_batch(ctx: *mut blsgpu_ctx, pks48: *const u8, msg: *const u8, msg_off: *const u32, pair_off: *const u32,
                                          sig96: *const u8, nsig: usize, status: *mut u8) -> c_int;
+    // signature sets (Lighthouse verify_signature_sets / blst verify_multiple_aggregate_signatures shape): keys [key_off[s], key_off[s+1]),
+    // one message and one signature per set; seed16 non-null = per-piece random-linear-combination equations with the exact per-set outcome
+    pub fn blsgpu_verify_signature_sets(ctx: *mut blsgpu_ctx, pks48: *const u8, key_off: *const u32, bitmap: *const u64, msg: *const u8, msg_off: *const u32,
+                                        sig96: *const u8, nsets: usize, seed16: *const u8, status: *mut u8, ok_bitmap: *mut u64, fallback_sets: *mut u64) -> c_int;
+    pub fn blsgpu_pool_verify_signature_sets(ctx: *mut blsgpu_ctx, handle: c_int, idx: *const u32, key_off: *const u32, bitmap: *const u64, msg: *const u8,
+                                             msg_off: *const u32, sig96: *const u8, nsets: usize, seed16: *const u8, status: *mut u8, ok_bitmap: *mut u64,
+                                             fallback_sets: *mut u64) -> c_int;
     pub fn blsgpu_hash_to_g2_batch(ctx: *mut blsgpu_ctx, msg: *const u8, msg_off: *const u32, n: usize, out96: *mut u8) -> c_int;          // src/bls.rs:477-493
     pub fn blsgpu_g1_aggregate(ctx: *mut blsgpu_ctx, pts48: *const u8, seg_off: *const u32, nseg: usize, out48: *mut u8, status: *mut u8) -> c_int;   // src/bls.rs:183-195
     pub fn blsgpu_g2_aggregate(ctx: *mut blsgpu_ctx, pts96: *const u8, seg_off: *const u32, nseg: usize, out96: *mut u8, status: *mut u8) -> c_int;   // src/bls.rs:288-300

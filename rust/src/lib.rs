@@ -214,6 +214,23 @@ pub fn verify_batch(pk48: &[u8], messages: &[u8], msg_off: &[u32], sig96: &[u8])
     check(c, rc)?; Ok(st)
 }
 
+/// Signature sets: set s = the keys `pk48[key_off[s]..key_off[s+1]]` (48 bytes each), the message `messages[msg_off[s]..msg_off[s+1]]` and
+/// `sig96[s]`.  `status[s]` as [`verify_batch`] for the set's aggregate key (2 also for an empty set or an identity aggregate).  `seed16`:
+/// `Some` = one random-linear-combination equation per 4,096 sets with the failing pieces re-run per set inside the library (same status except with
+/// probability <= 2^-64 per failing piece; the seed must be unpredictable to whoever produced the sets).  -> (status, sets re-run per set)
+pub fn verify_signature_sets(pk48: &[u8], key_off: &[u32], messages: &[u8], msg_off: &[u32], sig96: &[u8], seed16: Option<&[u8; 16]>) -> Result<(Vec<u8>, u64), Error> {
+    let n = sig96.len() / 96;
+    assert!(sig96.len() == 96 * n && key_off.len() == n + 1 && msg_off.len() == n + 1 && key_off.windows(2).all(|w| w[0] <= w[1]));
+    assert!(48 * *key_off.last().unwrap() as usize <= pk48.len() && *msg_off.last().unwrap() as usize <= messages.len());
+    let mut st = vec![0u8; n]; let mut rerun = 0u64;
+    let dummy = [0u8; 1];
+    let pk = if pk48.is_empty() { dummy.as_ptr() } else { pk48.as_ptr() }; let m = if messages.is_empty() { dummy.as_ptr() } else { messages.as_ptr() };
+    let seed = seed16.map_or(std::ptr::null(), |s| s.as_ptr());
+    let (c, rc) = with_ctx(|c| (c, unsafe { blsgpu_verify_signature_sets(c, pk, key_off.as_ptr(), std::ptr::null(), m, msg_off.as_ptr(), sig96.as_ptr(), n, seed,
+                                                                         st.as_mut_ptr(), std::ptr::null_mut(), &mut rerun) }))?;
+    check(c, rc)?; Ok((st, rerun))
+}
+
 /// Every GPU of the box (blsgpu_create_multi): contiguous shards, NCCL all-gather of the bitmap shards and GT partials inside the library.
 pub struct MultiGpu(*mut blsgpu_multi);
 impl MultiGpu {
