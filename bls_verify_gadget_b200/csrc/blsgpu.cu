@@ -8,7 +8,8 @@
 //                                   in verify_batch the last pair of launches also tests sig in G2 on the running point [|x|] sig -> ST_BAD_SIG
 //   k_final_exp                 K5  Fp12 -> GT, is_one -> status                   | split form: k_final_step<0>, 5 x (k_final_squarings -> k_final_step<k>)
 //   k_miller_accum_coop, k_final_hard_coop   six lanes per item: passes of at most VERIFY_COOP_BELOW items (latency), blsgpu_set_coop
-//   k_gt_reduce                 K5' strided product of GT values (per-batch accumulator)
+//   k_gt_reduce_seg             K5' strided product of GT values per piece (one piece: the per-batch accumulator) | k_g2_jac_reduce_seg: sums of G2 points
+//   k_rlc_scale, k_rlc_finish_seg   random-linear-combination checks: [r] pk and [r] sig per item; one equation per piece
 //   k_status_bitmap                 status -> packed ok bitmap
 //   k_segsum_g1 / k_segsum_g2   K3  warp-per-segment aggregation, tree reduction in shared memory
 //   k_sets_rlc_prep                 signature sets, RLC form: status rule of the aggregate, [r] aggregate key, [r] signature (sets.cuh)
@@ -140,19 +141,25 @@ template <bool SUBGROUP> __global__ void __launch_bounds__(TPB, BLS_MINB_DG2) k_
     if (soa) soa_store_g2(soa, n, i, p);
     code[i] = (uint8_t)rc;
 }
-// status/flags from the two decode codes (bls.rs:434-447), then H(m) for the items still alive
+// the status / flags rule of the verify paths from the two decode codes (bls.rs:434-447): a bad key wins over a bad signature, and an
+// identity signature switches pair 0 of the Miller loop off.  st and fl keep their values when the rule leaves them alone.
+__device__ __forceinline__ void decode_status(const uint8_t* code_pk, const uint8_t* code_sig, size_t i, uint8_t& st, uint8_t& fl) {
+    if (code_pk[i] != DEC_OK) st = ST_BAD_PK;
+    else if (code_sig[i] != DEC_OK && code_sig[i] != DEC_INF) st = ST_BAD_SIG;
+    else if (code_sig[i] == DEC_INF) fl = FL_SIG_INF;
+}
+// message i of (msg, off): off[i] .. off[i + 1] are absolute offsets into msg; off == NULL: 32-byte messages
+__device__ __forceinline__ void item_msg(const uint8_t* msg, const uint32_t* off, size_t i, const uint8_t*& m, uint32_t& len) {
+    if (off) { m = msg + off[i]; len = off[i + 1] - off[i]; } else { m = msg + 32 * i; len = 32; }
+}
+// status/flags from the two decode codes, then H(m) for the items still alive
 __global__ void __launch_bounds__(TPB, BLS_MINB_HASH) k_hash_to_g2(const uint8_t* msg, const uint32_t* off, size_t n, const uint8_t* code_pk, const uint8_t* code_sig,
                                                     u32x4* hm_soa, uint8_t* flags, uint8_t* status) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     uint8_t st = ST_OK, fl = 0;
-    if (code_pk) {
-        if (code_pk[i] != DEC_OK) st = ST_BAD_PK;
-        else if (code_sig[i] != DEC_OK && code_sig[i] != DEC_INF) st = ST_BAD_SIG;
-        else if (code_sig[i] == DEC_INF) fl = FL_SIG_INF;
-    }
+    if (code_pk) decode_status(code_pk, code_sig, i, st, fl);
     if (st == ST_OK) {
-        const uint8_t* m; uint32_t len;
-        if (off) { m = msg + off[i]; len = off[i + 1] - off[i]; } else { m = msg + 32 * i; len = 32; }
+        const uint8_t* m; uint32_t len; item_msg(msg, off, i, m, len);
         g2_aff hm; uint8_t f2; stage_hash(hm, f2, m, len);
         soa_store_g2(hm_soa, n, i, hm); fl |= f2;
     }
@@ -164,14 +171,9 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_HFIELD) k_hash_field(const uint8
                                                                u32x4* u_soa, uint8_t* flags, uint8_t* status) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     uint8_t st = ST_OK, fl = 0;
-    if (code_pk) {
-        if (code_pk[i] != DEC_OK) st = ST_BAD_PK;
-        else if (code_sig[i] != DEC_OK && code_sig[i] != DEC_INF) st = ST_BAD_SIG;
-        else if (code_sig[i] == DEC_INF) fl = FL_SIG_INF;
-    }
+    if (code_pk) decode_status(code_pk, code_sig, i, st, fl);
     if (st == ST_OK) {
-        const uint8_t* m; uint32_t len;
-        if (off) { m = msg + off[i]; len = off[i + 1] - off[i]; } else { m = msg + 32 * i; len = 32; }
+        const uint8_t* m; uint32_t len; item_msg(msg, off, i, m, len);
         fp2 u0, u1; hash_to_field(u0, u1, m, len);
         soa_store_fp2(u_soa, n, i, 0, u0); soa_store_fp2(u_soa, n, i, 1, u1);
     }
@@ -181,9 +183,7 @@ __global__ void __launch_bounds__(TPB, BLS_MINB_HFIELD) k_hash_field(const uint8
 __global__ void k_status_merge(const uint8_t* code_pk, const uint8_t* code_sig, size_t n, uint8_t* flags, uint8_t* status) {
     size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (i >= n) return;
     uint8_t st = ST_OK, fl = 0;
-    if (code_pk[i] != DEC_OK) st = ST_BAD_PK;
-    else if (code_sig[i] != DEC_OK && code_sig[i] != DEC_INF) st = ST_BAD_SIG;
-    else if (code_sig[i] == DEC_INF) fl = FL_SIG_INF;
+    decode_status(code_pk, code_sig, i, st, fl);
     flags[i] = (uint8_t)((flags[i] & FL_HM_INF) | fl); status[i] = st;
 }
 __global__ void __launch_bounds__(TPB, BLS_MINB_HMAP) k_hash_map(const u32x4* u_soa, const uint8_t* status, size_t n, u32x4* q_soa) {
@@ -383,16 +383,6 @@ __global__ void __launch_bounds__(128, 2) k_miller_accum_coop(const uint8_t* fla
     if (active && i_lo == 0 && sig_sub && use[0] && !sig_sub[item]) { if (c.k == 0) status[item] = ST_BAD_SIG; return; }
     if (active) soa_store_fp2(f_soa, n, item, COOP_TOWER_POS[c.k], f);
 }
-// out[t] = prod_{i = t, t+T, ...} in[i] over items with status <= ST_FALSE (status == NULL: all items)
-__global__ void __launch_bounds__(TPB, BLS_MINB) k_gt_reduce(const u32x4* in_soa, const uint8_t* status, size_t n, u32x4* out_soa, size_t T) {
-    size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (t >= T) return;
-    fp12 acc, x; fp12_one(acc);
-    for (size_t i = t; i < n; i += T) {
-        if (status && status[i] > ST_FALSE) continue;
-        soa_load_fp12(x, in_soa, n, i); fp12_mul(acc, acc, x);
-    }
-    soa_store_fp12(out_soa, T, t, acc);
-}
 __global__ void k_gt_mul_into(u32x4* acc_soa, const u32x4* x_soa) {      // single thread: acc *= x
     if (threadIdx.x || blockIdx.x) return;
     fp12 a, x; soa_load_fp12(a, acc_soa, 1, 0); soa_load_fp12(x, x_soa, 1, 0); fp12_mul(a, a, x); soa_store_fp12(acc_soa, 1, 0, a);
@@ -556,13 +546,6 @@ __global__ void __launch_bounds__(TPB, BLS_MINB) k_rlc_scale(u32x4* pk_soa, cons
     }
     segsum_traits<fp2>::storej(rsig_jac, n, i, rs);
 }
-// out[t] = sum_{i = t, t+T, ...} in[i] (Jacobian G2)
-__global__ void __launch_bounds__(TPB, BLS_MINB) k_g2_jac_reduce(const u32x4* in_jac, size_t n, u32x4* out_jac, size_t T) {
-    size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; if (t >= T) return;
-    g2_jac acc, x; jac_set_identity(acc);
-    for (size_t i = t; i < n; i += T) { segsum_traits<fp2>::loadj(x, in_jac, n, i); jac_add(acc, acc, x); }
-    segsum_traits<fp2>::storej(out_jac, T, t, acc);
-}
 __global__ void k_g2_jac_add_into(u32x4* acc_jac, const u32x4* x_jac) {
     if (threadIdx.x || blockIdx.x) return;
     g2_jac a, x; segsum_traits<fp2>::loadj(a, acc_jac, 1, 0); segsum_traits<fp2>::loadj(x, x_jac, 1, 0); jac_add(a, a, x); segsum_traits<fp2>::storej(acc_jac, 1, 0, a);
@@ -574,21 +557,8 @@ __global__ void k_any_bad(const uint8_t* status, size_t n, uint32_t* bad) {
     bool b = i < n && status[i] != ST_OK;
     if (__any_sync(0xffffffffu, b) && (threadIdx.x & 31) == 0) atomicOr(bad, 1u);
 }
-// single thread: F * miller(-g1, S), final exponentiation, is_one
-__global__ void __launch_bounds__(32, 1) k_rlc_finish(const u32x4* f_acc, const u32x4* s_jac, const uint32_t* bad, uint8_t* all_ok) {
-    if (threadIdx.x || blockIdx.x) return;
-    fp12 F, f2, gt; soa_load_fp12(F, f_acc, 1, 0);
-    g2_jac S; segsum_traits<fp2>::loadj(S, s_jac, 1, 0);
-    g2_aff sa; bool have = jac_to_aff(sa, S);
-    g1_aff ng; ng.x = fp_const(C_G1X); ng.y = fp_const(C_G1Y_NEG);
-    miller_loop2(f2, ng, sa, have, ng, sa, false);
-    fp12_mul(F, F, f2);
-    final_exponentiation(gt, F);
-    all_ok[0] = (fp12_is_one(gt) && !bad[0]) ? 1 : 0;
-}
-
-// ---- per-piece forms for the bisecting batch check: the batch is cut into pieces of L items; products / sums are kept per piece
-// out[p * T + t] = prod_{i = t, t + T, ... < len_p} in[p * L + i]   (len_p = min(L, n - p L); status filter as k_gt_reduce)
+// ---- reduction trees over pieces of L items (one piece of L = n for a whole batch); products / sums are kept per piece
+// out[p * T + t] = prod_{i = t, t + T, ... < len_p} in[p * L + i]   (len_p = min(L, n - p L)) over items with status <= ST_FALSE (status == NULL: all items)
 __global__ void __launch_bounds__(TPB, BLS_MINB) k_gt_reduce_seg(const u32x4* in_soa, const uint8_t* status, size_t n, size_t L, u32x4* out_soa, size_t T, size_t P) {
     size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x, p = blockIdx.y; if (t >= T) return;
     size_t lo = p * L, hi = lo + L < n ? lo + L : n;
@@ -607,8 +577,8 @@ __global__ void __launch_bounds__(TPB, BLS_MINB) k_g2_jac_reduce_seg(const u32x4
     segsum_traits<fp2>::storej(out_jac, P * T, p * T + t, acc);
 }
 // one block per piece (thread 0 works): ok[p] = [ F_p * miller(-g1, S_p) ]^((p^12-1)/r) == 1  -- the pieces' finishes run side by side,
-// so locating the failing pieces costs one single-thread latency (~20 ms) whatever their number
-__global__ void __launch_bounds__(32, 1) k_rlc_finish_seg(const u32x4* f_piece, const u32x4* s_piece, size_t P, uint8_t* ok) {
+// so locating the failing pieces costs one single-thread latency (~20 ms) whatever their number.  bad (nullable): bad[0] != 0 fails every piece.
+__global__ void __launch_bounds__(32, 1) k_rlc_finish_seg(const u32x4* f_piece, const u32x4* s_piece, size_t P, const uint32_t* bad, uint8_t* ok) {
     size_t p = blockIdx.x; if (threadIdx.x || p >= P) return;
     fp12 F, f2, gt; soa_load_fp12(F, f_piece, P, p);
     g2_jac S; segsum_traits<fp2>::loadj(S, s_piece, P, p);
@@ -617,7 +587,7 @@ __global__ void __launch_bounds__(32, 1) k_rlc_finish_seg(const u32x4* f_piece, 
     miller_loop2(f2, ng, sa, have, ng, sa, false);
     fp12_mul(F, F, f2);
     final_exponentiation(gt, F);
-    ok[p] = fp12_is_one(gt) ? 1 : 0;
+    ok[p] = (fp12_is_one(gt) && !(bad && bad[0])) ? 1 : 0;
 }
 
 // ---- uncompressed <-> compressed point encodings (K7'): status = BLSGPU_DE_* of the INPUT; an undecodable input gives an all-zero output
@@ -724,15 +694,50 @@ static size_t msg_bytes_total(blsgpu_ctx* ctx, const uint32_t* off, size_t n, in
     return last;
 }
 
-// GT product of n values (limb-SoA, filtered by status) into a single value at dst (limb-SoA, n = 1)
-static int gt_product(blsgpu_ctx* ctx, const u32x4* in_soa, const uint8_t* status, size_t n, u32x4* tmp_a, u32x4* tmp_b, u32x4* dst) {
-    const u32x4* cur = in_soa; size_t cnt = n; const uint8_t* st = status; u32x4* bufs[2] = {tmp_a, tmp_b}; int which = 0;
-    while (true) {
-        size_t T = (cnt + 7) / 8;                       // radix-8 tree: every pass multiplies 8 values per thread
-        u32x4* out = T == 1 ? dst : bufs[which];
-        LAUNCH(k_gt_reduce, nblk(T), TPB, cur, st, cnt, out, T);
+// A batch of items whose message offsets are absolute into msg (msg_off NULL: 32-byte messages); pk48 is NULL for signature sets.
+struct batch_in { const uint8_t* pk48; const uint8_t* msg; const uint32_t* msg_off; const uint8_t* sig96; };
+struct batch_dev { const uint8_t *pk48, *msg, *sig96; const uint32_t* msg_off; };
+// message bytes that a pass over items [lo, hi) stages: host mode copies them, device mode uses msg as it is (0)
+static size_t pass_msg_bytes(const blsgpu_ctx* ctx, const batch_in& in, size_t lo, size_t hi) {
+    if (ctx->ptr_mode != BLSGPU_HOST) return 0;
+    return in.msg_off ? in.msg_off[hi] - in.msg_off[lo] : 32 * (hi - lo);
+}
+// workspace of stage_items over m items with mb = pass_msg_bytes, plus the m status bytes of the pass
+static size_t stage_ws_bytes(size_t m, size_t mb) { return al(48 * m) + al(96 * m) + al(mb + 1) + al(4 * (m + 1)) + al(m); }
+// the device views of items [lo, hi).  The offsets stay absolute: host mode copies the range's message bytes only and rebases msg by the
+// range's first offset instead, so a kernel reads message i at msg + msg_off[i] in both modes.
+static int stage_items(blsgpu_ctx* ctx, const batch_in& in, size_t lo, size_t hi, batch_dev& d) {
+    size_t m = hi - lo, mb0 = in.msg_off ? (ctx->ptr_mode == BLSGPU_HOST ? in.msg_off[lo] : 0) : 32 * lo, mb = pass_msg_bytes(ctx, in, lo, hi);
+    if (int rc = stage_in(ctx, d.pk48, in.pk48 ? in.pk48 + 48 * lo : nullptr, 48 * m)) return rc;
+    if (int rc = stage_in(ctx, d.sig96, in.sig96 + 96 * lo, 96 * m)) return rc;
+    if (int rc = stage_in(ctx, d.msg, in.msg + mb0, mb ? mb : 1)) return rc;
+    if (in.msg_off) d.msg -= mb0;
+    return stage_in(ctx, d.msg_off, in.msg_off ? in.msg_off + lo : nullptr, m + 1);
+}
+
+// Radix-8 reduction trees over the pieces of L items of n values (L = n: one piece), all pieces in one launch per level: GT products of
+// the Miller values of the items with status <= ST_FALSE (status == NULL: all), or sums of Jacobian G2 points.  Level by level into a, b,
+// a, ... (a: ceil(L / 8) P rows, b: ceil(L / 64) P rows) until one value per piece is left; out = those P values (P rows, in a or b).
+template <bool GT> static int piece_tree(blsgpu_ctx* ctx, const u32x4* in, const uint8_t* status, size_t n, size_t L, u32x4* a, u32x4* b, const u32x4*& out) {
+    const size_t P = (n + L - 1) / L; u32x4* bufs[2] = {a, b};
+    for (int w = 0; ; w ^= 1) {
+        size_t T = (L + 7) / 8; dim3 grid(nblk(T), (unsigned)P);
+        if (GT) LAUNCH(k_gt_reduce_seg, grid, TPB, in, status, n, L, bufs[w], T, P);
+        else LAUNCH(k_g2_jac_reduce_seg, grid, TPB, in, n, L, bufs[w], T, P);
+        in = bufs[w]; status = nullptr; n = P * T; L = T;
         if (T == 1) break;
-        cur = out; cnt = T; st = nullptr; which ^= 1;
+    }
+    out = in; return 0;
+}
+// the exact fallback of the piece-wise checks: fn(lo, hi) re-runs each range of adjacent failing pieces; rerun = items re-run
+template <class Fn> static int rerun_failing_pieces(const std::vector<uint8_t>& piece_ok, size_t n, size_t L, uint64_t& rerun, Fn fn) {
+    rerun = 0;
+    for (size_t p = 0; p < piece_ok.size(); ) {
+        if (piece_ok[p]) { p++; continue; }
+        size_t q = p; while (q < piece_ok.size() && !piece_ok[q]) q++;
+        size_t lo = p * L, hi = q * L < n ? q * L : n;
+        if (int rc = fn(lo, hi)) return rc;
+        rerun += hi - lo; p = q;
     }
     return 0;
 }
@@ -969,9 +974,9 @@ static int verify_core(blsgpu_ctx* ctx, const u32x4* pk_soa, const uint8_t* code
     STAGE_MARK(5);
     if (dbitmap) LAUNCH(k_status_bitmap, nblk(((n + 31) / 32) * 32, 256), 256, (const uint8_t*)dstatus, n, dbitmap);
     if (gt_acc) {
-        u32x4* ta = ws_take<u32x4>(ctx, 36 * ((n + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((n + 63) / 64)); u32x4* one = ws_take<u32x4>(ctx, 36);
-        if (int rc = gt_product(ctx, f_soa, dstatus, n, ta, tb, one)) return rc;
-        LAUNCH(k_gt_mul_into, 1, 32, gt_acc, (const u32x4*)one);
+        u32x4* ta = ws_take<u32x4>(ctx, 36 * ((n + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((n + 63) / 64)); const u32x4* prod;
+        if (int rc = piece_tree<true>(ctx, f_soa, dstatus, n, n, ta, tb, prod)) return rc;
+        LAUNCH(k_gt_mul_into, 1, 32, gt_acc, prod);
     }
     STAGE_MARK(6);
     return 0;
@@ -983,18 +988,9 @@ static size_t verify_ws_bytes(size_t n, size_t mb) {
 static int ensure_lanes(blsgpu_ctx* ctx);
 // One contiguous sub-range [base, base+m) of a verify batch, enqueued entirely on ctx->stream (the caller may have pointed
 // it at a lane stream): staging, the five stage kernels, epilogue, outputs, and the range's GT partial (limb-SoA, n = 1).
-static int verify_range(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t base, size_t m,
-                        uint8_t* status, uint64_t* ok_bitmap, u32x4* gt_acc, size_t mb0, size_t mb) {
+static int verify_range(blsgpu_ctx* ctx, const batch_in& in, size_t base, size_t m, uint8_t* status, uint64_t* ok_bitmap, u32x4* gt_acc) {
     int rc = 0;
-    const uint8_t *dpk, *dsig, *dmsg; const uint32_t* doff;
-    if ((rc = stage_in(ctx, dpk, pk48 + 48 * base, 48 * m))) return rc;
-    if ((rc = stage_in(ctx, dsig, sig96 + 96 * base, 96 * m))) return rc;
-    if (ctx->ptr_mode == BLSGPU_HOST) {
-        // offsets in a host range are rebased by the kernel through (msg - mb0): stage the range's bytes only
-        if ((rc = stage_in(ctx, dmsg, msg + mb0, mb ? mb : 1))) return rc;
-        dmsg -= msg_off ? mb0 : 0;
-    } else dmsg = msg_off ? msg : msg + mb0;
-    if ((rc = stage_in(ctx, doff, msg_off ? msg_off + base : nullptr, m + 1))) return rc;
+    batch_dev d; if ((rc = stage_items(ctx, in, base, base + m, d))) return rc;
     uint8_t* dstatus = stage_out(ctx, status + base, m);
     uint32_t* dbitmap = (uint32_t*)stage_out(ctx, ok_bitmap ? ok_bitmap + base / 64 : nullptr, (m + 63) / 64);
     u32x4* pk_soa = ws_take<u32x4>(ctx, 6 * m); uint8_t* code_pk = ws_take<uint8_t>(ctx, m);
@@ -1005,8 +1001,8 @@ static int verify_range(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg
     bool forked = ctx->coop == 2 && m <= VERIFY_COOP_BELOW && !ctx->prof && ctx->split && ctx->stream != ctx->lane_stream[0] && ctx->stream != ctx->lane_stream[1];
     if (forked) { if ((rc = ensure_lanes(ctx))) return rc; forked = ctx->stream != ctx->lane_stream[0] && ctx->stream != ctx->lane_stream[1]; }
     if (forked) CU(cudaEventRecord(ctx->fork, ctx->stream));
-    LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-    if ((rc = verify_core(ctx, pk_soa, code_pk, dmsg, doff, dsig, m, dstatus, dbitmap, gt_acc, forked, true))) return rc;
+    LAUNCH(k_decode_g1, nblk(m), TPB, d.pk48, m, pk_soa, code_pk);
+    if ((rc = verify_core(ctx, pk_soa, code_pk, d.msg, d.msg_off, d.sig96, m, dstatus, dbitmap, gt_acc, forked, true))) return rc;
     if ((rc = finish_out(ctx, status + base, dstatus, m))) return rc;
     if (ok_bitmap && (rc = finish_out(ctx, ok_bitmap + base / 64, (uint64_t*)dbitmap, (m + 63) / 64))) return rc;
     return 0;
@@ -1019,28 +1015,24 @@ static int ensure_lanes(blsgpu_ctx* ctx) {
     return 0;
 }
 
-int blsgpu_verify_batch(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t n,
-                        uint8_t* status, uint64_t* ok_bitmap, uint8_t* gt_acc_le576) {
-    ENTER(); if (!pk48 || !msg || !sig96 || !status) return fail(ctx, BLSGPU_ERR_ARG, "null pointer");
-    int rc = 0;
+// blsgpu_verify_batch over the items [lo, hi) of a batch, lo a multiple of 64: status and ok_bitmap are indexed over the whole batch,
+// gt_acc_le576 receives the product over the range.
+static int verify_items(blsgpu_ctx* ctx, const batch_in& in, size_t lo, size_t hi, uint8_t* status, uint64_t* ok_bitmap, uint8_t* gt_acc_le576) {
+    int rc = 0; const size_t n = hi - lo;
     // Passes of <= ctx->chunk items bound the workspace (8.7 KB per item: ~9 GB at 2^20, of which 6.3 KB is the line buffer of the split Miller loop).  Inside a pass the items are split into `lanes`
     // contiguous sub-ranges enqueued on separate streams: the stage kernels of different sub-ranges are independent, so the
     // tail wave of one kernel overlaps the next sub-range's kernels (and, in host mode, its H2D copies) instead of idling SMs.
     // All range boundaries are multiples of 64 so bitmap words never straddle ranges.
     uint8_t gt_host[576];
-    const uint32_t* off_host = ctx->ptr_mode == BLSGPU_HOST ? msg_off : nullptr;
-    size_t total_mb = 0;
-    if (msg_off && !off_host) { total_mb = msg_bytes_total(ctx, msg_off, n, rc); if (rc) return fail(ctx, rc, "reading msg_off failed"); }
-    for (size_t base = 0; base < n; base += ctx->chunk) {
-        size_t m = n - base < ctx->chunk ? n - base : ctx->chunk;
+    for (size_t base = lo; base < hi; base += ctx->chunk) {
+        size_t m = hi - base < ctx->chunk ? hi - base : ctx->chunk;
         int lanes = ctx->lanes; if (lanes > MAX_LANES) lanes = MAX_LANES;
         while (lanes > 1 && m / lanes < 8192) lanes--;                     // keep every lane above ~0.2 waves of CTAs
         size_t per = ((m + lanes - 1) / lanes + 63) & ~(size_t)63;
         size_t ws = 65536;
         for (int l = 0; l < lanes; l++) {
-            size_t lo = base + l * per, hi = lo + per < base + m ? lo + per : base + m; if (lo >= hi) break;
-            size_t mb = msg_off ? (off_host ? off_host[hi] - off_host[lo] : total_mb) : 32 * (hi - lo);
-            ws += verify_ws_bytes(hi - lo, ctx->ptr_mode == BLSGPU_HOST ? mb : 0) + 4096;
+            size_t a = base + l * per, b = a + per < base + m ? a + per : base + m; if (a >= b) break;
+            ws += verify_ws_bytes(b - a, pass_msg_bytes(ctx, in, a, b)) + 4096;
         }
         if ((rc = ws_reserve(ctx, ws))) return rc;
         u32x4* gt_lane[MAX_LANES] = {nullptr, nullptr, nullptr, nullptr};
@@ -1048,12 +1040,10 @@ int blsgpu_verify_batch(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg
         if (lanes > 1) { if ((rc = ensure_lanes(ctx))) return rc; CU(cudaEventRecord(ctx->fork, main_stream)); }
         int used = 0;
         for (int l = 0; l < lanes; l++) {
-            size_t lo = base + l * per, hi = lo + per < base + m ? lo + per : base + m; if (lo >= hi) break;
-            size_t mb0 = msg_off ? (off_host ? off_host[lo] : 0) : 32 * lo;
-            size_t mb = msg_off ? (off_host ? off_host[hi] - off_host[lo] : 0) : 32 * (hi - lo);
+            size_t a = base + l * per, b = a + per < base + m ? a + per : base + m; if (a >= b) break;
             if (gt_acc_le576) gt_lane[l] = ws_take<u32x4>(ctx, 36);
             if (lanes > 1) { ctx->stream = ctx->lane_stream[l]; cudaStreamWaitEvent(ctx->stream, ctx->fork, 0); }
-            rc = verify_range(ctx, pk48, msg, msg_off, sig96, lo, hi - lo, status, ok_bitmap, gt_lane[l], mb0, mb);
+            rc = verify_range(ctx, in, a, b - a, status, ok_bitmap, gt_lane[l]);
             if (lanes > 1) { if (!rc) cudaEventRecord(ctx->lane_done[l], ctx->stream); ctx->stream = main_stream; }
             if (rc) return rc;
             used = l + 1;
@@ -1069,13 +1059,13 @@ int blsgpu_verify_batch(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg
                 // several passes: fold the pass partials one by one (synchronises; only taken for n > chunk)
                 uint8_t part[2][576];
                 CU(cudaMemcpyAsync(part[1], dgt, 576, cudaMemcpyDeviceToHost, ctx->stream)); CU(cudaStreamSynchronize(ctx->stream));
-                if (base == 0) memcpy(gt_host, part[1], 576);
+                if (base == lo) memcpy(gt_host, part[1], 576);
                 else {
                     memcpy(part[0], gt_host, 576);
                     int saved = ctx->ptr_mode; ctx->ptr_mode = BLSGPU_HOST;
                     rc = blsgpu_gt_fold(ctx, &part[0][0], 2, gt_host); ctx->ptr_mode = saved; if (rc) return rc;
                 }
-                if (base + m >= n) {
+                if (base + m >= hi) {
                     if (ctx->ptr_mode == BLSGPU_DEVICE) { CU(cudaMemcpyAsync(gt_acc_le576, gt_host, 576, cudaMemcpyHostToDevice, ctx->stream)); CU(cudaStreamSynchronize(ctx->stream)); }
                     else memcpy(gt_acc_le576, gt_host, 576);
                 }
@@ -1086,173 +1076,124 @@ int blsgpu_verify_batch(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg
     return 0;
 }
 
-// Random-linear-combination batch check: see include/blsgpu.h.  Single stream, passes of <= ctx->chunk items.
+int blsgpu_verify_batch(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t n,
+                        uint8_t* status, uint64_t* ok_bitmap, uint8_t* gt_acc_le576) {
+    ENTER(); if (!pk48 || !msg || !sig96 || !status) return fail(ctx, BLSGPU_ERR_ARG, "null pointer");
+    return verify_items(ctx, batch_in{pk48, msg, msg_off, sig96}, 0, n, status, ok_bitmap, gt_acc_le576);
+}
+
+// ---- random-linear-combination batch checks (SURVEY 8(f)-3): a pass of m items is cut into pieces of L items, and each piece is one equation
+#define RLC_PIECE 4096
+// piece-wise checks run passes of whole pieces: the chunk rounded down to a multiple of RLC_PIECE, at least one piece
+static size_t piece_chunk(const blsgpu_ctx* ctx) { return ctx->chunk >= RLC_PIECE ? ctx->chunk / RLC_PIECE * RLC_PIECE : RLC_PIECE; }
+// the seed on the device, in ctx->rlc_acc (allocated on first use; it also holds the accumulators of blsgpu_verify_batch_rlc)
+static int rlc_seed(blsgpu_ctx* ctx, const uint8_t* seed16, uint8_t*& dseed) {
+    if (!ctx->rlc_acc) CU(cudaMalloc(&ctx->rlc_acc, 2048));
+    dseed = ctx->rlc_acc + 1040;
+    CU(cudaMemcpyAsync(dseed, seed16, 16, ctx->ptr_mode == BLSGPU_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, ctx->stream));
+    return 0;
+}
+// The workspace of an RLC pass of m items in pieces of L besides its staging: the verify arrays, the weighted signatures rs, the levels of
+// the two piece trees (ja, jb: G2 sums, ta, tb: GT products), one ok flag per piece and the state of the split Miller loop.
+// rlc_ws_bytes is what rlc_carve takes.
+struct rlc_bufs { u32x4 *pk_soa, *sig_soa, *hm_soa, *f_soa, *rs, *ja, *jb, *ta, *tb, *t_soa, *lines; uint8_t *code_pk, *code_sig, *flags, *ok; };
+static size_t rlc_ws_bytes(const blsgpu_ctx* ctx, size_t m, size_t L) {
+    size_t P = (m + L - 1) / L, T0 = (L + 7) / 8;
+    return al(96 * m) + 2 * al(192 * m) + al(576 * m) + al(288 * m) + 2 * al(288 * P * T0) + 2 * al(576 * P * T0) +
+           (ctx->split ? al(576 * m) + al((size_t)MILLER_LINE_STEPS * 576 * m) : 0) + 3 * al(m) + al(P);
+}
+static rlc_bufs rlc_carve(blsgpu_ctx* ctx, size_t m, size_t L) {
+    size_t P = (m + L - 1) / L, T0 = (L + 7) / 8; rlc_bufs b;
+    b.pk_soa = ws_take<u32x4>(ctx, 6 * m); b.sig_soa = ws_take<u32x4>(ctx, 12 * m); b.hm_soa = ws_take<u32x4>(ctx, 12 * m); b.f_soa = ws_take<u32x4>(ctx, 36 * m);
+    b.rs = ws_take<u32x4>(ctx, 18 * m); b.ja = ws_take<u32x4>(ctx, 18 * P * T0); b.jb = ws_take<u32x4>(ctx, 18 * P * T0);
+    b.ta = ws_take<u32x4>(ctx, 36 * P * T0); b.tb = ws_take<u32x4>(ctx, 36 * P * T0);
+    b.t_soa = ctx->split ? ws_take<u32x4>(ctx, 36 * m) : nullptr; b.lines = ctx->split ? ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 36 * m) : nullptr;
+    b.code_pk = ws_take<uint8_t>(ctx, m); b.code_sig = ws_take<uint8_t>(ctx, m); b.flags = ws_take<uint8_t>(ctx, m); b.ok = ws_take<uint8_t>(ctx, P);
+    return b;
+}
+// the weights of items [base, base + m): decode, status / flags and H(m), then pk <- [r_i] pk and rs = [r_i] sig, pair 0 switched off
+static int rlc_item_front(blsgpu_ctx* ctx, const batch_dev& d, size_t base, size_t m, const uint8_t* dseed, uint8_t* dstatus, const rlc_bufs& b) {
+    LAUNCH(k_decode_g1, nblk(m), TPB, d.pk48, m, b.pk_soa, b.code_pk);
+    LAUNCH(k_decode_g2<true>, nblk(m), TPB, d.sig96, m, b.sig_soa, b.code_sig);
+    if (int rc = hash_stage(ctx, d.msg, d.msg_off, m, b.code_pk, b.code_sig, b.hm_soa, b.f_soa, b.flags, dstatus)) return rc;
+    LAUNCH(k_rlc_scale, nblk(m), TPB, b.pk_soa, (const u32x4*)b.sig_soa, b.flags, (const uint8_t*)dstatus, m, base, dseed, b.rs);
+    return 0;
+}
+// The equations of a pass whose weights are applied: per piece of L the sum of the weighted signatures (s_piece) and the product of the Miller
+// values with pair 0 switched off (f_piece), P rows each, not finished.
+static int rlc_pieces(blsgpu_ctx* ctx, const rlc_bufs& b, uint8_t* dstatus, size_t m, size_t L, const u32x4*& f_piece, const u32x4*& s_piece) {
+    if (int rc = piece_tree<false>(ctx, b.rs, nullptr, m, L, b.ja, b.jb, s_piece)) return rc;
+    if (ctx->split) { if (int rc = miller_stage_split(ctx, b.pk_soa, b.hm_soa, b.sig_soa, b.flags, dstatus, m, b.f_soa, b.t_soa, b.lines, nullptr)) return rc; }
+    else LAUNCH(k_miller, nblk(m), TPB, b.pk_soa, b.hm_soa, b.sig_soa, b.flags, (const uint8_t*)dstatus, m, b.f_soa);
+    return piece_tree<true>(ctx, b.f_soa, dstatus, m, L, b.ta, b.tb, f_piece);
+}
+// ok_bitmap (nullable) from the final status bytes of a call: bit i set <=> status[i] == ST_OK
+static int bitmap_from_status(blsgpu_ctx* ctx, const uint8_t* status, size_t n, uint64_t* ok_bitmap) {
+    if (!ok_bitmap) return 0;
+    if (ctx->ptr_mode == BLSGPU_HOST) { size_t words = (n + 63) / 64; for (size_t w = 0; w < words; w++) ok_bitmap[w] = 0; for (size_t i = 0; i < n; i++) if (status[i] == ST_OK) ok_bitmap[i >> 6] |= 1ull << (i & 63); }
+    else { CU(cudaMemsetAsync(ok_bitmap, 0, 8 * ((n + 63) / 64), ctx->stream)); LAUNCH(k_status_bitmap, nblk(((n + 31) / 32) * 32, 256), 256, status, n, (uint32_t*)ok_bitmap); }
+    return 0;
+}
+
+// Random-linear-combination batch check: see include/blsgpu.h.  Single stream, passes of <= ctx->chunk items, one piece per pass: the
+// pass's (F, S) are folded into accumulators that live across passes, and one equation decides.
 int blsgpu_verify_batch_rlc(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t n,
                             const uint8_t seed16[16], uint8_t* status, uint8_t* all_ok) {
     ENTER(); if (!pk48 || !msg || !sig96 || !seed16 || !all_ok) return fail(ctx, BLSGPU_ERR_ARG, "null pointer");
-    int rc = 0;
-    const uint32_t* off_host = ctx->ptr_mode == BLSGPU_HOST ? msg_off : nullptr;
-    size_t total_mb = 0;
-    if (msg_off && !off_host) { total_mb = msg_bytes_total(ctx, msg_off, n, rc); if (rc) return fail(ctx, rc, "reading msg_off failed"); }
-    // accumulators that live across passes are separate allocations (the workspace is re-carved per pass)
-    if (!ctx->rlc_acc) CU(cudaMalloc(&ctx->rlc_acc, 2048));
-    u32x4* f_acc = reinterpret_cast<u32x4*>(ctx->rlc_acc); u32x4* s_acc = f_acc + 36; uint32_t* bad = reinterpret_cast<uint32_t*>(ctx->rlc_acc + 1024);
-    uint8_t* dseed = ctx->rlc_acc + 1040; uint8_t* dok = ctx->rlc_acc + 1056;
-    auto release = [&]() {};
-    cudaMemcpyKind in_kind = ctx->ptr_mode == BLSGPU_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    CU(cudaMemcpyAsync(dseed, seed16, 16, in_kind, ctx->stream)); CU(cudaMemsetAsync(bad, 0, 4, ctx->stream));
+    int rc = 0; uint8_t* dseed;
+    if ((rc = rlc_seed(ctx, seed16, dseed))) return rc;
+    u32x4* f_acc = reinterpret_cast<u32x4*>(ctx->rlc_acc); u32x4* s_acc = f_acc + 36; uint32_t* bad = reinterpret_cast<uint32_t*>(ctx->rlc_acc + 1024); uint8_t* dok = ctx->rlc_acc + 1056;
+    CU(cudaMemsetAsync(bad, 0, 4, ctx->stream));
     LAUNCH(k_gt_set_one, 1, 32, f_acc); LAUNCH(k_g2_jac_set_identity, 1, 32, s_acc);
-    for (size_t base = 0; base < n && !rc; base += ctx->chunk) {
+    const batch_in in = {pk48, msg, msg_off, sig96};
+    for (size_t base = 0; base < n; base += ctx->chunk) {
         size_t m = n - base < ctx->chunk ? n - base : ctx->chunk;
-        size_t mb0 = msg_off ? (off_host ? off_host[base] : 0) : 32 * base;
-        size_t mb = msg_off ? (off_host ? off_host[base + m] - off_host[base] : total_mb) : 32 * m;
-        if ((rc = ws_reserve(ctx, verify_ws_bytes(m, ctx->ptr_mode == BLSGPU_HOST ? mb : 0) + al(288 * m) + al(288 * ((m + 7) / 8)) + al(288 * ((m + 63) / 64)) + al(288) + 65536))) break;
-        const uint8_t *dpk, *dsig, *dmsg; const uint32_t* doff;
-        if ((rc = stage_in(ctx, dpk, pk48 + 48 * base, 48 * m))) break;
-        if ((rc = stage_in(ctx, dsig, sig96 + 96 * base, 96 * m))) break;
-        if (ctx->ptr_mode == BLSGPU_HOST) { if ((rc = stage_in(ctx, dmsg, msg + mb0, mb ? mb : 1))) break; dmsg -= msg_off ? mb0 : 0; }
-        else dmsg = msg_off ? msg : msg + mb0;
-        if ((rc = stage_in(ctx, doff, msg_off ? msg_off + base : nullptr, m + 1))) break;
+        if ((rc = ws_reserve(ctx, stage_ws_bytes(m, pass_msg_bytes(ctx, in, base, base + m)) + rlc_ws_bytes(ctx, m, m) + 65536))) return rc;
+        batch_dev d; if ((rc = stage_items(ctx, in, base, base + m, d))) return rc;
         uint8_t* dstatus = status ? stage_out(ctx, status + base, m) : ws_take<uint8_t>(ctx, m);
-        u32x4* pk_soa = ws_take<u32x4>(ctx, 6 * m); uint8_t* code_pk = ws_take<uint8_t>(ctx, m);
-        u32x4* sig_soa = ws_take<u32x4>(ctx, 12 * m); u32x4* hm_soa = ws_take<u32x4>(ctx, 12 * m); u32x4* f_soa = ws_take<u32x4>(ctx, 36 * m);
-        uint8_t* code_sig = ws_take<uint8_t>(ctx, m); uint8_t* flags = ws_take<uint8_t>(ctx, m);
-        u32x4* rs = ws_take<u32x4>(ctx, 18 * m); u32x4* ja = ws_take<u32x4>(ctx, 18 * ((m + 7) / 8)); u32x4* jb = ws_take<u32x4>(ctx, 18 * ((m + 63) / 64)); u32x4* jone = ws_take<u32x4>(ctx, 18);
-        u32x4* ta = ws_take<u32x4>(ctx, 36 * ((m + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((m + 63) / 64)); u32x4* one = ws_take<u32x4>(ctx, 36);
-        LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-        LAUNCH(k_decode_g2<true>, nblk(m), TPB, dsig, m, sig_soa, code_sig);
-        if ((rc = hash_stage(ctx, dmsg, doff, m, code_pk, code_sig, hm_soa, f_soa, flags, dstatus))) break;
+        rlc_bufs b = rlc_carve(ctx, m, m); const u32x4 *f, *s;
+        if ((rc = rlc_item_front(ctx, d, base, m, dseed, dstatus, b))) return rc;
         LAUNCH(k_any_bad, nblk(((m + 31) / 32) * 32, 256), 256, (const uint8_t*)dstatus, m, bad);
-        LAUNCH(k_rlc_scale, nblk(m), TPB, pk_soa, (const u32x4*)sig_soa, flags, (const uint8_t*)dstatus, m, base, (const uint8_t*)dseed, rs);
-        {   // sum of the scaled signatures (radix-8 tree, like the GT product)
-            const u32x4* cur = rs; size_t cnt = m; u32x4* bufs[2] = {ja, jb}; int which = 0;
-            while (true) {
-                size_t T = (cnt + 7) / 8; u32x4* out = T == 1 ? jone : bufs[which];
-                LAUNCH(k_g2_jac_reduce, nblk(T), TPB, cur, cnt, out, T);
-                if (T == 1) break;
-                cur = out; cnt = T; which ^= 1;
-            }
-            LAUNCH(k_g2_jac_add_into, 1, 32, s_acc, (const u32x4*)jone);
-        }
-        if (ctx->split) {                                        // verify_ws_bytes counts the running-point array and the line buffer
-            u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
-            if ((rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr))) break;
-        } else LAUNCH(k_miller, nblk(m), TPB, (const u32x4*)pk_soa, (const u32x4*)hm_soa, (const u32x4*)sig_soa, (const uint8_t*)flags, (const uint8_t*)dstatus, m, f_soa);
-        if ((rc = gt_product(ctx, f_soa, dstatus, m, ta, tb, one))) break;
-        LAUNCH(k_gt_mul_into, 1, 32, f_acc, (const u32x4*)one);
-        if (status && (rc = finish_out(ctx, status + base, dstatus, m))) break;
-        if (ctx->ptr_mode == BLSGPU_HOST || n > ctx->chunk) { cudaError_t e = cudaStreamSynchronize(ctx->stream); if (e != cudaSuccess) { rc = fail(ctx, BLSGPU_ERR_CUDA, "sync failed: %s", cudaGetErrorString(e)); break; } }
+        if ((rc = rlc_pieces(ctx, b, dstatus, m, m, f, s))) return rc;
+        LAUNCH(k_g2_jac_add_into, 1, 32, s_acc, s); LAUNCH(k_gt_mul_into, 1, 32, f_acc, f);
+        if (status && (rc = finish_out(ctx, status + base, dstatus, m))) return rc;
+        if (ctx->ptr_mode == BLSGPU_HOST || n > ctx->chunk) CU(cudaStreamSynchronize(ctx->stream));
     }
-    if (!rc) {
-        k_rlc_finish<<<1, 32, 0, ctx->stream>>>(f_acc, s_acc, bad, dok); ctx->launches++;
-        cudaError_t e = cudaMemcpyAsync(all_ok, dok, 1, ctx->ptr_mode == BLSGPU_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess && ctx->ptr_mode == BLSGPU_HOST) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = fail(ctx, BLSGPU_ERR_CUDA, "rlc finish failed: %s", cudaGetErrorString(e));
-    }
-    release();
-    return rc;
+    LAUNCH(k_rlc_finish_seg, 1, 32, (const u32x4*)f_acc, (const u32x4*)s_acc, (size_t)1, (const uint32_t*)bad, dok);
+    CU(cudaMemcpyAsync(all_ok, dok, 1, ctx->ptr_mode == BLSGPU_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, ctx->stream));
+    return finish_call(ctx);
 }
 
 // Batch check that returns the EXACT per-item outcome (SURVEY 8(f)-3: "fall back to per-item checks to recover the exact bitmap when
 // the batch fails").  One random-linear-combination equation per PIECE of RLC_PIECE items, all pieces finished side by side; a piece
-// whose equation fails is re-run through the per-item path (blsgpu_verify_batch) inside this call.  status[i] and ok_bitmap equal
+// whose equation fails is re-run through the per-item path (verify_items) inside this call.  status[i] and ok_bitmap equal
 // blsgpu_verify_batch's except with probability <= 2^-64 per failing piece over the seed; fallback_items (nullable, host) = items re-run.
-#define RLC_PIECE 4096
-// The per-piece equations of a pass of m items whose weights are applied (pk_soa = [r] pk, rs = [r] sig, pair 0 switched off in flags):
-// per-piece sums of the scaled signatures and products of the Miller values (radix-8 trees, all pieces in one launch per level), then
-// ok[p] for every piece.  ja, jb: 18 P T0 rows, ta, tb: 36 P T0 rows (T0 = RLC_PIECE / 8); the split Miller loop takes its state from the workspace.
-static int rlc_pieces(blsgpu_ctx* ctx, const u32x4* rs, const u32x4* pk_soa, const u32x4* hm_soa, const u32x4* sig_soa, const uint8_t* flags, uint8_t* dstatus, size_t m,
-                      u32x4* f_soa, u32x4* ja, u32x4* jb, u32x4* ta, u32x4* tb, uint8_t* dok) {
-    const size_t L = RLC_PIECE, P = (m + L - 1) / L;
-    const u32x4* s_piece; const u32x4* f_piece;
-    {   // per-piece sums of the scaled signatures: radix-8 trees, all pieces in one launch per level
-        const u32x4* cur = rs; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ja, jb}; int which = 0;
-        while (true) {
-            size_t T = (len + 7) / 8; u32x4* out = bufs[which];
-            k_g2_jac_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
-            cur = out; cnt_n = P * T; len = T; which ^= 1;
-            if (T == 1) break;
-        }
-        s_piece = cur;
-    }
-    if (ctx->split) {
-        u32x4* t_soa = ws_take<u32x4>(ctx, 36 * m); u32x4* lines = ws_take<u32x4>(ctx, (size_t)MILLER_LINE_STEPS * 2 * 18 * m);
-        if (int rc = miller_stage_split(ctx, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, t_soa, lines, nullptr)) return rc;
-    } else LAUNCH(k_miller, nblk(m), TPB, pk_soa, hm_soa, sig_soa, flags, (const uint8_t*)dstatus, m, f_soa);
-    {
-        const u32x4* cur = f_soa; const uint8_t* st = dstatus; size_t cnt_n = m, len = L; u32x4* bufs[2] = {ta, tb}; int which = 0;
-        while (true) {
-            size_t T = (len + 7) / 8; u32x4* out = bufs[which];
-            k_gt_reduce_seg<<<dim3(nblk(T), (unsigned)P), TPB, 0, ctx->stream>>>(cur, st, cnt_n, len, out, T, P); ctx->launches++; CU(cudaGetLastError());
-            cur = out; st = nullptr; cnt_n = P * T; len = T; which ^= 1;
-            if (T == 1) break;
-        }
-        f_piece = cur;
-    }
-    LAUNCH(k_rlc_finish_seg, (unsigned)P, 32, f_piece, s_piece, P, dok);
-    return 0;
-}
 int blsgpu_verify_batch_rlc_bisect(blsgpu_ctx* ctx, const uint8_t* pk48, const uint8_t* msg, const uint32_t* msg_off, const uint8_t* sig96, size_t n,
                                    const uint8_t seed16[16], uint8_t* status, uint64_t* ok_bitmap, uint64_t* fallback_items) {
     ENTER(); if (!pk48 || !msg || !sig96 || !seed16 || !status) return fail(ctx, BLSGPU_ERR_ARG, "null pointer");
     if (fallback_items) *fallback_items = 0;
     if (!n) return 0;
-    int rc = 0; bool host = ctx->ptr_mode == BLSGPU_HOST;
-    const uint32_t* off_host = host ? msg_off : nullptr;
-    size_t total_mb = 0;
-    if (msg_off && !off_host) { total_mb = msg_bytes_total(ctx, msg_off, n, rc); if (rc) return fail(ctx, rc, "reading msg_off failed"); }
-    if (!ctx->rlc_acc) CU(cudaMalloc(&ctx->rlc_acc, 2048));
-    uint8_t* dseed = ctx->rlc_acc + 1040;
-    CU(cudaMemcpyAsync(dseed, seed16, 16, host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, ctx->stream));
-    const size_t L = RLC_PIECE;
+    int rc = 0; uint8_t* dseed; const size_t L = RLC_PIECE, chunk = piece_chunk(ctx);
+    if ((rc = rlc_seed(ctx, seed16, dseed))) return rc;
+    const batch_in in = {pk48, msg, msg_off, sig96};
     std::vector<uint8_t> piece_ok((n + L - 1) / L, 1);
-    size_t chunk = ctx->chunk >= L ? ctx->chunk / L * L : L;                 // pieces never straddle passes
     for (size_t base = 0; base < n; base += chunk) {
-        size_t m = n - base < chunk ? n - base : chunk, P = (m + L - 1) / L, T0 = (L + 7) / 8;
-        size_t mb0 = msg_off ? (off_host ? off_host[base] : 0) : 32 * base;
-        size_t mb = msg_off ? (off_host ? off_host[base + m] - off_host[base] : total_mb) : 32 * m;
-        if ((rc = ws_reserve(ctx, verify_ws_bytes(m, host ? mb : 0) + al(288 * m) + 2 * al(288 * P * T0) + 2 * al(576 * P * T0) + al(P) + 65536))) return rc;
-        const uint8_t *dpk, *dsig, *dmsg; const uint32_t* doff;
-        if ((rc = stage_in(ctx, dpk, pk48 + 48 * base, 48 * m))) return rc;
-        if ((rc = stage_in(ctx, dsig, sig96 + 96 * base, 96 * m))) return rc;
-        if (host) { if ((rc = stage_in(ctx, dmsg, msg + mb0, mb ? mb : 1))) return rc; dmsg -= msg_off ? mb0 : 0; }
-        else dmsg = msg_off ? msg : msg + mb0;
-        if ((rc = stage_in(ctx, doff, msg_off ? msg_off + base : nullptr, m + 1))) return rc;
+        size_t m = n - base < chunk ? n - base : chunk, P = (m + L - 1) / L;
+        if ((rc = ws_reserve(ctx, stage_ws_bytes(m, pass_msg_bytes(ctx, in, base, base + m)) + rlc_ws_bytes(ctx, m, L) + 65536))) return rc;
+        batch_dev d; if ((rc = stage_items(ctx, in, base, base + m, d))) return rc;
         uint8_t* dstatus = stage_out(ctx, status + base, m);
-        u32x4* pk_soa = ws_take<u32x4>(ctx, 6 * m); uint8_t* code_pk = ws_take<uint8_t>(ctx, m);
-        u32x4* sig_soa = ws_take<u32x4>(ctx, 12 * m); u32x4* hm_soa = ws_take<u32x4>(ctx, 12 * m); u32x4* f_soa = ws_take<u32x4>(ctx, 36 * m);
-        uint8_t* code_sig = ws_take<uint8_t>(ctx, m); uint8_t* flags = ws_take<uint8_t>(ctx, m);
-        u32x4* rs = ws_take<u32x4>(ctx, 18 * m); u32x4* ja = ws_take<u32x4>(ctx, 18 * P * T0); u32x4* jb = ws_take<u32x4>(ctx, 18 * P * T0);
-        u32x4* ta = ws_take<u32x4>(ctx, 36 * P * T0); u32x4* tb = ws_take<u32x4>(ctx, 36 * P * T0); uint8_t* dok = ws_take<uint8_t>(ctx, P);
-        LAUNCH(k_decode_g1, nblk(m), TPB, dpk, m, pk_soa, code_pk);
-        LAUNCH(k_decode_g2<true>, nblk(m), TPB, dsig, m, sig_soa, code_sig);
-        if ((rc = hash_stage(ctx, dmsg, doff, m, code_pk, code_sig, hm_soa, f_soa, flags, dstatus))) return rc;
-        LAUNCH(k_rlc_scale, nblk(m), TPB, pk_soa, (const u32x4*)sig_soa, flags, (const uint8_t*)dstatus, m, base, (const uint8_t*)dseed, rs);
-        if ((rc = rlc_pieces(ctx, rs, pk_soa, hm_soa, sig_soa, flags, dstatus, m, f_soa, ja, jb, ta, tb, dok))) return rc;
+        rlc_bufs b = rlc_carve(ctx, m, L); const u32x4 *f, *s;
+        if ((rc = rlc_item_front(ctx, d, base, m, dseed, dstatus, b))) return rc;
+        if ((rc = rlc_pieces(ctx, b, dstatus, m, L, f, s))) return rc;
+        LAUNCH(k_rlc_finish_seg, (unsigned)P, 32, f, s, P, (const uint32_t*)nullptr, b.ok);
         if ((rc = finish_out(ctx, status + base, dstatus, m))) return rc;
-        CU(cudaMemcpyAsync(piece_ok.data() + base / L, dok, P, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(piece_ok.data() + base / L, b.ok, P, cudaMemcpyDeviceToHost, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
     }
-    // failing pieces: the per-item path on exactly those items (adjacent failing pieces are merged into one call)
-    uint64_t rerun = 0;
-    for (size_t p = 0; p < piece_ok.size(); ) {
-        if (piece_ok[p]) { p++; continue; }
-        size_t q = p; while (q < piece_ok.size() && !piece_ok[q]) q++;
-        size_t lo = p * L, hi = q * L < n ? q * L : n;
-        const uint8_t* m_ptr; const uint32_t* o_ptr;
-        std::vector<uint32_t> rebased;
-        if (!msg_off) { m_ptr = msg + 32 * lo; o_ptr = nullptr; }
-        else if (host) { rebased.resize(hi - lo + 1); for (size_t i = 0; i <= hi - lo; i++) rebased[i] = msg_off[lo + i] - msg_off[lo]; m_ptr = msg + msg_off[lo]; o_ptr = rebased.data(); }
-        else { m_ptr = msg; o_ptr = msg_off + lo; }                       // device offsets are absolute into msg
-        if ((rc = blsgpu_verify_batch(ctx, pk48 + 48 * lo, m_ptr, o_ptr, sig96 + 96 * lo, hi - lo, status + lo, nullptr, nullptr))) return rc;
-        if (!host) CU(cudaStreamSynchronize(ctx->stream));
-        rerun += hi - lo; p = q;
-    }
+    uint64_t rerun;
+    if ((rc = rerun_failing_pieces(piece_ok, n, L, rerun, [&](size_t lo, size_t hi) { return verify_items(ctx, in, lo, hi, status, nullptr, nullptr); }))) return rc;
     if (fallback_items) *fallback_items = rerun;
-    if (ok_bitmap) {
-        if (host) { size_t words = (n + 63) / 64; for (size_t w = 0; w < words; w++) ok_bitmap[w] = 0; for (size_t i = 0; i < n; i++) if (status[i] == ST_OK) ok_bitmap[i >> 6] |= 1ull << (i & 63); }
-        else { CU(cudaMemsetAsync(ok_bitmap, 0, 8 * ((n + 63) / 64), ctx->stream)); LAUNCH(k_status_bitmap, nblk(((n + 31) / 32) * 32, 256), 256, (const uint8_t*)status, n, (uint32_t*)ok_bitmap); }
-    }
+    if ((rc = bitmap_from_status(ctx, status, n, ok_bitmap))) return rc;
     return finish_call(ctx);
 }
 
@@ -1260,11 +1201,11 @@ int blsgpu_gt_fold(blsgpu_ctx* ctx, const uint8_t* parts, size_t nparts, uint8_t
     ENTER(); if (!parts || !out || !nparts) return fail(ctx, BLSGPU_ERR_ARG, "bad argument");
     if (int rc = ws_reserve(ctx, al(576 * nparts) * 2 + al(576 * ((nparts + 7) / 8)) + al(576 * ((nparts + 63) / 64)) + 2 * al(576) + 8192)) return rc;
     const uint8_t* din; if (int rc = stage_in(ctx, din, parts, 576 * nparts)) return rc;
-    u32x4* soa = ws_take<u32x4>(ctx, 36 * nparts); u32x4* ta = ws_take<u32x4>(ctx, 36 * ((nparts + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((nparts + 63) / 64)); u32x4* one = ws_take<u32x4>(ctx, 36);
+    u32x4* soa = ws_take<u32x4>(ctx, 36 * nparts); u32x4* ta = ws_take<u32x4>(ctx, 36 * ((nparts + 7) / 8)); u32x4* tb = ws_take<u32x4>(ctx, 36 * ((nparts + 63) / 64)); const u32x4* prod;
     uint8_t* dout = stage_out(ctx, out, 576);
     LAUNCH(k_gt_from_bytes, nblk(nparts), TPB, din, nparts, soa);
-    if (int rc = gt_product(ctx, soa, nullptr, nparts, ta, tb, one)) return rc;
-    LAUNCH(k_gt_to_bytes, 1, TPB, (const u32x4*)one, (size_t)1, dout, (const uint8_t*)nullptr);
+    if (int rc = piece_tree<true>(ctx, soa, nullptr, nparts, nparts, ta, tb, prod)) return rc;
+    LAUNCH(k_gt_to_bytes, 1, TPB, prod, (size_t)1, dout, (const uint8_t*)nullptr);
     if (int rc = finish_out(ctx, out, dout, 576)) return rc;
     return finish_call(ctx);
 }
